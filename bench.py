@@ -61,6 +61,32 @@ def cfg_dims():
     return N, N * L, 3 * L, CFG["H"], CFG["C"]
 
 
+# --------------------------------------------------------------------------- --dump-outputs
+DUMP_MAX_ELEMS = 1 << 22          # per array; the largest outputs (config A's 246 MB `out`) are sampled down to this
+DUMP_MAX_BYTES = 64 << 20         # all arrays together
+
+
+def sample_rows(t: torch.Tensor, seed: int = 0) -> torch.Tensor:
+    """t itself, or - when it holds more than DUMP_MAX_ELEMS elements - a fixed, seeded sample of its rows, in row order."""
+    if t.numel() <= DUMP_MAX_ELEMS:
+        return t
+    keep = max(1, DUMP_MAX_ELEMS // (t.numel() // t.shape[0]))
+    idx = torch.randperm(t.shape[0], generator=torch.Generator().manual_seed(seed))[:keep].sort().values
+    return t[idx.to(t.device)]
+
+
+def dump_outputs(path: str, arrays: dict) -> None:
+    """Writes {name: tensor} as <path>/<name>.npy in float32, rows sampled as by sample_rows."""
+    import numpy as np
+    host = {k: sample_rows(v.detach()).float().cpu().numpy() for k, v in arrays.items()}
+    total = sum(a.nbytes for a in host.values())
+    if total > DUMP_MAX_BYTES:
+        raise SystemExit(f"bench.py: --dump-outputs would write {total} bytes (> {DUMP_MAX_BYTES})")
+    os.makedirs(path, exist_ok=True)
+    for k, a in host.items():
+        np.save(os.path.join(path, k + ".npy"), a)
+
+
 # --------------------------------------------------------------------------- clocks
 class ClockSampler:
     """nvidia-smi clocks / throttle reasons sampled during the timed region (B200_PROFILING.md)."""
@@ -317,6 +343,15 @@ class HotPath:
             allreduce(self.arena)
             mark("allreduce")
 
+    def outputs(self) -> dict:
+        """What GATConv forward + backward hands its caller after the last step: the layer output and each parameter's
+        gradient, shaped like the parameter."""
+        grads = (("lin_src.weight", self.g_W), ("att_src", self.g_as), ("att_dst", self.g_ad),
+                 ("lin_edge.weight", self.g_We), ("att_edge", self.g_ae), ("bias", self.g_b))
+        res = {"out": self.out}
+        res.update({f"{k}.grad": g.view_as(self.layer.get_parameter(k)) for k, g in grads})
+        return res
+
 
 def bind_to_gpu_numa(local: int):
     """Pin this rank's threads to the CPUs NVML lists as local to its GPU, BEFORE any pinned host buffer is allocated (first
@@ -395,6 +430,8 @@ def run_ours(args):
     barrier()
     elapsed_ms = e0.elapsed_time(e1)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, hp.outputs())
     if world > 1:
         t = torch.tensor([elapsed_ms], device=dev, dtype=torch.float64)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -616,6 +653,8 @@ def run_config_c(args):
                      "timing": "median of per-step CUDA-event times"}
         if prec == "half":
             clocks = sampler.stop()
+            if args.dump_outputs:
+                dump_outputs(args.dump_outputs, {"loss": loss, **{f"{k}.grad": p.grad for k, p in model.named_parameters()}})
         # the attention kernels' share (incl. the backward's operand preparation of dout): one extra step under torch.profiler
         try:
             from torch.profiler import profile, ProfilerActivity
@@ -912,7 +951,15 @@ def main():
     ap.add_argument("--no-graph", action="store_true", help="skip the CUDA-graph replay side measurement")
     ap.add_argument("--p-format", type=int, default=None, choices=[0, 1], help="0: fp32 P_aug between GEMM and attention (round 1); 1: fp16 operand pair (default where it applies)")
     ap.add_argument("--split-x-in-step", action="store_true", help="derive x's operand pair from the fp32 x inside every step (round-1 behaviour)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (config A / D: out and the parameter gradients; "
+                         "config C: loss and the parameter gradients of the half-precision mode) as DIR/<name>.npy, float32; arrays "
+                         f"above {DUMP_MAX_ELEMS} elements are a fixed, seeded sample of their rows")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the CUDA path's outputs; the reference arm has none")
     CFG["N"] = CONFIGS[args.config]["N"]
     HotPath.SPLIT_X_IN_STEP = args.split_x_in_step
     HotPath.P_FORMAT = args.p_format

@@ -1,6 +1,6 @@
 """bench.py output contract, checked on CPU through the reference arm (the only arm that runs without a GPU):
-stdout carries exactly ONE JSON line with the keys the driver reads; under torchrun only rank 0 prints; our arm
-refuses to run without a CUDA device instead of falling back to anything."""
+stdout carries exactly ONE JSON line with the keys a caller reads; under torchrun only rank 0 prints; our arm
+refuses to run without a CUDA device instead of falling back to anything.  On a GPU: what --dump-outputs writes."""
 import json
 import os
 import subprocess
@@ -49,6 +49,29 @@ def test_reference_arm_under_torchrun_only_rank0_prints():
     assert r.returncode == 0, r.stderr[-2000:]
     d = _check_reference_line(r.stdout)
     assert d["n_gpus"] == 2
+
+
+@pytest.mark.gpu
+def test_dump_outputs_repeat_from_run_to_run(cuda_lib, tmp_path):
+    """--dump-outputs writes the last timed step's output and gradients as float32 .npy files, 64 MB at most (the output
+    rows above 2^22 elements sampled), and two runs with the same arguments write the same arrays."""
+    import numpy as np
+    args = [sys.executable, BENCH, "--batch", "512", "--steps", "2", "--warmup", "1", "--no-cpu-baseline", "--no-e2e",
+            "--no-structured", "--no-graph"]
+    shapes = {"out": (4194304 // 500, 500), "lin_src.weight.grad": (3000, 1260), "att_src.grad": (1, 6, 500),
+              "att_dst.grad": (1, 6, 500), "lin_edge.weight.grad": (3000, 126), "att_edge.grad": (1, 6, 500), "bias.grad": (500,)}
+    dumps = []
+    for k in range(2):
+        r = _run(args + ["--dump-outputs", str(tmp_path / str(k))])
+        assert r.returncode == 0, r.stderr[-2000:]
+        assert json.loads(r.stdout)["steps"] == 2
+        dumps.append({p.name[:-4]: np.load(p) for p in (tmp_path / str(k)).glob("*.npy")})
+    a, b = dumps
+    assert {k: v.shape for k, v in a.items()} == shapes
+    assert all(v.dtype == np.float32 for v in a.values()) and sum(v.nbytes for v in a.values()) <= 64 << 20
+    for k in shapes:
+        assert np.isfinite(a[k]).all() and np.abs(a[k]).max() > 0, k
+        assert np.abs(a[k] - b[k]).max() <= 1e-6 * np.abs(b[k]).max(), k
 
 
 def test_our_arm_fails_loudly_without_cuda():

@@ -1,6 +1,4 @@
-"""The torch_geometric import shim: the reference's OWN model file builds on our GATConv, unmodified.
-Runs only where /root/reference is mounted (this container); the GPU box does not have it."""
-import importlib.util
+"""The torch_geometric import shim exposes, backed by this package, the names SpotV2Net's own modules import."""
 import os
 import sys
 
@@ -8,7 +6,6 @@ import pytest
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF_MODELS = "/root/reference/utils/models.py"
 
 
 @pytest.fixture
@@ -37,28 +34,3 @@ def test_shim_exposes_the_names_the_reference_imports(shim_on_path):
     assert d.x.shape == (2, 3)
     with pytest.raises(TypeError):
         DataLoader([1, 2, 3], batch_size=2)
-
-
-@pytest.mark.skipif(not os.path.exists(REF_MODELS), reason="/root/reference is not mounted here")
-def test_reference_model_file_builds_on_our_layer_unmodified(shim_on_path):
-    import spotv2net_b200 as sv
-    spec = importlib.util.spec_from_file_location("ref_models", REF_MODELS)
-    ref_models = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(ref_models)                     # utils/models.py:11 imports torch_geometric.nn
-    kw = dict(num_node_features=30 * 42, num_edge_features=3 * 42, num_heads=6, output_node_channels=1,
-              dim_hidden_layers=[500], dropout_att=0.0, dropout=0.0, activation="relu", concat_heads=True,
-              negative_slope=0.2, standardize=False)        # config/GNN_param.yaml:26-38
-    torch.manual_seed(0)
-    theirs = ref_models.GATModel(**kw)
-    torch.manual_seed(0)
-    ours = sv.GATModel(**kw)
-    assert all(isinstance(l, sv.GATConv) for l in theirs.gat_layers)
-    sd_t, sd_o = theirs.state_dict(), ours.state_dict()
-    assert list(sd_t.keys()) == list(sd_o.keys())
-    assert all(sd_t[k].shape == sd_o[k].shape for k in sd_t)
-    assert all(torch.equal(sd_t[k], sd_o[k]) for k in sd_t)   # same construction order, same RNG draws
-    ours.load_state_dict(sd_t)                                # checkpoints are interchangeable
-    for cfg in (dict(dim_hidden_layers=[64, 32], concat_heads=True), dict(dim_hidden_layers=[64, 32, 16], concat_heads=False)):
-        a, b = ref_models.GATModel(**dict(kw, **cfg)), sv.GATModel(**dict(kw, **cfg))
-        assert [(l.in_channels, l.out_channels, l.concat) for l in a.gat_layers] == \
-               [(l.in_channels, l.out_channels, l.concat) for l in b.gat_layers]
