@@ -316,9 +316,10 @@ int spotv2_diag_dout_pair(const float* dout, int32_t B, int32_t N, int32_t C, in
  * Profiling aid only. */
 int spotv2_diag_counters(unsigned long long* host_out, int reset);
 
-/* Split-K factor spotv2_gat_proj_bwd_weight uses for dW_aug[m, n] = sum over `rows` (host-side rule, no device work):
- * ceil(rows / 8192) clamped to [1, 32], then raised by up to a quarter so that (128 x 256 output tiles) x splits fills
- * the last wave of the 148 persistent CTAs.  spotv2_gat_workspace_bytes sizes the partial buffers with the same rule. */
+/* Split-K factor spotv2_gat_proj_bwd_weight uses for dW_aug[m, n] = sum over `rows` (host-side rule, no kernel launch):
+ * ceil(rows / 8192) clamped to [1, 32], then raised by up to a quarter so that (256 x 256 pair tiles) x splits fills
+ * the last wave of the GEMM's resident CTA pairs (an occupancy query; 74 on a B200, sm_count / 2 without a device).
+ * spotv2_gat_workspace_bytes sizes the partial buffers with the same rule. */
 int32_t spotv2_diag_weight_grad_splits(int32_t rows, int32_t m, int32_t n);
 
 #ifdef __cplusplus

@@ -29,21 +29,27 @@ struct BGemm {
 };
 int bgemm_simt(bool a_kc, bool b_kc, BGemm g, int batches, cudaStream_t st);
 
+// CTA pairs of the fp16-pair GEMM kernel resident at once on the current device (sm_count / 2 without one).
+int gemm3x_f16_resident_pairs();
+
 // Split-K factor used for the weight-gradient GEMM (contraction over all B*N node rows): keeps
-// every fp32 accumulation chain short (<= ~8K terms) and fills the machine.
-inline int weight_grad_splits(int rows, int m, int n) {
+// every fp32 accumulation chain short (<= ~8K terms) and fills the machine.  pair_tiles: the product runs on 256 x 256
+// pair tiles over the resident CTA pairs (the 3-product class); false: 128 x 256 tiles over the SMs (half precision).
+inline int weight_grad_splits(int rows, int m, int n, bool pair_tiles = true) {
   int base = (rows + 8191) / 8192;
   if (base < 1) base = 1;
   if (base > 32) base = 32;
   if (base == 1) return 1;
-  // among base .. 1.25 base, the count whose (128 x 256 tile, split) work items fill the 148 persistent CTAs' last wave best
-  // (config A: 120 tiles x 15 splits = 12.16 waves, x 16 = 12.97)
-  const int tiles = ((m + 127) / 128) * ((n + 255) / 256);
+  // among base .. 1.25 base, the count whose (tile, split) work items fill the resident slots' last wave best
+  // (config A on 74 pairs: 60 pair tiles x 15 splits = 12.16 waves, x 16 = 12.97)
+  const int tile_m = pair_tiles ? 256 : 128;
+  const int tiles = ((m + tile_m - 1) / tile_m) * ((n + 255) / 256);
+  const int pairs = pair_tiles ? gemm3x_f16_resident_pairs() : sm_count();
   int best = base;
   double best_eff = 0.0;
   for (int s = base; s <= base + base / 4 + 1 && s <= 32; ++s) {
     const int items = tiles * s;
-    const double eff = (double)items / (double)(((items + 147) / 148) * 148);
+    const double eff = (double)items / (double)(((items + pairs - 1) / pairs) * pairs);
     if (eff > best_eff + 1e-9) { best = s; best_eff = eff; }
   }
   return best;

@@ -20,8 +20,13 @@
 // operand PAIR of C * s (hi | lo planes; s from an a-priori bound, see pair_out_scale), split in the epilogue registers and
 // stored through the same TMA path; the second column group (the logit terms s | d) additionally in fp32.
 //
-// Kernel shape: persistent, one CTA per SM, 384 threads (warp 0 TMA, warp 1 MMA issue, warp 2 TMEM
-// allocator, warps 4-11 accumulate + epilogue), tile 128 x 256 x TBK, TBK = 64 | 32 fp16 elements.
+// Kernel shape: persistent clusters of two CTAs (one per SM), 384 threads each (warp 0 TMA, warp 1 MMA issue, warp 2 TMEM
+// allocator, warps 4-11 accumulate + epilogue).  A work item is a PAIR tile of 256 x BN x TBK: CTA rank r loads A rows
+// pair_mt * 256 + r * 128 and half of B's BN columns, the leader (rank 0) issues cta_group::2 MMAs of M = 256 that read
+// both CTAs' shared memory, and each CTA drains its own 128 rows from its own TMEM.  Against a CTA that computes a 128 x BN
+// tile alone this cuts the TMA loads and the tensor core's shared-memory operand reads per SM by a third (B is no longer
+// loaded twice).  The single-product half-precision class runs the same template as one CTA per 128 x BN tile (see
+// gemm3x_f16).  TBK = 64 | 32 fp16 elements.
 #include <cuda_fp16.h>
 #include <stdio.h>
 #include <stdlib.h>
@@ -46,7 +51,7 @@ struct HParams {
   int M, N, K;
   int ldc;
   float* C;
-  int m_tiles, n_tiles, splits, kb_per_split, kb_total, kb_per_chunk;
+  int pm_tiles, n_tiles, splits, kb_per_split, kb_total, kb_per_chunk;   // pm_tiles: 256-row pair tiles
   size_t split_stride;
   const float* a_inv;   // 2 inverse scales of A's groups (null = 1)
   const float* b_inv;
@@ -70,17 +75,19 @@ struct HParams {
 #define SPOTV2_DBG(p) 0
 #endif
 
-template <int BN, int TBK, bool A_KM, bool B_KM>
+template <int BN, int TBK, bool A_KM, bool B_KM, int CTAS>
 struct HSmem {
-  static constexpr int kAOp = HBM_ * TBK * 2;              // one A operand tile (hi or lo), bytes
-  static constexpr int kBOp = BN * TBK * 2;
+  static constexpr int kAOp = HBM_ * TBK * 2;              // this CTA's 128 rows of one A operand tile (hi or lo), bytes
+  static constexpr int kBOp = (BN / CTAS) * TBK * 2;       // this CTA's share of the B tile's columns
   static constexpr int kStage = 2 * kAOp + 2 * kBOp;
-  // K-major x K-major with 32-element k-blocks (the forward projection): three 48 KB stages and FOUR 2 KB store boxes per
+  // K-major x K-major with 32-element k-blocks (the forward projection): three stages and FOUR 2 KB store boxes per
   // epilogue warp.  With two boxes the pair epilogue waited on the copy engine before six of its eight pieces (the stores
   // queue behind the operand loads); the MMA warp, which can run only two accumulation chunks ahead, stalled for it: 0.17 ms
-  // of the K = 1260 product (bring-up probe, tools/gemm_dbg_probe.sh).
+  // of the K = 1260 product (bring-up probe, tools/gemm_dbg_probe.sh).  Pair tiles keep the ring depths in k-blocks of the
+  // 1-CTA tiles (3, 4 at TBK = 32, 2 at TBK = 64), whose stages are half as large again.
   static constexpr bool kWideEpi = (TBK == 32) && A_KM && B_KM;
-  static constexpr int kStages = kWideEpi ? 3 : ((200 * 1024) / kStage > 6 ? 6 : (200 * 1024) / kStage);
+  static constexpr int kRingBytes = CTAS == 2 ? 160 * 1024 : 200 * 1024, kMaxStages = CTAS == 2 ? 4 : 6;
+  static constexpr int kStages = kWideEpi ? 3 : (kRingBytes / kStage > kMaxStages ? kMaxStages : kRingBytes / kStage);
   static constexpr int kBarOff = kStages * kStage;
   static constexpr int kEpiOff = kBarOff + 1024;                     // 8 epilogue warps x 4224 B: a 32 x 32 fp32 output block each
   static constexpr int kEpiWarpBytes = kWideEpi ? 8192 : 32 * 33 * 4;    // ([32][33] transpose, or 2 KB swizzled TMA store boxes)
@@ -88,15 +95,36 @@ struct HSmem {
   static constexpr int kPairBoxes = kWideEpi ? 4 : 2;
   static constexpr int kEpiBytes = kHEpiWarps * kEpiWarpBytes;
   static constexpr int kTotal = kEpiOff + kEpiBytes + 1024;
-  static constexpr uint32_t kTxBytes = kStage;
+  static constexpr uint32_t kTxBytes = CTAS * kStage;        // both CTAs' loads complete on the leader's full barrier
 };
 
-template <int BN, int TBK, bool A_KM, bool B_KM>
+// Bounded wait that names the barrier that starved before it traps: a lost arrival from the other CTA of the pair must
+// fail loudly instead of hanging the GPU.
+enum { kWaitFull = 0, kWaitEmpty, kWaitTempty, kWaitPeerEmpty };
+__device__ __noinline__ void gemm_wait_report(int id, uint32_t parity) {
+  const char* const names[] = {"full (operands landed)", "empty (stage consumed)", "tempty (accumulator drained)",
+                               "empty at exit (last stage released)"};
+  printf("gemm3x_f16: wait on %s timed out (block %d rank %u thread %d parity %u)\n", names[id], (int)blockIdx.x,
+         cluster_ctarank(), (int)threadIdx.x, parity);
+}
+__device__ __forceinline__ void hwait(uint64_t* bar, uint32_t parity, int id) {
+  for (int spin = 0; spin < 16; ++spin)
+    if (mbar_try_wait(bar, parity)) return;
+  const long long t0 = clock64();
+  while (!mbar_try_wait(bar, parity)) {
+    __nanosleep(64);
+    if (clock64() - t0 > 4000000000LL) { gemm_wait_report(id, parity); __trap(); }
+  }
+}
+
+// CTAS = 2: pair tiles on a cluster of two CTAs (launched with cluster dimension 2); CTAS = 1: every CTA computes a
+// 128 x BN tile alone (see gemm3x_f16 for which products take which).
+template <int BN, int TBK, bool A_KM, bool B_KM, int CTAS>
 __global__ void __launch_bounds__(kHThreads, 1)
 gemm3x_f16_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constant__ CUtensorMap tmAl,
                   const __grid_constant__ CUtensorMap tmBh, const __grid_constant__ CUtensorMap tmBl,
                   const __grid_constant__ CUtensorMap tmC, const HParams p) {
-  using S = HSmem<BN, TBK, A_KM, B_KM>;
+  using S = HSmem<BN, TBK, A_KM, B_KM, CTAS>;
   constexpr int kStages = S::kStages;
   extern __shared__ unsigned char smem_dyn[];
   unsigned char* smem = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(smem_dyn) + 1023) & ~uintptr_t(1023));
@@ -107,76 +135,107 @@ gemm3x_f16_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constan
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tempty + 2);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int total_tiles = p.m_tiles * p.n_tiles * p.splits;
+  const uint32_t rank = CTAS == 2 ? cluster_ctarank() : 0;
+  const int pair_id = blockIdx.x / CTAS, num_pairs = gridDim.x / CTAS;
+  const int total_items = p.pm_tiles * p.n_tiles * p.splits;
   constexpr uint32_t kTmemCols = 2 * BN;
 
   if (warp == 0 && lane == 0) {
     prefetch_tmap(&tmAh); prefetch_tmap(&tmAl); prefetch_tmap(&tmBh); prefetch_tmap(&tmBl);
   }
   if (warp == 1 && lane == 0) {
+    // full and tempty are used in the leader only: full completes on both CTAs' loads, tempty on both CTAs' drains
     for (int s = 0; s < kStages; ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], 1); }
-    for (int s = 0; s < 2; ++s) { mbar_init(&tfull[s], 1); mbar_init(&tempty[s], kHEpiWarps); }
+    for (int s = 0; s < 2; ++s) { mbar_init(&tfull[s], 1); mbar_init(&tempty[s], CTAS * kHEpiWarps); }
     fence_mbar_init();
   }
-  if (warp == 2) tmem_alloc(tmem_slot, kTmemCols);
-  tc_fence_before();
-  __syncthreads();
+  if constexpr (CTAS == 2) {
+    if (warp == 2) tmem_alloc_pair(tmem_slot, kTmemCols);
+    tc_fence_before();
+    cluster_sync();           // the peer's barriers are initialised before anything signals them
+  } else {
+    if (warp == 2) tmem_alloc(tmem_slot, kTmemCols);
+    tc_fence_before();
+    __syncthreads();
+  }
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
 
-  // n fastest: the CTAs of one wave share the A rows (x / dP tiles) through L2, B (weights) is small
-  auto tile_coords = [&](int tile, int& mt, int& nt, int& sp) {
-    nt = tile % p.n_tiles;
-    const int r = tile / p.n_tiles;
-    mt = r % p.m_tiles;
-    sp = r / p.m_tiles;
+  // n fastest: the pairs of one wave share the A rows (x / dP tiles) through L2, B (weights) is small.  This CTA's
+  // 128-row tile of the pair tile is mt; when m_tiles is odd the last pair's second half reads zeros (TMA fills rows >= M)
+  // and stores nothing.
+  auto tile_coords = [&](int item, int& mt, int& nt, int& sp) {
+    nt = item % p.n_tiles;
+    const int r = item / p.n_tiles;
+    mt = CTAS * (r % p.pm_tiles) + (int)rank;
+    sp = r / p.pm_tiles;
   };
 
   if (warp == 0) {
-    // ===================== TMA producer =====================
+    // ===================== TMA producer (both CTAs) =====================
     if (elect_one()) {
+      const uint32_t full_leader = CTAS == 2 ? mapa_shared(full, 0) : 0;
       int stage = 0; uint32_t phase = 0;
-      for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x) {
-        int mt, nt, sp; tile_coords(tile, mt, nt, sp);
+      for (int item = pair_id; item < total_items; item += num_pairs) {
+        int mt, nt, sp; tile_coords(item, mt, nt, sp);
         const int kb0 = sp * p.kb_per_split;
         const int kb1 = min(p.kb_total, kb0 + p.kb_per_split);
+        const int n0 = nt * BN + (int)rank * (BN / CTAS);
         for (int kb = kb0; kb < kb1; ++kb) {
-          mbar_wait(&empty[stage], phase ^ 1);
+          hwait(&empty[stage], phase ^ 1, kWaitEmpty);
           unsigned char* st = smem + stage * S::kStage;
           const bool lo = !p.single;
-          mbar_expect_tx(&full[stage], lo ? S::kTxBytes : S::kTxBytes / 2);
+          const uint32_t fb = full_leader + stage * (uint32_t)sizeof(uint64_t);
+          if (rank == 0) mbar_expect_tx(&full[stage], lo ? S::kTxBytes : S::kTxBytes / 2);
+          auto tma_load = [&](void* dst, const CUtensorMap* tm, int c0, int c1) {
+            if constexpr (CTAS == 2) tma_load_2d_pair(dst, tm, c0, c1, fb);
+            else tma_load_2d(dst, tm, c0, c1, &full[stage]);
+          };
           const int k = kb * TBK;
           if (A_KM) {
-            tma_load_2d(st, &tmAh, k, mt * HBM_, &full[stage]);
-            if (lo) tma_load_2d(st + S::kAOp, &tmAl, k, mt * HBM_, &full[stage]);
+            tma_load(st, &tmAh, k, mt * HBM_);
+            if (lo) tma_load(st + S::kAOp, &tmAl, k, mt * HBM_);
           } else {
 #pragma unroll
             for (int blk = 0; blk < HBM_ / 64; ++blk) {
-              tma_load_2d(st + blk * (TBK * 128), &tmAh, mt * HBM_ + blk * 64, k, &full[stage]);
-              if (lo) tma_load_2d(st + S::kAOp + blk * (TBK * 128), &tmAl, mt * HBM_ + blk * 64, k, &full[stage]);
+              tma_load(st + blk * (TBK * 128), &tmAh, mt * HBM_ + blk * 64, k);
+              if (lo) tma_load(st + S::kAOp + blk * (TBK * 128), &tmAl, mt * HBM_ + blk * 64, k);
             }
           }
           unsigned char* sb = st + 2 * S::kAOp;
           if (B_KM) {
-            tma_load_2d(sb, &tmBh, k, nt * BN, &full[stage]);
-            if (lo) tma_load_2d(sb + S::kBOp, &tmBl, k, nt * BN, &full[stage]);
+            tma_load(sb, &tmBh, k, n0);
+            if (lo) tma_load(sb + S::kBOp, &tmBl, k, n0);
           } else {
 #pragma unroll
-            for (int blk = 0; blk < BN / 64; ++blk) {
-              tma_load_2d(sb + blk * (TBK * 128), &tmBh, nt * BN + blk * 64, k, &full[stage]);
-              if (lo) tma_load_2d(sb + S::kBOp + blk * (TBK * 128), &tmBl, nt * BN + blk * 64, k, &full[stage]);
+            for (int blk = 0; blk < BN / CTAS / 64; ++blk) {
+              tma_load(sb + blk * (TBK * 128), &tmBh, n0 + blk * 64, k);
+              if (lo) tma_load(sb + S::kBOp + blk * (TBK * 128), &tmBl, n0 + blk * 64, k);
             }
           }
           if (++stage == kStages) { stage = 0; phase ^= 1; }
         }
       }
+      // the leader's last commits to this CTA's empty barriers must land before the CTA exits (pairs)
+      for (int s = 0; s < kStages; ++s) {
+        hwait(&empty[stage], phase ^ 1, kWaitPeerEmpty);
+        if (++stage == kStages) { stage = 0; phase ^= 1; }
+      }
     }
   } else if (warp == 1) {
-    // ===================== MMA issuer =====================
-    if (elect_one()) {
-      // instruction descriptor: D = f32 (1 << 4), A/B = f16 (0), majors, N >> 3, M >> 4
+    // ===================== MMA issuer (leader CTA only) =====================
+    if (rank == 0 && elect_one()) {
+      auto mma = [&](uint32_t d, uint64_t a, uint64_t b, uint32_t idesc, uint32_t acc) {
+        if constexpr (CTAS == 2) umma_f16_pair(d, a, b, idesc, acc);
+        else umma_f16(d, a, b, idesc, acc);
+      };
+      auto commit = [&](uint64_t* bar) {
+        if constexpr (CTAS == 2) umma_commit_pair(bar, 0x3);
+        else umma_commit(bar);
+      };
+      // instruction descriptor: D = f32 (1 << 4), A/B = f16 (0), majors, N >> 3, M >> 4 (pairs: M = 256, both CTAs' rows)
       constexpr uint32_t idesc = (1u << 4) | ((A_KM ? 0u : 1u) << 15) | ((B_KM ? 0u : 1u) << 16) |
-                                 ((uint32_t)(BN >> 3) << 17) | ((uint32_t)(HBM_ >> 4) << 24);
+                                 ((uint32_t)(BN >> 3) << 17) | ((uint32_t)((CTAS * HBM_) >> 4) << 24);
       // K-major: rows of TBK*2 bytes (128 B -> SWIZZLE_128B, 64 B -> SWIZZLE_64B), 8-row atoms.
       // MN-major: 64-element (128 B) rows along M|N, 8 k-rows per 1024 B atom (SBO), LBO = one 64-wide block.
       constexpr uint32_t k_sbo = 8 * TBK * 2, k_lt = (TBK == 64) ? 2 : 4;
@@ -187,19 +246,19 @@ gemm3x_f16_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constan
       constexpr uint32_t b_kstep = B_KM ? HUMMA_K * 2 : HUMMA_K * 128;
       int stage = 0; uint32_t phase = 0;
       uint32_t chunk_ctr = 0;
-      for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x) {
-        int mt, nt, sp; tile_coords(tile, mt, nt, sp);
+      for (int item = pair_id; item < total_items; item += num_pairs) {
+        int mt, nt, sp; tile_coords(item, mt, nt, sp);
         const int kb0 = sp * p.kb_per_split;
         const int kb1 = min(p.kb_total, kb0 + p.kb_per_split);
         for (int kc = kb0; kc < kb1; kc += p.kb_per_chunk, ++chunk_ctr) {
           const int as = chunk_ctr & 1;
-          mbar_wait(&tempty[as], ((chunk_ctr >> 1) & 1) ^ 1);
+          hwait(&tempty[as], ((chunk_ctr >> 1) & 1) ^ 1, kWaitTempty);
           tc_fence_after();
           const uint32_t d_tmem = tmem_base + (uint32_t)(as * BN);
           uint32_t accum = 0;
           const int kce = min(kb1, kc + p.kb_per_chunk);
           for (int kb = kc; kb < kce; ++kb) {
-            mbar_wait(&full[stage], phase);
+            hwait(&full[stage], phase, kWaitFull);
             tc_fence_after();
             const uint32_t sa = smem_u32(smem + stage * S::kStage);
             const uint32_t sb = sa + 2 * S::kAOp;
@@ -210,28 +269,29 @@ gemm3x_f16_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constan
               const uint64_t bh = make_desc(sb + ks * b_kstep, b_lbo, b_sbo, b_lt);
               const uint64_t bl = make_desc(sb + S::kBOp + ks * b_kstep, b_lbo, b_sbo, b_lt);
               if (!p.single) {
-                umma_f16(d_tmem, al, bh, idesc, accum);
-                umma_f16(d_tmem, ah, bl, idesc, 1);
+                mma(d_tmem, al, bh, idesc, accum);
+                mma(d_tmem, ah, bl, idesc, 1);
                 accum = 1;
               }
-              umma_f16(d_tmem, ah, bh, idesc, accum);
+              mma(d_tmem, ah, bh, idesc, accum);
               accum = 1;
             }
-            umma_commit(&empty[stage]);
+            commit(&empty[stage]);
             if (++stage == kStages) { stage = 0; phase ^= 1; }
           }
-          umma_commit(&tfull[as]);
+          commit(&tfull[as]);
         }
       }
     }
   } else if (warp >= 4) {
-    // ===================== accumulate + epilogue =====================
+    // ===================== accumulate + epilogue (both CTAs, each its own 128 rows) =====================
     constexpr int HALF = BN / 2;
     const int q = warp & 3;
     const int ch = (warp - 4) >> 2;
+    const uint32_t tempty_leader = CTAS == 2 ? mapa_shared(tempty, 0) : 0;
     uint32_t chunk_ctr = 0;
-    for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x) {
-      int mt, nt, sp; tile_coords(tile, mt, nt, sp);
+    for (int item = pair_id; item < total_items; item += num_pairs) {
+      int mt, nt, sp; tile_coords(item, mt, nt, sp);
       const int kb0 = sp * p.kb_per_split;
       const int kb1 = min(p.kb_total, kb0 + p.kb_per_split);
       float acc[HALF];
@@ -239,6 +299,8 @@ gemm3x_f16_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constan
       for (int e = 0; e < HALF; ++e) acc[e] = 0.f;
       for (int kc = kb0; kc < kb1; kc += p.kb_per_chunk, ++chunk_ctr) {
         const int as = chunk_ctr & 1;
+        // plain bounded wait: a report call here costs the register-bound epilogue spills, and a lost tfull in either CTA
+        // starves the leader's tempty wait, which names it
         mbar_wait(&tfull[as], (chunk_ctr >> 1) & 1);
         tc_fence_after();
         const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(as * BN + ch * HALF);
@@ -254,7 +316,10 @@ gemm3x_f16_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constan
         }
         tc_fence_before();
         __syncwarp();
-        if (lane == 0) mbar_arrive(&tempty[as]);
+        if (lane == 0) {
+          if constexpr (CTAS == 2) mbar_arrive_cluster(tempty_leader + as * (uint32_t)sizeof(uint64_t));
+          else mbar_arrive(&tempty[as]);
+        }
       }
       const int row = mt * HBM_ + q * 32 + lane;
       const int col0 = nt * BN + ch * HALF;
@@ -381,10 +446,18 @@ gemm3x_f16_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constan
 
   if (warp >= 4 && lane == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");   // this lane's bulk stores have landed
   tc_fence_before();
-  __syncthreads();
-  if (warp == 2) {
-    tc_fence_after();
-    tmem_dealloc(tmem_base, kTmemCols);
+  if constexpr (CTAS == 2) {
+    cluster_sync();           // both CTAs have drained their TMEM and sent their last arrivals to the leader
+    if (warp == 2) {
+      tc_fence_after();
+      tmem_dealloc_pair(tmem_base, kTmemCols);
+    }
+  } else {
+    __syncthreads();
+    if (warp == 2) {
+      tc_fence_after();
+      tmem_dealloc(tmem_base, kTmemCols);
+    }
   }
 }
 
@@ -400,17 +473,62 @@ __global__ void f16_splitk_reduce_kernel(const float* __restrict__ ws, int split
   C[(size_t)m * ldc + n] = s * f;
 }
 
+// CTA pairs of this instantiation that fit on the device at once (how the GPCs divide the SMs decides it, not just
+// sm_count / 2); sets the kernel's shared-memory limit on the way.  Per device; 0 when the query fails.
 template <int BN, int TBK, bool A_KM, bool B_KM>
+int resident_pairs_h() {
+  constexpr int CTAS = 2;
+  static int cached[64] = {0};
+  int dev = 0;
+  if (cudaGetDevice(&dev) != cudaSuccess) return 0;
+  if (dev >= 0 && dev < 64 && cached[dev]) return cached[dev];
+  using S = HSmem<BN, TBK, A_KM, B_KM, CTAS>;
+  auto kern = gemm3x_f16_kernel<BN, TBK, A_KM, B_KM, CTAS>;
+  if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, S::kTotal) != cudaSuccess) return 0;
+  cudaLaunchAttribute attr;
+  attr.id = cudaLaunchAttributeClusterDimension;
+  attr.val.clusterDim.x = CTAS; attr.val.clusterDim.y = 1; attr.val.clusterDim.z = 1;
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = dim3(CTAS * sm_count());
+  cfg.blockDim = dim3(kHThreads);
+  cfg.dynamicSmemBytes = S::kTotal;
+  cfg.attrs = &attr;
+  cfg.numAttrs = 1;
+  int n = 0;
+  if (cudaOccupancyMaxActiveClusters(&n, kern, &cfg) != cudaSuccess || n <= 0) return 0;
+  if (dev >= 0 && dev < 64) cached[dev] = n;
+  return n;
+}
+
+template <int BN, int TBK, bool A_KM, bool B_KM, int CTAS>
 int launch_h(const CUtensorMap& tAh, const CUtensorMap& tAl, const CUtensorMap& tBh, const CUtensorMap& tBl,
              const CUtensorMap& tC, const HParams& p, cudaStream_t st) {
-  using S = HSmem<BN, TBK, A_KM, B_KM>;
-  auto kern = gemm3x_f16_kernel<BN, TBK, A_KM, B_KM>;
-  SPOTV2_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, S::kTotal));
-  int grid = sm_count();
-  const int total = p.m_tiles * p.n_tiles * p.splits;
-  if (grid > total) grid = total;
-  kern<<<grid, kHThreads, S::kTotal, st>>>(tAh, tAl, tBh, tBl, tC, p);
-  SPOTV2_CUDA_OK(cudaGetLastError());
+  using S = HSmem<BN, TBK, A_KM, B_KM, CTAS>;
+  auto kern = gemm3x_f16_kernel<BN, TBK, A_KM, B_KM, CTAS>;
+  int slots;                 // resident work-item slots: CTA pairs or single CTAs
+  if constexpr (CTAS == 2) {
+    slots = resident_pairs_h<BN, TBK, A_KM, B_KM>();
+    if (slots <= 0) {
+      cudaGetLastError();
+      return fail(SPOTV2_ERR_CUDA, "gemm3x_f16: no cluster of two CTAs with %d B of shared memory fits on this device", S::kTotal);
+    }
+  } else {
+    SPOTV2_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, S::kTotal));
+    slots = sm_count();
+  }
+  const int total = p.pm_tiles * p.n_tiles * p.splits;
+  if (slots > total) slots = total;
+  cudaLaunchAttribute attr;
+  attr.id = cudaLaunchAttributeClusterDimension;
+  attr.val.clusterDim.x = CTAS; attr.val.clusterDim.y = 1; attr.val.clusterDim.z = 1;
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = dim3(CTAS * slots);
+  cfg.blockDim = dim3(kHThreads);
+  cfg.dynamicSmemBytes = S::kTotal;
+  cfg.stream = st;
+  cfg.attrs = &attr;
+  cfg.numAttrs = CTAS == 2 ? 1 : 0;
+  SPOTV2_CUDA_OK(cudaLaunchKernelEx(&cfg, kern, tAh, tAl, tBh, tBl, tC, p));
   return SPOTV2_OK;
 }
 
@@ -725,7 +843,18 @@ int split_f16(const float* src, int rows, int cols, size_t ld, int split_dim, in
   return SPOTV2_OK;
 }
 
+// The weight-gradient product's kernel (MN-major x MN-major, 256 x 256 x 32 pair tiles) sizes the split-K factor.
+int gemm3x_f16_resident_pairs() {
+  const int n = resident_pairs_h<256, 32, false, false>();
+  if (n > 0) return n;
+  cudaGetLastError();
+  return sm_count() / 2;      // no device: the pairs of a B200's 148 SMs
+}
+
 // C[M,N] = A . B^T with operands pre-split into scaled fp16 pairs.  bn: 256 -> TBK 64, 256 + 16 -> TBK 32.
+// The 3-product (fp32-accurate) class runs on pair tiles; the single-product half-precision class keeps 1-CTA tiles: with
+// a third of the MMA work per k-block it is bound by its operand pipeline, which the cross-CTA hand-offs lengthen (config C
+// half mode on a B200: forward 2.17 -> 2.51 ms, dW 1.73 -> 2.29, dX 1.09 -> 1.34 on pair tiles; profiles/r3a_pair_gemm_ab.txt).
 int gemm3x_f16(bool a_kc, bool b_kc, int M, int N, int K, const F16Operand& A, const F16Operand& B, float* C, int ldc,
                int splits, int bn, int kb_per_chunk, void* ws, size_t ws_bytes, cudaStream_t st, float* amax_out,
                int amax_cols, bool single, const PairOut* pair) {
@@ -736,7 +865,8 @@ int gemm3x_f16(bool a_kc, bool b_kc, int M, int N, int K, const F16Operand& A, c
     return fail(SPOTV2_ERR_INVALID_ARG, "fp16 GEMM operands need 16-byte aligned bases and leading dimensions % 8 == 0");
   HParams p;
   p.M = M; p.N = N; p.K = K;
-  p.m_tiles = (M + HBM_ - 1) / HBM_;
+  const int ctas = single ? 1 : 2;
+  p.pm_tiles = (M + ctas * HBM_ - 1) / (ctas * HBM_);
   p.n_tiles = (N + bn - 1) / bn;
   p.kb_total = (K + TBK - 1) / TBK;
   if (splits < 1) splits = 1;
@@ -801,8 +931,8 @@ int gemm3x_f16(bool a_kc, bool b_kc, int M, int N, int K, const F16Operand& A, c
       return rc;
     p.tma_store = 1;
   }
-  // K-major operand: tensor [rows = M|N, cols = K], box TBK(k) x tile rows (rows of 128 or 64 bytes).
-  // MN-major operand: tensor [rows = K, cols = M|N], box 64(m|n) x TBK(k); one box per 64-wide block.
+  // K-major operand: tensor [rows = M|N, cols = K], box TBK(k) x this CTA's tile rows (128 of A, bn / ctas of B; rows of
+  // 128 or 64 bytes).  MN-major operand: tensor [rows = K, cols = M|N], box 64(m|n) x TBK(k); one box per 64-wide block.
   const CUtensorMapSwizzle kSw = TBK == 64 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B;
   const CUtensorMapSwizzle mnSw = CU_TENSOR_MAP_SWIZZLE_128B;
   if (a_kc) {
@@ -813,13 +943,14 @@ int gemm3x_f16(bool a_kc, bool b_kc, int M, int N, int K, const F16Operand& A, c
     if ((rc = make_tmap_f16(&tAl, A.lo, K, M, A.ld, 64, TBK, mnSw))) return rc;
   }
   if (b_kc) {
-    if ((rc = make_tmap_f16(&tBh, B.hi, N, K, B.ld, TBK, bn, kSw))) return rc;
-    if ((rc = make_tmap_f16(&tBl, B.lo, N, K, B.ld, TBK, bn, kSw))) return rc;
+    if ((rc = make_tmap_f16(&tBh, B.hi, N, K, B.ld, TBK, bn / ctas, kSw))) return rc;
+    if ((rc = make_tmap_f16(&tBl, B.lo, N, K, B.ld, TBK, bn / ctas, kSw))) return rc;
   } else {
     if ((rc = make_tmap_f16(&tBh, B.hi, K, N, B.ld, 64, TBK, mnSw))) return rc;
     if ((rc = make_tmap_f16(&tBl, B.lo, K, N, B.ld, 64, TBK, mnSw))) return rc;
   }
-#define SPOTV2_H(BN_, TBK_, AK, BK_) rc = launch_h<BN_, TBK_, AK, BK_>(tAh, tAl, tBh, tBl, tC, p, st)
+#define SPOTV2_H(BN_, TBK_, AK, BK_) \
+  rc = single ? launch_h<BN_, TBK_, AK, BK_, 1>(tAh, tAl, tBh, tBl, tC, p, st) : launch_h<BN_, TBK_, AK, BK_, 2>(tAh, tAl, tBh, tBl, tC, p, st)
 #define SPOTV2_H_MAJ(BN_, TBK_)                            \
   do {                                                     \
     if (a_kc && b_kc) SPOTV2_H(BN_, TBK_, true, true);     \

@@ -57,7 +57,7 @@ extern "C" int spotv2_gat_workspace_bytes(const spotv2_gat_desc* d, size_t* proj
   if (proj_fwd) *proj_fwd = 1024 + (tc ? pair_bytes(s.rows, s.ldf16) + pair_bytes(s.n_aug, s.ldf16) : 0);
   if (attn_bwd) *attn_bwd = attn_bwd_ws_bytes(d) + 256;
   if (proj_bwd) {
-    const int splits = weight_grad_splits(s.rows, s.n_aug, s.F);
+    const int splits = weight_grad_splits(s.rows, s.n_aug, s.F, !single_product(d));
     size_t w = round_up((size_t)splits * s.n_aug * s.F * sizeof(float), 256) + 1024;
     if (tc) w += pair_bytes(s.rows, s.ldp16) + pair_bytes(s.rows, s.ldf16) + pair_bytes(s.n_aug, s.ldf16);
     *proj_bwd = w;
@@ -157,7 +157,7 @@ extern "C" int spotv2_proj_bwd_weight(const spotv2_gat_desc* d, const float* x, 
                  "proj_bwd_weight: p_format 1 takes x and dP as pairs");
   const ProjShape s = shape_of(d);
   cudaStream_t st = as_stream(stream);
-  const int splits = weight_grad_splits(s.rows, s.n_aug, s.F);
+  const int splits = weight_grad_splits(s.rows, s.n_aug, s.F, !single_product(d));
   if (!use_tc(d)) {
     SPOTV2_REQUIRE(dP_aug, "proj_bwd_weight: the CUDA-core path takes the fp32 dP_aug");
     return sgemm_simt(false, false, s.n_aug, s.F, s.rows, dP_aug, s.ldp, x, s.F, dW_aug, s.F, splits, ws, ws_bytes, st);

@@ -35,6 +35,52 @@ __device__ __forceinline__ void umma_f16(uint32_t tmem_d, uint64_t adesc, uint64
 __device__ __forceinline__ void umma_commit(uint64_t* bar) {   // implies tcgen05.fence::before_thread_sync
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
+
+// ---- CTA pairs (cluster of 2, cta_group::2): one MMA of M = 256 spans both CTAs' shared memory and TMEM -------------
+__device__ __forceinline__ uint32_t cluster_ctarank() {
+  uint32_t r;
+  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
+  return r;
+}
+// all threads of both CTAs; release/acquire orders barrier initialisation and the last remote arrivals
+__device__ __forceinline__ void cluster_sync() {
+  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
+}
+// shared::cluster address of the same shared-memory object in CTA `rank` of the cluster
+__device__ __forceinline__ uint32_t mapa_shared(const void* p, uint32_t rank) {
+  uint32_t r;
+  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(smem_u32(p)), "r"(rank));
+  return r;
+}
+__device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_addr) {
+  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
+}
+// one warp of EACH CTA of the pair: every CTA gets the same columns of its own TMEM
+__device__ __forceinline__ void tmem_alloc_pair(uint32_t* smem_dst, uint32_t ncols) {
+  asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(smem_dst)), "r"(ncols)
+               : "memory");
+  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
+}
+__device__ __forceinline__ void tmem_dealloc_pair(uint32_t taddr, uint32_t ncols) {
+  asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
+}
+// issued by the leader CTA only: A rows 0-127 from the leader's shared memory, 128-255 from the peer's (same offsets),
+// B columns likewise split in halves; D rows land in the TMEM of the CTA that supplied them
+__device__ __forceinline__ void umma_f16_pair(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accum) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(tmem_d),
+      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accum)
+      : "memory");
+}
+// arrive on the barrier at this shared-memory offset in every CTA of cta_mask once the leader's MMAs have completed
+__device__ __forceinline__ void umma_commit_pair(uint64_t* bar, uint16_t cta_mask) {
+  asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
+                   smem_u32(bar)),
+               "h"(cta_mask)
+               : "memory");
+}
+
 __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&r)[32]) {
   asm volatile(
       "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,%21,"

@@ -143,6 +143,15 @@ __device__ __forceinline__ void tma_load_2d(void* smem_dst, const CUtensorMap* t
       "l"(tm), "r"(smem_u32(bar)), "r"(c0), "r"(c1)
       : "memory");
 }
+// pair form: the bytes land in this CTA's shared memory and complete on an mbarrier of either CTA of the pair
+// (bar_cluster: a shared::cluster address, mapa_shared)
+__device__ __forceinline__ void tma_load_2d_pair(void* smem_dst, const CUtensorMap* tm, int c0, int c1, uint32_t bar_cluster) {
+  asm volatile(
+      "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];" ::"r"(
+          smem_u32(smem_dst)),
+      "l"(tm), "r"(bar_cluster), "r"(c0), "r"(c1)
+      : "memory");
+}
 __device__ __forceinline__ void tma_load_2d_hint(void* smem_dst, const CUtensorMap* tm, int c0, int c1, uint64_t* bar,
                                                  uint64_t hint) {
   asm volatile(
