@@ -192,8 +192,11 @@ int spotv2_gat_attn_fwd(const spotv2_gat_desc* d, const float* P_aug, const floa
 
 /* autograd of the above with the attention coefficients recomputed, not stored (edge_terms_or_null: what the
  * forward wrote, see spotv2_gat_edge_terms_bytes; null = recompute the edge terms from edge_rows as well).
- * edge_mode 1: edge_terms is required, d_edge_terms_or_null (same size and layout) receives the gradient w.r.t.
- * the edge terms and dv is left to spotv2_windows_dv.
+ * d_edge_terms_or_null (16-byte aligned, spotv2_gat_edge_terms_bytes, the edge-term tile layout) receives dz', the
+ * gradient w.r.t. the edge terms <e_ij, v_h> with the mean self-loop fill folded in (0 on the diagonal).
+ * edge_mode 1: edge_terms and d_edge_terms are required and dv is left to spotv2_windows_dv.  edge_mode 0: optional;
+ * dv is formed as usual, and spotv2_gat_edge_rows_grad turns d_edge_terms into the edge rows' gradient.  Null: none of
+ * that work is done.
  * dout [B*N, C or HC] -> dP_aug (dP | ds | dd), dv [H, Fe], dbias.  The gradient is emitted either as
  * fp32 dP_aug [B*N, ldp] (CUDA-core GEMM path) or, when dP_hi/dP_lo/dp_scale are given, directly as the
  * fp16 pair [B*N, ld16(HC+2H)] the tensor-core GEMMs consume (two scale groups: columns < HC from a
@@ -205,6 +208,17 @@ int spotv2_gat_attn_bwd(const spotv2_gat_desc* d, const float* P_aug, const floa
                         void* dP_hi_or_null, void* dP_lo_or_null, float* dp_scale_or_null,
                         float* dv_or_null, float* d_edge_terms_or_null, float* dbias_or_null, void* ws, size_t ws_bytes,
                         void* stream);
+
+/* Gradient w.r.t. the edge rows (edge_mode 0): d_edge_rows [B, R, Fe] in PyG row order,
+ *   d_edge_rows[b*R + r, :] = sum_h d_edge_terms[b][h][j][i] * v[h, :]   for table[r] = (i << 16) | j,
+ *   d_edge_rows[b*R + r, :] = 0                                           for SPOTV2_ROW_SKIP rows,
+ * from what spotv2_gat_attn_bwd / _attn_bwd_pair wrote to d_edge_terms_or_null, the row table and the folded edge
+ * vector v [H, Fe] the forward used (spotv2_gat_fold's output, after any per-feature scaling the caller applied).
+ * Stands in for the autograd of `lin_edge(edge_attr)` + `(e * att_edge).sum(-1)`, of the mean self-loop fill
+ * (add_self_loops(fill_value='mean')) and of remove_self_loops in [PyG] gat_conv.py.  d_edge_rows is 16-byte aligned;
+ * H <= 8, Fe <= 512; any N and row pitch. */
+int spotv2_gat_edge_rows_grad(const spotv2_gat_desc* d, const float* d_edge_terms, const int32_t* table, const float* v,
+                              float* d_edge_rows, void* stream);
 
 /* ---- p_format 1: the projection as an fp16 operand pair end to end ---------------------------------------------
  * Same operators as spotv2_proj_fwd / spotv2_gat_attn_fwd / spotv2_gat_attn_bwd ([PyG] F.linear, edge_update,

@@ -53,6 +53,7 @@ SIGNATURES = {
     "spotv2_gat_edge_terms_bytes": (C.c_int, [_DP, C.POINTER(_sz)]),
     "spotv2_gat_attn_fwd": (C.c_int, [_DP] + [_vp] * 9 + [_sz, _vp]),
     "spotv2_gat_attn_bwd": (C.c_int, [_DP] + [_vp] * 15 + [_sz, _vp]),
+    "spotv2_gat_edge_rows_grad": (C.c_int, [_DP] + [_vp] * 5),
     "spotv2_edge_terms_from_windows_workspace_bytes": (C.c_int, [_DP, C.POINTER(_sz)]),
     "spotv2_edge_terms_from_windows": (C.c_int, [_DP, _vp, _i32, _i32, _vp, _vp, _vp, _vp, _sz, _vp]),
     "spotv2_windows_dv_workspace_bytes": (C.c_int, [_DP, C.POINTER(_sz)]),

@@ -18,7 +18,7 @@ CSRC = PKG / "csrc"
 OBJ = PKG / "_build"
 LIB = PKG / "libspotv2_gat.so"
 
-SOURCES = ["api.cu", "fold.cu", "gemm_simt.cu", "gemm_tc.cu", "gemm_f16.cu", "proj.cu", "attn_fwd.cu", "attn_fwd16.cu", "attn_prep.cu", "attn_bwd.cu", "attn_bwd2.cu", "attn_bwd3.cu", "attn_large.cu", "windows.cu"]
+SOURCES = ["api.cu", "fold.cu", "gemm_simt.cu", "gemm_tc.cu", "gemm_f16.cu", "proj.cu", "attn_fwd.cu", "attn_fwd16.cu", "attn_prep.cu", "attn_bwd.cu", "attn_bwd2.cu", "attn_bwd3.cu", "attn_large.cu", "windows.cu", "edge_grad.cu"]
 # SPOTV2_BRINGUP=1 in the environment compiles the cycle counters of the attention kernels (tools/fwd16_waits.py,
 # tools/fwd_waits.py) and the GEMM's timing probe in; the product build carries none of them
 NVCC_FLAGS = (["-DSPOTV2_BRINGUP"] if os.environ.get("SPOTV2_BRINGUP") else []) + [

@@ -444,6 +444,14 @@ gat_attn_bwd_kernel(const AttnBwdArgs args, const BwdSmem sm) {
       }
     }
     __syncthreads();
+    if (p.dterms_out) {
+      // d(edge terms) out (the caller's d_edge_terms): dz' in the forward's edge-term layout [H][N][kEdgeTermNS]
+      float* dst = p.dterms_out + (size_t)b * H * N * kEdgeTermNS;
+      for (int idx = tid; idx < H * N * N; idx += kAttnThreads) {
+        const int hj = idx / N, i = idx - hj * N;
+        dst[hj * kEdgeTermNS + i] = D[hj * NS + i];
+      }
+    }
 
     lap(4);
     // ---- B4: dv += dz'^T . edge rows -------------------------------------------------------------
@@ -744,9 +752,10 @@ extern "C" int spotv2_gat_attn_bwd(const spotv2_gat_desc* d, const float* P_aug,
   a.p.drop = dropout_params(d);
   a.p.lg_tensor_cores = d->gemm_algo != 1;
   SPOTV2_REQUIRE(!edge_terms_or_null || aligned16(edge_terms_or_null), "attn_bwd: edge_terms must be 16-byte aligned");
+  SPOTV2_REQUIRE(!d_edge_terms_or_null || aligned16(d_edge_terms_or_null), "attn_bwd: d_edge_terms must be 16-byte aligned");
   a.p.edge_terms = d->Fe > 0 ? const_cast<float*>(edge_terms_or_null) : nullptr;
   a.p.terms_in = structured ? 1 : 0;
-  a.p.dterms_out = structured ? d_edge_terms_or_null : nullptr;
+  a.p.dterms_out = d->Fe > 0 ? d_edge_terms_or_null : nullptr;      // both edge modes (edge_mode 0: spotv2_gat_edge_rows_grad)
   a.p.P_aug = P_aug; a.p.edge_rows = edge_rows; a.p.table = table; a.p.v = v;
   a.p.bulk_ok = d->Fe > 0 && aligned16(edge_rows) && ((size_t)d->R * d->Fe) % 4 == 0;
   a.p.vec2_ok = (d->C % 2 == 0);
@@ -855,9 +864,10 @@ extern "C" int spotv2_gat_attn_bwd_pair(const spotv2_gat_desc* d, const void* P_
   a.p.drop = dropout_params(d);
   a.p.lg_tensor_cores = 1;
   SPOTV2_REQUIRE(!edge_terms_or_null || aligned16(edge_terms_or_null), "attn_bwd_pair: edge_terms must be 16-byte aligned");
+  SPOTV2_REQUIRE(!d_edge_terms_or_null || aligned16(d_edge_terms_or_null), "attn_bwd_pair: d_edge_terms must be 16-byte aligned");
   a.p.edge_terms = d->Fe > 0 ? const_cast<float*>(edge_terms_or_null) : nullptr;
   a.p.terms_in = structured ? 1 : 0;
-  a.p.dterms_out = structured ? d_edge_terms_or_null : nullptr;
+  a.p.dterms_out = d->Fe > 0 ? d_edge_terms_or_null : nullptr;      // both edge modes (edge_mode 0: spotv2_gat_edge_rows_grad)
   a.p.alpha_rec = attn_record_of(d);
   a.p.P_aug = nullptr; a.p.edge_rows = edge_rows; a.p.table = table; a.p.v = v;
   a.p.P_hi = static_cast<const __half*>(P_hi);

@@ -596,11 +596,13 @@ int attn_large_bwd(const spotv2_gat_desc* d, AttnBwdArgs& a, float* dv, float* d
     SPOTV2_CUDA_OK(cudaGetLastError());
   }
   if (p.Fe > 0 && p.dterms_out) {
-    // structured source: the gradient w.r.t. the edge terms leaves as w[b][h][j][i] = dz + fill[b][h][i] (0 on the
-    // diagonal); dv is formed from the windows by spotv2_windows_dv
+    // the gradient w.r.t. the edge terms leaves as w[b][h][j][i] = dz + fill[b][h][i] (0 on the diagonal).  Structured
+    // source: dv is formed from the windows by spotv2_windows_dv; edge rows: dv below, and the caller expands w into
+    // the edge rows' gradient (spotv2_gat_edge_rows_grad)
     lg_dterms_kernel<<<(unsigned)((size_t)p.B * p.H * p.N), 128, 0, st>>>(dA, fill, p.dterms_out, p.N);
     SPOTV2_CUDA_OK(cudaGetLastError());
-  } else if (p.Fe > 0 && dv) {
+  }
+  if (p.Fe > 0 && dv && !p.terms_in) {
     LgDvArgs v;
     v.rg = lg_ring(p, pl);
     v.table = p.table; v.dZ = dA; v.fill = fill; v.part = dv_part; v.N = p.N; v.H = p.H;

@@ -304,8 +304,8 @@ class _GatLayerFn(torch.autograd.Function):
         lib = _lib.load()
         x, ea, W, a_src, a_dst, W_e, a_edge, W_aug, v, P_aug, x16, x_blk, p_amax, et, sd32 = ctx.saved_tensors
         desc, topo, Fe = ctx.desc, ctx.topo, ctx.Fe
-        if ctx.needs_input_grad[1]:
-            raise SpotV2Error("gradient w.r.t. edge_attr is not provided (the reference never needs it)")
+        # d edge_attr: the attention backward hands out dz' (gradient w.r.t. the edge terms), expanded below into rows
+        want_dea = bool(ctx.needs_input_grad[1]) and ea is not None
         dev = x.device
         st = stream_ptr(dev)
         H, Cc = desc.H, desc.C
@@ -329,7 +329,8 @@ class _GatLayerFn(torch.autograd.Function):
         dv = torch.empty(H, Fe, device=dev, dtype=torch.float32) if Fe else None
         dbias = torch.empty(dout.shape[1], device=dev, dtype=torch.float32) if ctx.has_bias else None
         win = ctx.windows
-        d_et = torch.empty_like(et) if win is not None else None     # structured source: d(edge terms) out, dv from the windows
+        # d(edge terms) out: structured source (dv from the windows), or edge_attr.grad wanted (dv as usual)
+        d_et = torch.empty_like(et) if (win is not None or want_dea) else None
         if pair:
             check(lib.spotv2_gat_attn_bwd_pair(C.byref(desc), ptr(P_aug[0]), ptr(P_aug[1]) if P_aug.shape[0] > 1 else None, ptr(p_amax),
                                                ptr(sd32), ptr(ea), ptr(et), ptr(topo.table) if (Fe and win is None) else None, ptr(v),
@@ -346,16 +347,31 @@ class _GatLayerFn(torch.autograd.Function):
             ws_dv = torch.empty(wsz.value, device=dev, dtype=torch.uint8)
             check(lib.spotv2_windows_dv(C.byref(desc), ptr(win.volvol), win.volvol.shape[0], win.L, ptr(win.t0), ptr(d_et),
                                         ptr(dv), ptr(ws_dv), wsz.value, st), "spotv2_windows_dv")
+        d_ea = None
+        if want_dea:
+            # d edge_attr[e, :] = sum_h dz'[e, h] v'_h (v' = the folded, scaled edge vector the forward used); input self
+            # loops (rows PyG's remove_self_loops drops) get zero rows
+            d_ea = torch.empty_like(ea)
+            check(lib.spotv2_gat_edge_rows_grad(C.byref(desc), ptr(d_et), ptr(topo.table), ptr(v), ptr(d_ea), st),
+                  "spotv2_gat_edge_rows_grad")
+        d_scale = d_mean = None
         if ctx.edge_scale is not None:
             # the layer saw e_hat = (e - mean) * scale through v' = scale * v and the per-head logit shift -<mean, v'> on the
             # d columns.  d/dv = scale * (sum dz' e - mean * sum of ALL dz of the head): the kernels formed the first sum (dv),
             # the second is the column sum of the dd block (LeakyReLU keeps a softmax row's dz from summing to zero).
+            T = None
             if ctx.edge_mean is not None:            # (p_format 0 by construction: see _forward)
                 if tc:
                     T = ((dP16[0][:, HC + H:HC + 2 * H].float() + dP16[1][:, HC + H:HC + 2 * H].float()).sum(0) * dp_blk[3])
                 else:
                     T = dP_aug[:, HC + H:HC + 2 * H].sum(0)
                 dv.sub_(T.view(H, 1) * ctx.edge_mean.view(1, Fe))
+            # batch statistics that depend on edge_attr (training mode with edge_attr.requires_grad): with g_h = dv here,
+            # dL/dscale = sum_h v_h * g_h (v unscaled) and dL/dmean = -sum_h T_h v'_h
+            if ctx.needs_input_grad[19]:
+                d_scale = (v * dv).sum(0) / ctx.edge_scale
+            if ctx.needs_input_grad[20] and T is not None:
+                d_mean = -(T.view(H, 1) * v).sum(0)
             dv.mul_(ctx.edge_scale.view(1, Fe))
         if _KEEP is not None:                      # bring-up aid (tools/): the kernel-level gradient of the projection
             _KEEP.update(dP16=dP16, dp_blk=dp_blk, dP_aug=dP_aug, n_aug=lib.spotv2_gat_n_aug(C.byref(desc)),
@@ -381,7 +397,7 @@ class _GatLayerFn(torch.autograd.Function):
                                     ptr(da_dst), ptr(dW_e), ptr(da_edge), st), "spotv2_gat_unfold")
         if not Fe and W_e is not None:          # layer has lin_edge but was called with edge_attr=None
             dW_e, da_edge = torch.zeros_like(W_e), torch.zeros_like(a_edge)
-        return (dx, None, dW, da_src, da_dst, dW_e, da_edge, dbias) + (None,) * 13
+        return (dx, d_ea, dW, da_src, da_dst, dW_e, da_edge, dbias) + (None,) * 11 + (d_scale, d_mean)
 
 
 # --------------------------------------------------------------------------- module

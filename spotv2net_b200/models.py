@@ -15,6 +15,7 @@ import torch.distributed as dist
 import torch.nn.functional as F
 from torch import nn
 
+from ._lib import SpotV2Error
 from .gat_conv import GATConv, topology_from_edge_index
 
 
@@ -86,14 +87,25 @@ class GATModel(nn.Module):
             if edge_attr is not None:
                 tag = getattr(edge_attr, "_spot_stats_src", None)      # attached by WindowDataset.collate to this very tensor
                 src = tag[0] if (tag is not None and tag[1] == edge_attr._version) else None
+                # the statistics are functions of edge_attr: when it wants a gradient they are formed from edge_attr itself
+                # (the window-stack shortcut has the same value but no autograd graph back to the edge rows)
+                if edge_attr.requires_grad:
+                    src = None
             if src is not None:
                 se, qe, ne = src.edge_stats()                          # [Fe] float64 sums over the batch's real edges
             else:
                 if edge_attr is None:
                     raise ValueError("standardize=True needs edge_attr or a WindowDataset batch")
                 ne = float(edge_attr.shape[0])
-                se, qe = edge_attr.sum(0, dtype=torch.float64), (edge_attr * edge_attr).sum(0, dtype=torch.float64)
+                if edge_attr.requires_grad:          # squares in fp64 as well: the shortcut's accuracy, and its gradient
+                    e64 = edge_attr.double()
+                    se, qe = e64.sum(0), (e64 * e64).sum(0)
+                else:
+                    se, qe = edge_attr.sum(0, dtype=torch.float64), (edge_attr * edge_attr).sum(0, dtype=torch.float64)
             if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
+                if edge_attr is not None and edge_attr.requires_grad:
+                    raise SpotV2Error("standardize=True in training mode with edge_attr.requires_grad under torch.distributed: "
+                                      "the all-reduce of the batch statistics is not differentiable")
                 buf = torch.cat([sx, qx, se, qe, torch.tensor([nx, ne], device=x.device, dtype=torch.float64)])
                 dist.all_reduce(buf)
                 F_, Fe_ = sx.numel(), se.numel()
