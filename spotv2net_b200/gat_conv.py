@@ -459,8 +459,10 @@ class GATConv(nn.Module):
             self.register_parameter("bias", None)
         self.nodes_per_graph: Optional[int] = None     # optional hint; inferred from edge_index otherwise
         # "fp32" (default): every product fp32-accurate (1e-5 parity).  "half": the projection GEMMs issue one fp16
-        # tensor-core product with fp32 accumulation (BASELINE config C's reduced-precision variant, ~1e-3);
-        # the attention kernels stay fp32-accurate either way.  Not a PyG ctor argument: set the attribute.
+        # tensor-core product with fp32 accumulation (BASELINE config C's reduced-precision variant, ~1e-3).  With the pair
+        # format (p_format 1) P, alpha, dout and dP also travel as single fp16 planes through the attention kernels; with
+        # p_format 0 the attention kernels stay fp32-accurate and the GEMMs read the fp16 hi plane of dP (DESIGN §6).  Not a PyG ctor
+        # argument: set the attribute.
         self.precision = "fp32"
         self.reset_parameters()
 

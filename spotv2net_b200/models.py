@@ -65,7 +65,8 @@ class GATModel(nn.Module):
             sys.exit()
 
     def set_precision(self, precision: str):
-        """"fp32" (default, 1e-5 parity) or "half" (one fp16 tensor-core product in every layer's projections)."""
+        """"fp32" (default, 1e-5 parity) or "half" (every layer's half-precision class: one fp16 tensor-core product in the
+        projections and, where a layer takes the pair format, P, alpha, dout and dP as single fp16 planes; see GATConv)."""
         for layer in self.gat_layers:
             layer.precision = precision
         return self
