@@ -653,27 +653,103 @@ int reduce_partials(const float* part, int nparts, int len, float* out, cudaStre
   return SPOTV2_OK;
 }
 
-size_t attn_bwd_partials_bytes(const spotv2_gat_desc* d) {
-  // per-CTA partials of dv [H, Fe] and dbias [C or HC]; at most 2 CTAs per SM
-  const size_t ctas = 2 * (size_t)sm_count();
-  const size_t ldo = d->concat ? (size_t)d->H * d->C : (size_t)d->C;
-  const size_t legacy = round_up(ctas * ((size_t)d->H * d->Fe + ldo) * sizeof(float), 256);
-  size_t piped = attn_bwd2_partials_bytes(d);
-  if (attn_bwd3_partials_bytes(d) > piped) piped = attn_bwd3_partials_bytes(d);
-  return legacy > piped ? legacy : piped;
-}
-// p_format 1: dout's operand pair (2 planes [B*N, ld16(ldo)]) | unit scales | the prepass's dbias partials
-static size_t attn_bwd_pair_extra_bytes(const spotv2_gat_desc* d) {
-  if (d->p_format != 1) return 0;
+// Workspace of the N <= 32 backward (byte offsets): per-CTA partials of dv and dbias (the most any kernel needs) | ds,dd fp32
+// [B*N, 2H] | scale blocks max|dout|, ds|dd, max|P| (256 B) | p_format 1: dout's pair (two planes [B*N, ld16(ldo)]) | its unit
+// scales [B * upg] | the prepass's dbias partials
+struct BwdWorkspace { size_t dsd, blocks, dout_pair, plane, unit_scales, dbias_part, total; };
+
+static BwdWorkspace bwd_workspace_of(const spotv2_gat_desc* d) {
   const size_t rows = (size_t)d->B * d->N, ldo = d->concat ? (size_t)d->H * d->C : (size_t)d->C;
-  const int upg = d->concat ? d->H : 1;
-  return 2 * round_up(rows * ld16_of((int)ldo) * 2, 256) + round_up((size_t)d->B * upg * sizeof(float), 256) +
-         round_up((size_t)dout_pair_grid(d->B * upg, upg) * ldo * sizeof(float), 256);
+  BwdWorkspace w{};
+  const size_t serial_partials = round_up(2 * (size_t)sm_count() * ((size_t)d->H * d->Fe + ldo) * sizeof(float), 256);
+  w.dsd = std::max({serial_partials, attn_bwd2_partials_bytes(d), attn_bwd3_partials_bytes(d)});
+  w.blocks = w.dsd + round_up(rows * 2 * d->H * sizeof(float), 256);
+  w.total = w.blocks + 256;
+  if (d->p_format == 1) {
+    const int upg = d->concat ? d->H : 1;
+    w.plane = round_up(rows * ld16_of((int)ldo) * 2, 256);
+    w.dout_pair = w.total;
+    w.unit_scales = w.dout_pair + 2 * w.plane;
+    w.dbias_part = w.unit_scales + round_up((size_t)d->B * upg * sizeof(float), 256);
+    w.total = w.dbias_part + round_up((size_t)dout_pair_grid(d->B * upg, upg) * ldo * sizeof(float), 256);
+  }
+  return w;
 }
+
 size_t attn_bwd_ws_bytes(const spotv2_gat_desc* d) {
-  if (attn_large_applies(d)) return attn_large_bwd_ws_bytes(d);
-  // partials | ds,dd in fp32 [B*N, 2H] | two scale blocks | (p_format 1) the dout pair and its by-products
-  return attn_bwd_partials_bytes(d) + round_up((size_t)d->B * d->N * 2 * d->H * sizeof(float), 256) + 256 + attn_bwd_pair_extra_bytes(d);
+  return attn_large_applies(d) ? attn_large_bwd_ws_bytes(d) : bwd_workspace_of(d).total;
+}
+
+int check_attn_inputs(const char* who, const spotv2_gat_desc* d, std::initializer_list<ArgCheck> own_args,
+                      std::initializer_list<ArgCheck> own_layout, const AttnEdgeArgs& e) {
+  for (const ArgCheck& c : own_args)
+    if (!c.ok) return fail(c.st, "%s", c.msg);
+  const bool structured = d->edge_mode == 1 && d->Fe > 0;
+  if (d->Fe > 0 && !structured && !(e.rows && e.table && e.v))
+    return fail(SPOTV2_ERR_INVALID_ARG, "%s: edge_rows, table and v are required when Fe > 0", who);
+  if (structured && !e.backward && !e.terms)
+    return fail(SPOTV2_ERR_INVALID_ARG, "%s: edge_mode 1 needs edge_terms (spotv2_edge_terms_from_windows)", who);
+  if (structured && e.backward && !(e.terms && e.dterms && aligned16(e.dterms)))
+    return fail(SPOTV2_ERR_INVALID_ARG, "%s: edge_mode 1 needs edge_terms and a 16-byte aligned d_edge_terms buffer", who);
+  for (const ArgCheck& c : own_layout)
+    if (!c.ok) return fail(c.st, "%s", c.msg);
+  if (d->H > kMaxHeads) return fail(SPOTV2_ERR_UNSUPPORTED, "H=%d > %d", d->H, kMaxHeads);
+  if (d->Fe > kMaxFe) return fail(SPOTV2_ERR_UNSUPPORTED, "Fe=%d > %d", d->Fe, kMaxFe);
+  if (!aligned16(e.terms)) return fail(SPOTV2_ERR_INVALID_ARG, "%s: edge_terms must be 16-byte aligned", who);
+  if (!aligned16(e.dterms)) return fail(SPOTV2_ERR_INVALID_ARG, "%s: d_edge_terms must be 16-byte aligned", who);
+  return SPOTV2_OK;
+}
+
+AttnParams attn_params_of(const spotv2_gat_desc* d, const AttnEdgeArgs& e) {
+  AttnParams p{};
+  p.B = d->B; p.N = d->N; p.F = d->F; p.Fe = d->Fe; p.H = d->H; p.C = d->C;
+  p.R = d->R; p.concat = d->concat; p.ldp = d->ldp;
+  p.ldo = d->concat ? d->H * d->C : d->C;
+  p.slope = d->negative_slope;
+  p.drop = dropout_params(d);
+  p.lg_tensor_cores = d->gemm_algo != 1;
+  p.edge_rows = e.rows; p.table = e.table; p.v = e.v;
+  p.bulk_ok = d->Fe > 0 && aligned16(e.rows) && ((size_t)d->R * d->Fe) % 4 == 0;
+  p.vec2_ok = (d->C % 2 == 0);
+  p.edge_terms = d->Fe > 0 ? const_cast<float*>(e.terms) : nullptr;
+  p.terms_in = (d->edge_mode == 1 && d->Fe > 0) ? 1 : 0;
+  p.dterms_out = d->Fe > 0 ? e.dterms : nullptr;      // both edge modes (edge_mode 0: spotv2_gat_edge_rows_grad)
+  if (d->p_format == 1) {
+    p.hp = head_pitch_of(d);
+    p.ldp16 = ld16_of(n_aug_of(d));
+    p.alpha_rec = attn_record_of(d);
+  }
+  return p;
+}
+
+enum class BwdKernel { kLarge, kTcgen05, kPipelined, kPhaseSerial };
+
+// N > 32: the large-universe path.  Else attn_bwd_algo 0 = the pipelined kernel (attn_bwd2.cu) when its shared-memory plan
+// fits, else the phase-serial one of this file; 1 = phase-serial; 2 = pipelined or error; 3 = tcgen05 (attn_bwd3.cu) or error,
+// opt-in because on a B200 the shared-memory port bounds it below the pipelined kernel (DESIGN.md section 6).
+static int choose_bwd_kernel(const spotv2_gat_desc* d, const AttnParams& p, BwdKernel* k) {
+  *k = attn_large_applies(d) ? BwdKernel::kLarge : d->attn_bwd_algo == 3 ? BwdKernel::kTcgen05 : BwdKernel::kPipelined;
+  if (*k == BwdKernel::kTcgen05 && !attn_bwd3_applies(p))
+    return fail(SPOTV2_ERR_UNSUPPORTED, "attn_bwd: the tcgen05 kernel covers head-mean layers with N <= 31, C %% 4 == 0, even Fe <= 128 "
+                                        "and the forward's edge terms");
+  if (*k != BwdKernel::kPipelined) return SPOTV2_OK;
+  if (p.terms_in && !attn_bwd2_fits(p))
+    return fail(SPOTV2_ERR_UNSUPPORTED, "attn_bwd: edge_mode 1 needs the pipelined kernel, whose shared-memory plan does not fit this shape");
+  if (d->attn_bwd_algo == 1 || (d->attn_bwd_algo != 2 && !attn_bwd2_fits(p))) *k = BwdKernel::kPhaseSerial;
+  return SPOTV2_OK;
+}
+
+// |dP_h[j,c]| = |g sum_i alpha_h[i,j] dO[i,c]| <= g N max|dout|  (g = 1/H for the head mean); attention dropout scales the
+// kept coefficients by 1/(1-p), and the bound grows with it
+static float dp_bound(const AttnParams& p) { return (float)p.N * (p.concat ? 1.f : 1.f / (float)p.H) * p.drop.scale; }
+
+// ds | dd (a.dsd) -> columns [hc, hc + 2H) of the dP operand pair (hc: first s|d column of the pair's layout)
+static int split_dsd(const AttnBwdArgs& a, int hc, cudaStream_t st) {
+  const size_t total = (size_t)a.p.B * a.p.N * 2 * a.p.H;
+  split_dsd_kernel<<<(unsigned)std::min<size_t>((total + 255) / 256, (size_t)8 * 148), 256, 0, st>>>(
+      a.dsd, total, 2 * a.p.H, a.dP_hi16 + hc, a.dP_lo16 ? a.dP_lo16 + hc : nullptr, a.ldp16, a.dp_blk);
+  SPOTV2_CUDA_OK(cudaGetLastError());
+  return SPOTV2_OK;
 }
 
 template <int NPAIRS>
@@ -728,54 +804,41 @@ extern "C" int spotv2_gat_attn_bwd(const spotv2_gat_desc* d, const float* P_aug,
                                    float* dp_scale_or_null, float* dv_or_null, float* d_edge_terms_or_null,
                                    float* dbias_or_null, void* ws, size_t ws_bytes, void* stream) {
   if (int rc = check_desc(d)) return rc;
-  SPOTV2_REQUIRE(P_aug && dout, "attn_bwd: P_aug and dout must be non-null");
-  const bool f16 = dP_hi_or_null != nullptr;
-  SPOTV2_REQUIRE(f16 || dP_aug_or_null, "attn_bwd: give dP_aug (fp32) or dP_hi/dP_lo/dp_scale (fp16 pairs)");
-  SPOTV2_REQUIRE(!f16 || (dP_lo_or_null && dp_scale_or_null), "attn_bwd: dP_hi needs dP_lo and dp_scale");
-  const bool structured = d->edge_mode == 1 && d->Fe > 0;
-  SPOTV2_REQUIRE(d->Fe == 0 || structured || (edge_rows && table && v),
-                 "attn_bwd: edge_rows, table and v are required when Fe > 0");
-  SPOTV2_REQUIRE(!structured || (edge_terms_or_null && d_edge_terms_or_null && aligned16(d_edge_terms_or_null)),
-                 "attn_bwd: edge_mode 1 needs edge_terms and a 16-byte aligned d_edge_terms buffer");
-  if (structured && d->N <= 32 && d->attn_bwd_algo == 1)
-    return fail(SPOTV2_ERR_UNSUPPORTED, "attn_bwd: for N <= 32, edge_mode 1 runs on the pipelined kernel only");
-  SPOTV2_REQUIRE(aligned16(P_aug) && aligned16(dout) && (f16 || aligned16(dP_aug_or_null)) &&
-                     (!f16 || (aligned16(dP_hi_or_null) && aligned16(dP_lo_or_null))),
-                 "attn_bwd: P_aug/dout/dP must be 16-byte aligned");
-  if (d->H > kMaxHeads) return fail(SPOTV2_ERR_UNSUPPORTED, "H=%d > %d", d->H, kMaxHeads);
-  if (d->Fe > kMaxFe) return fail(SPOTV2_ERR_UNSUPPORTED, "Fe=%d > %d", d->Fe, kMaxFe);
-  AttnBwdArgs a;
-  a.p.B = d->B; a.p.N = d->N; a.p.F = d->F; a.p.Fe = d->Fe; a.p.H = d->H; a.p.C = d->C;
-  a.p.R = d->R; a.p.concat = d->concat; a.p.ldp = d->ldp;
-  a.p.ldo = d->concat ? d->H * d->C : d->C;
-  a.p.slope = d->negative_slope;
-  a.p.drop = dropout_params(d);
-  a.p.lg_tensor_cores = d->gemm_algo != 1;
-  SPOTV2_REQUIRE(!edge_terms_or_null || aligned16(edge_terms_or_null), "attn_bwd: edge_terms must be 16-byte aligned");
-  SPOTV2_REQUIRE(!d_edge_terms_or_null || aligned16(d_edge_terms_or_null), "attn_bwd: d_edge_terms must be 16-byte aligned");
-  a.p.edge_terms = d->Fe > 0 ? const_cast<float*>(edge_terms_or_null) : nullptr;
-  a.p.terms_in = structured ? 1 : 0;
-  a.p.dterms_out = d->Fe > 0 ? d_edge_terms_or_null : nullptr;      // both edge modes (edge_mode 0: spotv2_gat_edge_rows_grad)
-  a.p.P_aug = P_aug; a.p.edge_rows = edge_rows; a.p.table = table; a.p.v = v;
-  a.p.bulk_ok = d->Fe > 0 && aligned16(edge_rows) && ((size_t)d->R * d->Fe) % 4 == 0;
-  a.p.vec2_ok = (d->C % 2 == 0);
-  a.dout = dout; a.dP_aug = f16 ? nullptr : dP_aug_or_null; a.dv_part = nullptr; a.dbias_part = nullptr;
+  const bool f16 = dP_hi_or_null != nullptr, structured = d->edge_mode == 1 && d->Fe > 0;
+  const AttnEdgeArgs e{edge_rows, table, v, edge_terms_or_null, d_edge_terms_or_null, true};
+  if (int rc = check_attn_inputs(
+          "attn_bwd", d,
+          {{P_aug && dout, "attn_bwd: P_aug and dout must be non-null"},
+           {f16 || dP_aug_or_null, "attn_bwd: give dP_aug (fp32) or dP_hi/dP_lo/dp_scale (fp16 pairs)"},
+           {!f16 || (dP_lo_or_null && dp_scale_or_null), "attn_bwd: dP_hi needs dP_lo and dp_scale"}},
+          {{!(structured && d->N <= 32 && d->attn_bwd_algo == 1), "attn_bwd: for N <= 32, edge_mode 1 runs on the pipelined kernel only",
+            SPOTV2_ERR_UNSUPPORTED},
+           {aligned16(P_aug) && aligned16(dout) && (f16 || aligned16(dP_aug_or_null)) &&
+                (!f16 || (aligned16(dP_hi_or_null) && aligned16(dP_lo_or_null))),
+            "attn_bwd: P_aug/dout/dP must be 16-byte aligned"}},
+          e))
+    return rc;
+  AttnBwdArgs a{};
+  a.p = attn_params_of(d, e);
+  a.p.P_aug = P_aug;
+  a.dout = dout; a.dP_aug = f16 ? nullptr : dP_aug_or_null;
   a.dP_hi16 = static_cast<__half*>(dP_hi_or_null); a.dP_lo16 = static_cast<__half*>(dP_lo_or_null);
   const int HC = d->H * d->C;
   a.ldp16 = ld16_of(HC + 2 * d->H);
-  a.dout_blk = nullptr; a.p_amax = nullptr; a.bound = 1.f; a.dsd = nullptr; a.dp_blk = dp_scale_or_null; a.dsd_amax = nullptr;
+  a.bound = 1.f; a.dp_blk = dp_scale_or_null;
   cudaStream_t st = as_stream(stream);
-  if (attn_large_applies(d))       // N > 32: several CTAs per graph (attn_large.cu); emits the pair through a split pass
+  BwdKernel kern;
+  if (int rc = choose_bwd_kernel(d, a.p, &kern)) return rc;
+  if (kern == BwdKernel::kLarge)       // several CTAs per graph (attn_large.cu); emits the pair through a split pass
     return attn_large_bwd(d, a, dv_or_null, dbias_or_null, ws, ws_bytes, st);
-  const size_t rows = (size_t)d->B * d->N;
-  if (!ws || ws_bytes < attn_bwd_ws_bytes(d))
-    return fail(SPOTV2_ERR_WORKSPACE, "attn_bwd needs %zu B of workspace, got %zu", attn_bwd_ws_bytes(d), ws_bytes);
-  // workspace: per-CTA partials | ds,dd in fp32 [B*N, 2H] | scale blocks (max|dout|, ds|dd scratch, max|P|)
-  const size_t part = attn_bwd_partials_bytes(d);
-  unsigned char* w = static_cast<unsigned char*>(ws);
-  float* blk_dout = reinterpret_cast<float*>(w + part + round_up(rows * 2 * d->H * sizeof(float), 256));
+  const BwdWorkspace w = bwd_workspace_of(d);
+  if (!ws || ws_bytes < w.total)
+    return fail(SPOTV2_ERR_WORKSPACE, "attn_bwd needs %zu B of workspace, got %zu", w.total, ws_bytes);
+  unsigned char* base = static_cast<unsigned char*>(ws);
+  float* blk_dout = reinterpret_cast<float*>(base + w.blocks);
   float* blk_tmp = blk_dout + kScaleBlockFloats;
   float* blk_p = blk_tmp + kScaleBlockFloats;
+  const size_t rows = (size_t)d->B * d->N;
   // the two big products run on fp16 operand pairs scaled by their tensors' maxima
   a.dout_blk = blk_dout;
   if (int rc = amax_flat(dout, rows * (size_t)a.p.ldo, blk_dout, st)) return rc;
@@ -784,47 +847,27 @@ extern "C" int spotv2_gat_attn_bwd(const spotv2_gat_desc* d, const float* P_aug,
     if (int rc = amax_2d(P_aug, (int)rows, HC, (size_t)d->ldp, blk_p, st)) return rc;
     a.p_amax = blk_p;
   }
+  // the pipelined and the tcgen05 kernels collect max |ds|, |dd| themselves (dp_scale block entry 1, zeroed here)
+  const bool dsd_fused = f16 && kern != BwdKernel::kPhaseSerial;
   if (f16) {
-    a.dsd = reinterpret_cast<float*>(w + part);
-    // |dP_h[j,c]| = |g sum_i alpha_h[i,j] dO[i,c]| <= g N max|dout|  (g = 1/H for the head mean)
-    // (attention dropout scales the kept coefficients by 1/(1-p): the bound grows with it)
-    a.bound = (float)d->N * (d->concat ? 1.f : 1.f / (float)d->H) * a.p.drop.scale;
+    a.dsd = reinterpret_cast<float*>(base + w.dsd);
+    a.bound = dp_bound(a.p);
     SPOTV2_CUDA_OK(cudaMemsetAsync(dp_scale_or_null, 0, kScaleBlockFloats * sizeof(float), st));
   }
+  if (dsd_fused) a.dsd_amax = reinterpret_cast<unsigned*>(dp_scale_or_null) + 1;
+  float* dv = structured ? nullptr : dv_or_null;      // edge_mode 1: spotv2_windows_dv forms dv
   const int np = (d->N + 1) / 2;
   int rc;
-  // d->attn_bwd_algo selects the kernel: 0 = pipelined (attn_bwd2.cu) whenever its shared-memory plan fits,
-  // 1 = the phase-serial kernel of this file, 2 = pipelined or error
-  // d->attn_bwd_algo: 0 = the library's choice (the pipelined mma.sync kernel when its shared-memory plan fits, else the
-  // phase-serial kernel), 1 = phase-serial, 2 = pipelined or error, 3 = the tcgen05 kernel (attn_bwd3.cu) or error.
-  // The tcgen05 kernel is NOT the default: measured on B200 it is bound by the shared-memory port (operand split passes
-  // plus tf32 operand reads, DESIGN.md section 6) and runs 2.0-2.2 ms where the pipelined kernel runs 1.95 ms.
-  const bool tc5 = d->attn_bwd_algo == 3 && attn_bwd3_applies(a.p);
-  if (d->attn_bwd_algo == 3 && !tc5)
-    return fail(SPOTV2_ERR_UNSUPPORTED, "attn_bwd: the tcgen05 kernel covers head-mean layers with N <= 31, C %% 4 == 0, even Fe <= 128 "
-                                        "and the forward's edge terms");
-  if (structured && !tc5 && !attn_bwd2_fits(a.p))
-    return fail(SPOTV2_ERR_UNSUPPORTED, "attn_bwd: edge_mode 1 needs the pipelined kernel, whose shared-memory plan does not fit this shape");
-  // the pipelined and the tcgen05 kernels collect max |ds|, |dd| themselves (dp_scale block entry 1, zeroed above)
-  const bool piped = !tc5 && d->attn_bwd_algo != 1 && (attn_bwd2_fits(a.p) || d->attn_bwd_algo == 2);
-  const bool dsd_fused = f16 && (tc5 || piped);
-  if (dsd_fused) a.dsd_amax = reinterpret_cast<unsigned*>(dp_scale_or_null) + 1;
-  if (tc5)
-    rc = launch_attn_bwd3(a, structured ? nullptr : dv_or_null, dbias_or_null, ws, ws_bytes, st);
-  else if (piped)
-    rc = launch_attn_bwd2(a, structured ? nullptr : dv_or_null, dbias_or_null, ws, ws_bytes, st);
+  if (kern == BwdKernel::kTcgen05) rc = launch_attn_bwd3(a, dv, dbias_or_null, ws, ws_bytes, st);
+  else if (kern == BwdKernel::kPipelined) rc = launch_attn_bwd2(a, dv, dbias_or_null, ws, ws_bytes, st);
   else if (np <= 4) rc = launch_bwd<4>(a, dv_or_null, dbias_or_null, ws, ws_bytes, st);
   else if (np <= 8) rc = launch_bwd<8>(a, dv_or_null, dbias_or_null, ws, ws_bytes, st);
   else if (np <= 15) rc = launch_bwd<15>(a, dv_or_null, dbias_or_null, ws, ws_bytes, st);
   else if (np <= 16) rc = launch_bwd<16>(a, dv_or_null, dbias_or_null, ws, ws_bytes, st);
   else return fail(SPOTV2_ERR_UNSUPPORTED, "N=%d > 32: the one-CTA-per-graph kernel covers N <= 32", d->N);
   if (rc) return rc;
-  if (dsd_fused) {
-    const size_t total = rows * 2 * (size_t)d->H;
-    split_dsd_kernel<<<(unsigned)std::min<size_t>((total + 255) / 256, (size_t)8 * 148), 256, 0, st>>>(
-        a.dsd, total, 2 * d->H, a.dP_hi16 + HC, a.dP_lo16 + HC, a.ldp16, dp_scale_or_null);
-    SPOTV2_CUDA_OK(cudaGetLastError());
-  } else if (f16) {
+  if (dsd_fused) return split_dsd(a, HC, st);
+  if (f16) {
     // ds | dd: own scale group (columns [HC, HC + 2H) of the fp16 pair arrays)
     const int none = 0x7fffffff;
     if ((rc = split_f16(a.dsd, (int)rows, 2 * d->H, 2 * d->H, 0, none, nullptr, 0, a.dP_hi16 + HC, a.dP_lo16 + HC,
@@ -844,84 +887,58 @@ extern "C" int spotv2_gat_attn_bwd_pair(const spotv2_gat_desc* d, const void* P_
                                         float* dv_or_null, float* d_edge_terms_or_null, float* dbias_or_null, void* ws,
                                         size_t ws_bytes, void* stream) {
   if (int rc = check_desc(d)) return rc;
-  SPOTV2_REQUIRE(d->p_format == 1, "attn_bwd_pair: the descriptor must say p_format 1");
   const bool single = d->gemm_algo == 3;
-  SPOTV2_REQUIRE(P_hi && p_scale && sd && dout && dP_hi && dp_scale, "attn_bwd_pair: P_hi, p_scale, sd, dout, dP_hi and dp_scale must be non-null");
-  SPOTV2_REQUIRE(single || (P_lo_or_null && dP_lo_or_null), "attn_bwd_pair: the lo planes may be omitted with gemm_algo 3 only");
-  const bool structured = d->edge_mode == 1 && d->Fe > 0;
-  SPOTV2_REQUIRE(d->Fe == 0 || structured || (edge_rows && table && v), "attn_bwd_pair: edge_rows, table and v are required when Fe > 0");
-  SPOTV2_REQUIRE(!structured || (edge_terms_or_null && d_edge_terms_or_null && aligned16(d_edge_terms_or_null)),
-                 "attn_bwd_pair: edge_mode 1 needs edge_terms and a 16-byte aligned d_edge_terms buffer");
-  SPOTV2_REQUIRE(aligned16(P_hi) && aligned16(dout) && aligned16(dP_hi) && (single || (aligned16(P_lo_or_null) && aligned16(dP_lo_or_null))),
-                 "attn_bwd_pair: P / dout / dP must be 16-byte aligned");
-  if (d->H > kMaxHeads) return fail(SPOTV2_ERR_UNSUPPORTED, "H=%d > %d", d->H, kMaxHeads);
-  if (d->Fe > kMaxFe) return fail(SPOTV2_ERR_UNSUPPORTED, "Fe=%d > %d", d->Fe, kMaxFe);
-  AttnBwdArgs a;
-  a.p.B = d->B; a.p.N = d->N; a.p.F = d->F; a.p.Fe = d->Fe; a.p.H = d->H; a.p.C = d->C;
-  a.p.R = d->R; a.p.concat = d->concat; a.p.ldp = d->ldp;
-  a.p.ldo = d->concat ? d->H * d->C : d->C;
-  a.p.slope = d->negative_slope;
-  a.p.drop = dropout_params(d);
-  a.p.lg_tensor_cores = 1;
-  SPOTV2_REQUIRE(!edge_terms_or_null || aligned16(edge_terms_or_null), "attn_bwd_pair: edge_terms must be 16-byte aligned");
-  SPOTV2_REQUIRE(!d_edge_terms_or_null || aligned16(d_edge_terms_or_null), "attn_bwd_pair: d_edge_terms must be 16-byte aligned");
-  a.p.edge_terms = d->Fe > 0 ? const_cast<float*>(edge_terms_or_null) : nullptr;
-  a.p.terms_in = structured ? 1 : 0;
-  a.p.dterms_out = d->Fe > 0 ? d_edge_terms_or_null : nullptr;      // both edge modes (edge_mode 0: spotv2_gat_edge_rows_grad)
-  a.p.alpha_rec = attn_record_of(d);
-  a.p.P_aug = nullptr; a.p.edge_rows = edge_rows; a.p.table = table; a.p.v = v;
+  const AttnEdgeArgs e{edge_rows, table, v, edge_terms_or_null, d_edge_terms_or_null, true};
+  if (int rc = check_attn_inputs(
+          "attn_bwd_pair", d,
+          {{d->p_format == 1, "attn_bwd_pair: the descriptor must say p_format 1"},
+           {P_hi && p_scale && sd && dout && dP_hi && dp_scale, "attn_bwd_pair: P_hi, p_scale, sd, dout, dP_hi and dp_scale must be non-null"},
+           {single || (P_lo_or_null && dP_lo_or_null), "attn_bwd_pair: the lo planes may be omitted with gemm_algo 3 only"}},
+          {{aligned16(P_hi) && aligned16(dout) && aligned16(dP_hi) && (single || (aligned16(P_lo_or_null) && aligned16(dP_lo_or_null))),
+            "attn_bwd_pair: P / dout / dP must be 16-byte aligned"}},
+          e))
+    return rc;
+  AttnBwdArgs a{};
+  a.p = attn_params_of(d, e);
   a.p.P_hi = static_cast<const __half*>(P_hi);
   a.p.P_lo = single ? nullptr : static_cast<const __half*>(P_lo_or_null);
   a.p.p_blk = p_scale;
   a.p.sd32 = sd;
-  a.p.hp = head_pitch_of(d);
-  a.p.ldp16 = ld16_of(n_aug_of(d));
-  a.p.bulk_ok = d->Fe > 0 && aligned16(edge_rows) && ((size_t)d->R * d->Fe) % 4 == 0;
-  a.p.vec2_ok = (d->C % 2 == 0);
-  a.dout = dout; a.dP_aug = nullptr; a.dv_part = nullptr; a.dbias_part = nullptr;
+  a.dout = dout;
   a.dP_hi16 = static_cast<__half*>(dP_hi);
   a.dP_lo16 = single ? nullptr : static_cast<__half*>(dP_lo_or_null);
   a.ldp16 = a.p.ldp16;
-  a.dp_blk = dp_scale; a.p_amax = nullptr;
+  a.dp_blk = dp_scale;
   cudaStream_t st = as_stream(stream);
   if (!attn_bwd2_fits(a.p))
     return fail(SPOTV2_ERR_UNSUPPORTED, "attn_bwd_pair: the pipelined kernel's shared-memory plan does not fit this shape");
-  const size_t rows = (size_t)d->B * d->N;
-  if (!ws || ws_bytes < attn_bwd_ws_bytes(d))
-    return fail(SPOTV2_ERR_WORKSPACE, "attn_bwd_pair needs %zu B of workspace, got %zu", attn_bwd_ws_bytes(d), ws_bytes);
-  const size_t part = attn_bwd_partials_bytes(d);
-  unsigned char* w = static_cast<unsigned char*>(ws);
-  float* blk_dout = reinterpret_cast<float*>(w + part + round_up(rows * 2 * d->H * sizeof(float), 256));
-  a.dout_blk = blk_dout;
+  const BwdWorkspace w = bwd_workspace_of(d);
+  if (!ws || ws_bytes < w.total)
+    return fail(SPOTV2_ERR_WORKSPACE, "attn_bwd_pair needs %zu B of workspace, got %zu", w.total, ws_bytes);
+  unsigned char* base = static_cast<unsigned char*>(ws);
   // dout -> operand pair, unit scales, max|dout|, dbias: one pass (attn_prep.cu)
   {
     const int upg = d->concat ? d->H : 1;
     const int ldo16 = ld16_of(a.p.ldo);
-    const size_t plane = round_up(rows * (size_t)ldo16 * 2, 256);
-    unsigned char* x = reinterpret_cast<unsigned char*>(blk_dout) + 256;
-    __half* dhi = reinterpret_cast<__half*>(x);
-    __half* dlo = single ? nullptr : reinterpret_cast<__half*>(x + plane);
-    float* scales = reinterpret_cast<float*>(x + 2 * plane);
-    float* bpart = reinterpret_cast<float*>(x + 2 * plane + round_up((size_t)d->B * upg * sizeof(float), 256));
+    float* blk_dout = reinterpret_cast<float*>(base + w.blocks);
+    __half* dhi = reinterpret_cast<__half*>(base + w.dout_pair);
+    __half* dlo = single ? nullptr : reinterpret_cast<__half*>(base + w.dout_pair + w.plane);
+    float* scales = reinterpret_cast<float*>(base + w.unit_scales);
     // (the bias gradient's per-CTA partials are reduced together with the dv partials, behind the attention kernel)
+    float* bpart = dbias_or_null ? reinterpret_cast<float*>(base + w.dbias_part) : nullptr;
     int n_parts = 0;
-    if (int rc = dout_pair_prepass(dout, d->B, d->N, d->C, upg, dhi, dlo, ldo16, scales, blk_dout, nullptr, dbias_or_null ? bpart : nullptr, st,
-                                   &n_parts))
+    if (int rc = dout_pair_prepass(dout, d->B, d->N, d->C, upg, dhi, dlo, ldo16, scales, blk_dout, nullptr, bpart, st, &n_parts))
       return rc;
+    a.dout_blk = blk_dout;
     a.dO_hi = dhi; a.dO_lo = dlo; a.dO_scale = scales; a.ldo16 = ldo16; a.units_per_graph = upg;
-    a.prep_dbias_part = dbias_or_null ? bpart : nullptr; a.prep_dbias_n = n_parts;
+    a.prep_dbias_part = bpart; a.prep_dbias_n = n_parts;
   }
-  a.dsd = reinterpret_cast<float*>(w + part);
-  a.bound = (float)d->N * (d->concat ? 1.f : 1.f / (float)d->H) * a.p.drop.scale;
+  a.dsd = reinterpret_cast<float*>(base + w.dsd);
+  a.bound = dp_bound(a.p);
   SPOTV2_CUDA_OK(cudaMemsetAsync(dp_scale, 0, kScaleBlockFloats * sizeof(float), st));
   a.dsd_amax = reinterpret_cast<unsigned*>(dp_scale) + 1;
-  if (int rc = launch_attn_bwd2(a, structured ? nullptr : dv_or_null, dbias_or_null, ws, ws_bytes, st)) return rc;
-  const size_t total = rows * 2 * (size_t)d->H;
-  const int HCp = d->H * a.p.hp;
-  split_dsd_kernel<<<(unsigned)std::min<size_t>((total + 255) / 256, (size_t)8 * 148), 256, 0, st>>>(
-      a.dsd, total, 2 * d->H, a.dP_hi16 + HCp, a.dP_lo16 ? a.dP_lo16 + HCp : nullptr, a.ldp16, dp_scale);
-  SPOTV2_CUDA_OK(cudaGetLastError());
-  return SPOTV2_OK;
+  if (int rc = launch_attn_bwd2(a, a.p.terms_in ? nullptr : dv_or_null, dbias_or_null, ws, ws_bytes, st)) return rc;
+  return split_dsd(a, d->H * a.p.hp, st);
 }
 
 
@@ -931,12 +948,8 @@ extern "C" int spotv2_gat_pair_format_supported(const spotv2_gat_desc* d) {
   if (!d || d->B <= 0 || d->N <= 0 || d->N > 32 || d->H <= 0 || d->H > kMaxHeads || d->C <= 0 || d->Fe < 0 || d->Fe > kMaxFe) return 0;
   if (d->gemm_algo == 1 || d->attn_bwd_algo == 1 || d->attn_bwd_algo == 3) return 0;
   if (d->C % 4 != 0 || d->C > 1024 || (d->concat && d->C % 8 != 0)) return 0;
-  AttnParams p{};
-  p.B = d->B; p.N = d->N; p.F = d->F; p.Fe = d->Fe; p.H = d->H; p.C = d->C; p.R = d->R; p.concat = d->concat; p.ldp = d->ldp;
-  p.ldo = d->concat ? d->H * d->C : d->C;
-  p.drop = dropout_params(d);
-  p.terms_in = (d->edge_mode == 1 && d->Fe > 0) ? 1 : 0;
-  p.hp = (d->C + 7) / 8 * 8;
-  p.ldp16 = ld16_of(d->H * p.hp + 2 * d->H);
+  spotv2_gat_desc pair = *d;
+  pair.p_format = 1;
+  const AttnParams p = attn_params_of(&pair, AttnEdgeArgs{});
   return (attn_fwd16_fits(p) && attn_bwd2_fits(p)) ? 1 : 0;
 }

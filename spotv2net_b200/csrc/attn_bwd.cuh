@@ -3,6 +3,7 @@
 // shared-memory plan fits).
 #pragma once
 #include <cuda_fp16.h>
+#include <initializer_list>
 
 #include "attn_common.cuh"
 #include "gemm.cuh"
@@ -15,6 +16,17 @@ struct AttnFwdArgs {
   float* out;
   float* alpha_out;
 };
+// Edge inputs of one attention entry point as the caller passed them (the forward has no d_edge_terms)
+struct AttnEdgeArgs { const float* rows; const int32_t* table; const float* v; const float* terms; float* dterms; bool backward; };
+// An entry point's own argument check: fails with `st` and the message `msg` when `ok` is false
+struct ArgCheck { bool ok; const char* msg; spotv2_status st = SPOTV2_ERR_INVALID_ARG; };
+// Input checks of the attention entry points after check_desc, in order: `own_args`; edge rows, table and v if Fe > 0; edge
+// mode 1's edge terms (backward: and d_edge_terms); `own_layout`; H, Fe limits; edge-term alignment.  `who` prefixes messages.
+int check_attn_inputs(const char* who, const spotv2_gat_desc* d, std::initializer_list<ArgCheck> own_args,
+                      std::initializer_list<ArgCheck> own_layout, const AttnEdgeArgs& e);
+// The kernels' view of a descriptor and its edge inputs; p_format 1 adds the head pitch, ld16 of the planes and the forward's
+// record flag.  The caller sets the projection's pointers (P_aug, or P_hi / P_lo / p_blk / sd32).
+AttnParams attn_params_of(const spotv2_gat_desc* d, const AttnEdgeArgs& e);
 // p_format 1 forward (attn_fwd16.cu): P as an fp16 operand pair, aggregation on m16n8k16 from ldmatrix fragments
 int attn_fwd16_dispatch(const AttnFwdArgs& a, cudaStream_t st);
 bool attn_fwd16_fits(const AttnParams& p);                        // its shared-memory plan fits this problem

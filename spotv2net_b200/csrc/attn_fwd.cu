@@ -515,29 +515,12 @@ extern "C" int spotv2_gat_attn_fwd(const spotv2_gat_desc* d, const float* P_aug,
                                    const float* bias_or_null, float* out, float* alpha_or_null,
                                    float* edge_terms_or_null, void* ws, size_t ws_bytes, void* stream) {
   if (int rc = check_desc(d)) return rc;
-  SPOTV2_REQUIRE(P_aug && out, "attn_fwd: P_aug and out must be non-null");
-  const bool structured = d->edge_mode == 1 && d->Fe > 0;
-  SPOTV2_REQUIRE(d->Fe == 0 || structured || (edge_rows && table && v),
-                 "attn_fwd: edge_rows, table and v are required when Fe > 0");
-  SPOTV2_REQUIRE(!structured || edge_terms_or_null, "attn_fwd: edge_mode 1 needs edge_terms (spotv2_edge_terms_from_windows)");
-  SPOTV2_REQUIRE(aligned16(P_aug) && aligned16(out), "attn_fwd: P_aug/out must be 16-byte aligned");
-  if (d->H > kMaxHeads) return fail(SPOTV2_ERR_UNSUPPORTED, "H=%d > %d", d->H, kMaxHeads);
-  if (d->Fe > kMaxFe) return fail(SPOTV2_ERR_UNSUPPORTED, "Fe=%d > %d", d->Fe, kMaxFe);
-  AttnFwdArgs a;
-  a.p.B = d->B; a.p.N = d->N; a.p.F = d->F; a.p.Fe = d->Fe; a.p.H = d->H; a.p.C = d->C;
-  a.p.R = d->R; a.p.concat = d->concat; a.p.ldp = d->ldp;
-  a.p.ldo = d->concat ? d->H * d->C : d->C;
-  a.p.slope = d->negative_slope;
-  a.p.drop = dropout_params(d);
-  a.p.lg_tensor_cores = d->gemm_algo != 1;
-  a.p.P_aug = P_aug; a.p.edge_rows = edge_rows; a.p.table = table; a.p.v = v;
-  a.p.bulk_ok = d->Fe > 0 && aligned16(edge_rows) && ((size_t)d->R * d->Fe) % 4 == 0;
-  a.p.vec2_ok = (d->C % 2 == 0);
-  SPOTV2_REQUIRE(!edge_terms_or_null || aligned16(edge_terms_or_null), "attn_fwd: edge_terms must be 16-byte aligned");
-  a.p.edge_terms = d->Fe > 0 ? edge_terms_or_null : nullptr;
-  a.p.terms_in = structured ? 1 : 0;
-  a.p.dterms_out = nullptr;
-  a.bias = bias_or_null; a.out = out; a.alpha_out = alpha_or_null;
+  const AttnEdgeArgs e{edge_rows, table, v, edge_terms_or_null, nullptr, false};
+  if (int rc = check_attn_inputs("attn_fwd", d, {{P_aug && out, "attn_fwd: P_aug and out must be non-null"}},
+                                 {{aligned16(P_aug) && aligned16(out), "attn_fwd: P_aug/out must be 16-byte aligned"}}, e))
+    return rc;
+  AttnFwdArgs a{attn_params_of(d, e), bias_or_null, out, alpha_or_null};
+  a.p.P_aug = P_aug;
   if (attn_large_applies(d))       // several CTAs per graph, attention tile in the workspace (or alpha_or_null)
     return attn_large_fwd(a.p, bias_or_null, out, alpha_or_null, ws, ws_bytes, as_stream(stream));
   return attn_fwd_dispatch(a, as_stream(stream));

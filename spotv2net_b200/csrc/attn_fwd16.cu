@@ -632,36 +632,20 @@ extern "C" int spotv2_gat_attn_fwd_pair(const spotv2_gat_desc* d, const void* P_
                                         const float* sd, const float* edge_rows, const int32_t* table, const float* v, const float* bias_or_null,
                                         float* out, float* alpha_or_null, float* edge_terms_or_null, void* stream) {
   if (int rc = check_desc(d)) return rc;
-  SPOTV2_REQUIRE(d->p_format == 1, "attn_fwd_pair: the descriptor must say p_format 1");
-  SPOTV2_REQUIRE(P_hi && p_scale && sd && out, "attn_fwd_pair: P_hi, p_scale, sd and out must be non-null");
-  SPOTV2_REQUIRE(P_lo_or_null || d->gemm_algo == 3, "attn_fwd_pair: the lo plane may be omitted with gemm_algo 3 only");
-  const bool structured = d->edge_mode == 1 && d->Fe > 0;
-  SPOTV2_REQUIRE(d->Fe == 0 || structured || (edge_rows && table && v), "attn_fwd_pair: edge_rows, table and v are required when Fe > 0");
-  SPOTV2_REQUIRE(!structured || edge_terms_or_null, "attn_fwd_pair: edge_mode 1 needs edge_terms (spotv2_edge_terms_from_windows)");
-  SPOTV2_REQUIRE(aligned16(P_hi) && (!P_lo_or_null || aligned16(P_lo_or_null)) && aligned16(out), "attn_fwd_pair: P planes / out must be 16-byte aligned");
-  if (d->H > kMaxHeads) return fail(SPOTV2_ERR_UNSUPPORTED, "H=%d > %d", d->H, kMaxHeads);
-  if (d->Fe > kMaxFe) return fail(SPOTV2_ERR_UNSUPPORTED, "Fe=%d > %d", d->Fe, kMaxFe);
-  AttnFwdArgs a;
-  a.p.B = d->B; a.p.N = d->N; a.p.F = d->F; a.p.Fe = d->Fe; a.p.H = d->H; a.p.C = d->C;
-  a.p.R = d->R; a.p.concat = d->concat; a.p.ldp = d->ldp;
-  a.p.ldo = d->concat ? d->H * d->C : d->C;
-  a.p.slope = d->negative_slope;
-  a.p.drop = dropout_params(d);
-  a.p.lg_tensor_cores = 1;
-  a.p.P_aug = nullptr; a.p.edge_rows = edge_rows; a.p.table = table; a.p.v = v;
+  const AttnEdgeArgs e{edge_rows, table, v, edge_terms_or_null, nullptr, false};
+  if (int rc = check_attn_inputs(
+          "attn_fwd_pair", d,
+          {{d->p_format == 1, "attn_fwd_pair: the descriptor must say p_format 1"},
+           {P_hi && p_scale && sd && out, "attn_fwd_pair: P_hi, p_scale, sd and out must be non-null"},
+           {P_lo_or_null || d->gemm_algo == 3, "attn_fwd_pair: the lo plane may be omitted with gemm_algo 3 only"}},
+          {{aligned16(P_hi) && (!P_lo_or_null || aligned16(P_lo_or_null)) && aligned16(out),
+            "attn_fwd_pair: P planes / out must be 16-byte aligned"}},
+          e))
+    return rc;
+  AttnFwdArgs a{attn_params_of(d, e), bias_or_null, out, alpha_or_null};
   a.p.P_hi = static_cast<const __half*>(P_hi);
   a.p.P_lo = d->gemm_algo == 3 ? nullptr : static_cast<const __half*>(P_lo_or_null);
   a.p.p_blk = p_scale;
   a.p.sd32 = sd;
-  a.p.hp = head_pitch_of(d);
-  a.p.ldp16 = ld16_of(n_aug_of(d));
-  a.p.bulk_ok = d->Fe > 0 && aligned16(edge_rows) && ((size_t)d->R * d->Fe) % 4 == 0;
-  a.p.vec2_ok = (d->C % 2 == 0);
-  SPOTV2_REQUIRE(!edge_terms_or_null || aligned16(edge_terms_or_null), "attn_fwd_pair: edge_terms must be 16-byte aligned");
-  a.p.edge_terms = d->Fe > 0 ? edge_terms_or_null : nullptr;
-  a.p.terms_in = structured ? 1 : 0;
-  a.p.dterms_out = nullptr;
-  a.p.alpha_rec = attn_record_of(d);
-  a.bias = bias_or_null; a.out = out; a.alpha_out = alpha_or_null;
   return attn_fwd16_dispatch(a, as_stream(stream));
 }

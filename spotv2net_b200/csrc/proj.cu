@@ -29,11 +29,15 @@ bool use_tc(const spotv2_gat_desc* d) { return d->gemm_algo != 1; }
 // A_hi * B_hi product of the scaled fp16 operands (11-bit significands, fp32 accumulate): a third of the tensor work.
 bool single_product(const spotv2_gat_desc* d) { return d->gemm_algo == 3; }
 
+// Carves the caller's workspace in 256-byte units.  With a null base it only counts (`used`): the workspace query runs the
+// products' own carving code that way.
 struct Carver {
   unsigned char* p;
   size_t left;
+  size_t used = 0;
   void* take(size_t bytes) {
     bytes = round_up(bytes, 256);
+    used += bytes;
     if (!p || bytes > left) return nullptr;
     void* r = p;
     p += bytes;
@@ -42,7 +46,32 @@ struct Carver {
   }
 };
 
-size_t pair_bytes(size_t rows, size_t ld16) { return 2 * round_up(rows * ld16 * 2, 256); }
+// Every tensor-core product carves its two scale blocks first.  The query reserves 1 KB for them, and adds 256 B to the
+// attention backward's own size: slack it has always given.
+constexpr size_t kBlocksBytes = 2 * kScaleBlockFloats * sizeof(float), kBlocksReserve = 1024, kAttnBwdReserve = 256;
+
+// A GEMM operand as an fp16 pair: the caller's (hi, lo and scale block all given), or two planes [rows, ld16] taken from the
+// workspace, which split() fills from the fp32 tensor.
+struct OperandPair {
+  void* hi;
+  void* lo;
+  const float* scale;
+  bool own;
+  bool ok() const { return hi && lo; }
+  int split(const float* src, int rows, int cols, size_t ld, int split_dim, int split_at, int ld16, float* blk, cudaStream_t st) {
+    if (!own) return SPOTV2_OK;
+    scale = blk;
+    return split_f16(src, rows, cols, ld, split_dim, split_at, nullptr, 0, hi, lo, ld16, blk, st);
+  }
+};
+
+OperandPair operand_pair(Carver& c, size_t rows, int ld16, const void* hi = nullptr, const void* lo = nullptr,
+                         const float* scale = nullptr) {
+  if (hi && lo && scale) return {const_cast<void*>(hi), const_cast<void*>(lo), scale, false};
+  void* h = c.take(rows * ld16 * 2);
+  void* l = c.take(rows * ld16 * 2);
+  return {h, l, nullptr, true};
+}
 
 }  // namespace
 
@@ -53,15 +82,21 @@ extern "C" int spotv2_gat_workspace_bytes(const spotv2_gat_desc* d, size_t* proj
                                           size_t* attn_bwd, size_t* proj_bwd) {
   if (int rc = check_desc(d)) return rc;
   const ProjShape s = shape_of(d);
-  const bool tc = use_tc(d);
-  if (proj_fwd) *proj_fwd = 1024 + (tc ? pair_bytes(s.rows, s.ldf16) + pair_bytes(s.n_aug, s.ldf16) : 0);
-  if (attn_bwd) *attn_bwd = attn_bwd_ws_bytes(d) + 256;
-  if (proj_bwd) {
-    const int splits = weight_grad_splits(s.rows, s.n_aug, s.F, !single_product(d));
-    size_t w = round_up((size_t)splits * s.n_aug * s.F * sizeof(float), 256) + 1024;
-    if (tc) w += pair_bytes(s.rows, s.ldp16) + pair_bytes(s.rows, s.ldf16) + pair_bytes(s.n_aug, s.ldf16);
-    *proj_bwd = w;
+  // The products' pairs, counted (proj_fwd_pair takes less than proj_fwd).  proj_bwd serves both backward products: the dP
+  // pair, dW's x pair and split-K partials, and dX's W_aug pair.
+  Carver f{nullptr, 0}, b{nullptr, 0};
+  if (use_tc(d)) {
+    operand_pair(f, s.rows, s.ldf16);
+    operand_pair(f, s.n_aug, s.ldf16);
+    operand_pair(b, s.rows, s.ldp16);
+    operand_pair(b, s.rows, s.ldf16);
+    operand_pair(b, s.n_aug, s.ldf16);
   }
+  const int splits = weight_grad_splits(s.rows, s.n_aug, s.F, !single_product(d));
+  b.take((size_t)splits * s.n_aug * s.F * sizeof(float));
+  if (proj_fwd) *proj_fwd = kBlocksReserve + f.used;
+  if (attn_bwd) *attn_bwd = attn_bwd_ws_bytes(d) + kAttnBwdReserve;
+  if (proj_bwd) *proj_bwd = kBlocksReserve + b.used;
   return SPOTV2_OK;
 }
 
@@ -106,22 +141,13 @@ extern "C" int spotv2_proj_fwd(const spotv2_gat_desc* d, const float* x, const v
     return p_amax_or_null ? amax_2d(P_aug, s.rows, s.HC, (size_t)s.ldp, p_amax_or_null, st) : SPOTV2_OK;
   }
   Carver c{static_cast<unsigned char*>(ws), ws ? ws_bytes : 0};
-  float* blk = static_cast<float*>(c.take(2 * kScaleBlockFloats * sizeof(float)));
-  const bool have_x = x_hi && x_lo && x_scale;
-  void* xh = have_x ? const_cast<void*>(x_hi) : c.take((size_t)s.rows * s.ldf16 * 2);
-  void* xl = have_x ? const_cast<void*>(x_lo) : c.take((size_t)s.rows * s.ldf16 * 2);
-  void* wh = c.take((size_t)s.n_aug * s.ldf16 * 2);
-  void* wl = c.take((size_t)s.n_aug * s.ldf16 * 2);
-  if (!blk || !xh || !xl || !wh || !wl) return fail(SPOTV2_ERR_WORKSPACE, "proj_fwd: workspace too small (%zu B)", ws_bytes);
-  const float* xs = x_scale;
-  if (!have_x) {
-    if (int rc = split_f16(x, s.rows, s.F, s.F, 0, kNone, nullptr, 0, xh, xl, s.ldf16, blk, st)) return rc;
-    xs = blk;
-  }
+  float* blk = static_cast<float*>(c.take(kBlocksBytes));
+  OperandPair xp = operand_pair(c, s.rows, s.ldf16, x_hi, x_lo, x_scale), wp = operand_pair(c, s.n_aug, s.ldf16);
+  if (!blk || !xp.ok() || !wp.ok()) return fail(SPOTV2_ERR_WORKSPACE, "proj_fwd: workspace too small (%zu B)", ws_bytes);
+  if (int rc = xp.split(x, s.rows, s.F, s.F, 0, kNone, s.ldf16, blk, st)) return rc;
   // W_aug = [W ; u_src ; u_dst]: the folded attention rows carry their own magnitude -> second scale group
-  float* wblk = blk + kScaleBlockFloats;
-  if (int rc = split_f16(W_aug, s.n_aug, s.F, s.F, 0, s.HC, nullptr, 0, wh, wl, s.ldf16, wblk, st)) return rc;
-  F16Operand A{xh, xl, s.ldf16, xs + 2, kNone}, B{wh, wl, s.ldf16, wblk + 2, s.HC};
+  if (int rc = wp.split(W_aug, s.n_aug, s.F, s.F, 0, s.HC, s.ldf16, blk + kScaleBlockFloats, st)) return rc;
+  F16Operand A{xp.hi, xp.lo, s.ldf16, xp.scale + 2, kNone}, B{wp.hi, wp.lo, s.ldf16, wp.scale + 2, s.HC};
   return gemm3x_f16(true, true, s.rows, s.n_aug, s.F, A, B, P_aug, s.ldp, 1, 256, 0, nullptr, 0, st, p_amax_or_null, s.HC,
                     single_product(d));
 }
@@ -136,12 +162,11 @@ extern "C" int spotv2_proj_fwd_pair(const spotv2_gat_desc* d, const void* x_hi, 
   const ProjShape s = shape_of(d);
   cudaStream_t st = as_stream(stream);
   Carver c{static_cast<unsigned char*>(ws), ws ? ws_bytes : 0};
-  float* wblk = static_cast<float*>(c.take(2 * kScaleBlockFloats * sizeof(float)));
-  void* wh = c.take((size_t)s.n_aug * s.ldf16 * 2);
-  void* wl = c.take((size_t)s.n_aug * s.ldf16 * 2);
-  if (!wblk || !wh || !wl) return fail(SPOTV2_ERR_WORKSPACE, "proj_fwd_pair: workspace too small (%zu B)", ws_bytes);
-  if (int rc = w_pair_and_out_scale(W_aug, s.n_aug, s.F, s.HC, wh, wl, s.ldf16, wblk, x_scale, p_scale, st)) return rc;
-  F16Operand A{x_hi, x_lo, s.ldf16, x_scale + 2, kNone}, B{wh, wl, s.ldf16, wblk + 2, s.HC};
+  float* wblk = static_cast<float*>(c.take(kBlocksBytes));
+  const OperandPair wp = operand_pair(c, s.n_aug, s.ldf16);
+  if (!wblk || !wp.ok()) return fail(SPOTV2_ERR_WORKSPACE, "proj_fwd_pair: workspace too small (%zu B)", ws_bytes);
+  if (int rc = w_pair_and_out_scale(W_aug, s.n_aug, s.F, s.HC, wp.hi, wp.lo, s.ldf16, wblk, x_scale, p_scale, st)) return rc;
+  F16Operand A{x_hi, x_lo, s.ldf16, x_scale + 2, kNone}, B{wp.hi, wp.lo, s.ldf16, wblk + 2, s.HC};
   PairOut out{P_hi, single_product(d) ? nullptr : P_lo_or_null, s.ldp16, p_scale + 4, sd, 2 * d->H};
   return gemm3x_f16(true, true, s.rows, s.n_aug, s.F, A, B, nullptr, 0, 1, 256 + 16, 0, nullptr, 0, st, nullptr, 0, single_product(d),
                     &out);
@@ -163,25 +188,15 @@ extern "C" int spotv2_proj_bwd_weight(const spotv2_gat_desc* d, const float* x, 
     return sgemm_simt(false, false, s.n_aug, s.F, s.rows, dP_aug, s.ldp, x, s.F, dW_aug, s.F, splits, ws, ws_bytes, st);
   }
   Carver c{static_cast<unsigned char*>(ws), ws ? ws_bytes : 0};
-  float* blk = static_cast<float*>(c.take(2 * kScaleBlockFloats * sizeof(float)));
-  const bool have_x = x_hi && x_lo && x_scale, have_p = dP_hi && dP_lo && dp_scale;
-  void* ph = have_p ? const_cast<void*>(dP_hi) : c.take((size_t)s.rows * s.ldp16 * 2);
-  void* pl = have_p ? const_cast<void*>(dP_lo) : c.take((size_t)s.rows * s.ldp16 * 2);
-  void* xh = have_x ? const_cast<void*>(x_hi) : c.take((size_t)s.rows * s.ldf16 * 2);
-  void* xl = have_x ? const_cast<void*>(x_lo) : c.take((size_t)s.rows * s.ldf16 * 2);
-  if (!blk || !ph || !pl || !xh || !xl) return fail(SPOTV2_ERR_WORKSPACE, "proj_bwd_weight: workspace too small (%zu B)", ws_bytes);
-  const float *ps = dp_scale, *xs = x_scale;
-  if (!have_p) {
-    SPOTV2_REQUIRE(dP_aug, "proj_bwd_weight: dP_aug or the complete pair (dP_hi, dP_lo, dp_scale)");
-    if (int rc = split_f16(dP_aug, s.rows, s.n_aug, s.ldp, 1, s.HC, nullptr, 0, ph, pl, s.ldp16, blk, st)) return rc;
-    ps = blk;
-  }
-  if (!have_x) {
-    if (int rc = split_f16(x, s.rows, s.F, s.F, 0, kNone, nullptr, 0, xh, xl, s.ldf16, blk + kScaleBlockFloats, st)) return rc;
-    xs = blk + kScaleBlockFloats;
-  }
+  float* blk = static_cast<float*>(c.take(kBlocksBytes));
+  OperandPair pp = operand_pair(c, s.rows, s.ldp16, dP_hi, dP_lo, dp_scale);
+  OperandPair xp = operand_pair(c, s.rows, s.ldf16, x_hi, x_lo, x_scale);
+  if (!blk || !pp.ok() || !xp.ok()) return fail(SPOTV2_ERR_WORKSPACE, "proj_bwd_weight: workspace too small (%zu B)", ws_bytes);
+  SPOTV2_REQUIRE(!pp.own || dP_aug, "proj_bwd_weight: dP_aug or the complete pair (dP_hi, dP_lo, dp_scale)");
+  if (int rc = pp.split(dP_aug, s.rows, s.n_aug, s.ldp, 1, s.HC, s.ldp16, blk, st)) return rc;
+  if (int rc = xp.split(x, s.rows, s.F, s.F, 0, kNone, s.ldf16, blk + kScaleBlockFloats, st)) return rc;
   // contraction over the B*N node rows: both operands are MN-major ([K, rows]) for this product
-  F16Operand A{ph, pl, s.ldp16, ps + 2, s.HC}, B{xh, xl, s.ldf16, xs + 2, kNone};
+  F16Operand A{pp.hi, pp.lo, s.ldp16, pp.scale + 2, s.HC}, B{xp.hi, xp.lo, s.ldf16, xp.scale + 2, kNone};
   return gemm3x_f16(false, false, s.n_aug, s.F, s.rows, A, B, dW_aug, s.F, splits, 256 + 16, 0, c.p, c.left, st, nullptr, 0,
                     single_product(d));
 }
@@ -200,25 +215,17 @@ extern "C" int spotv2_proj_bwd_input(const spotv2_gat_desc* d, const float* dP_a
     return sgemm_simt(true, false, s.rows, s.F, s.n_aug, dP_aug, s.ldp, W_aug, s.F, dX, s.F, 1, ws, ws_bytes, st);
   }
   Carver c{static_cast<unsigned char*>(ws), ws ? ws_bytes : 0};
-  float* blk = static_cast<float*>(c.take(2 * kScaleBlockFloats * sizeof(float)));
-  const bool have_p = dP_hi && dP_lo && dp_scale;
-  void* ph = have_p ? const_cast<void*>(dP_hi) : c.take((size_t)s.rows * s.ldp16 * 2);
-  void* pl = have_p ? const_cast<void*>(dP_lo) : c.take((size_t)s.rows * s.ldp16 * 2);
-  void* wh = c.take((size_t)s.n_aug * s.ldf16 * 2);
-  void* wl = c.take((size_t)s.n_aug * s.ldf16 * 2);
-  if (!blk || !ph || !pl || !wh || !wl) return fail(SPOTV2_ERR_WORKSPACE, "proj_bwd_input: workspace too small (%zu B)", ws_bytes);
-  const float* ps = dp_scale;
-  if (!have_p) {
-    SPOTV2_REQUIRE(dP_aug, "proj_bwd_input: dP_aug or the complete pair (dP_hi, dP_lo, dp_scale)");
-    if (int rc = split_f16(dP_aug, s.rows, s.n_aug, s.ldp, 1, s.HC, nullptr, 0, ph, pl, s.ldp16, blk, st)) return rc;
-    ps = blk;
-  }
+  float* blk = static_cast<float*>(c.take(kBlocksBytes));
+  OperandPair pp = operand_pair(c, s.rows, s.ldp16, dP_hi, dP_lo, dp_scale), wp = operand_pair(c, s.n_aug, s.ldf16);
+  if (!blk || !pp.ok() || !wp.ok()) return fail(SPOTV2_ERR_WORKSPACE, "proj_bwd_input: workspace too small (%zu B)", ws_bytes);
+  SPOTV2_REQUIRE(!pp.own || dP_aug, "proj_bwd_input: dP_aug or the complete pair (dP_hi, dP_lo, dp_scale)");
+  if (int rc = pp.split(dP_aug, s.rows, s.n_aug, s.ldp, 1, s.HC, s.ldp16, blk, st)) return rc;
   // dX[rows, F] = dP_aug[rows, n_aug] . W_aug[n_aug, F] contracts over the dimension that carries dP's two
   // scale groups, so the groups' inverse scales (powers of two) are folded into the rows of W_aug before
   // W_aug is split with one scale of its own: (dP s_g) . (W / s_g * t) / t.
   float* wblk = blk + kScaleBlockFloats;
-  if (int rc = split_f16(W_aug, s.n_aug, s.F, s.F, 0, kNone, ps + 2, s.HC, wh, wl, s.ldf16, wblk, st)) return rc;
-  F16Operand A{ph, pl, s.ldp16, nullptr, kNone}, B{wh, wl, s.ldf16, wblk + 2, kNone};
+  if (int rc = split_f16(W_aug, s.n_aug, s.F, s.F, 0, kNone, pp.scale + 2, s.HC, wp.hi, wp.lo, s.ldf16, wblk, st)) return rc;
+  F16Operand A{pp.hi, pp.lo, s.ldp16, nullptr, kNone}, B{wp.hi, wp.lo, s.ldf16, wblk + 2, kNone};
   return gemm3x_f16(true, false, s.rows, s.F, s.n_aug, A, B, dX, s.F, 1, 256 + 16, 0, nullptr, 0, st, nullptr, 0,
                     single_product(d));
 }
