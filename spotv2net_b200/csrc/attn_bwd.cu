@@ -784,12 +784,8 @@ static int launch_bwd(AttnBwdArgs& a, float* dv, float* dbias, void* ws, size_t 
 }  // namespace spotv2
 
 namespace spotv2 {
-int bwd_diag_read(unsigned long long* host_out, int reset) {
-  SPOTV2_CUDA_OK(cudaMemcpyFromSymbol(host_out, g_bwd_counters, sizeof(unsigned long long) * kNumCounters));
-  if (reset) {
-    unsigned long long zeros[kNumCounters] = {0};
-    SPOTV2_CUDA_OK(cudaMemcpyToSymbol(g_bwd_counters, zeros, sizeof(zeros)));
-  }
+int bwd_diag_add(unsigned long long* host_out, int reset) {
+  if (int rc = diag_add(host_out, g_bwd_counters, reset)) return rc;
   if (int rc = bwd2_diag_add(host_out, reset)) return rc;       // whichever kernel ran contributes; the others add zeros
   return bwd3_diag_add(host_out, reset);
 }

@@ -32,19 +32,6 @@ int attn_fwd16_dispatch(const AttnFwdArgs& a, cudaStream_t st);
 bool attn_fwd16_fits(const AttnParams& p);                        // its shared-memory plan fits this problem
 int fwd16_diag_add(unsigned long long* host_out, int reset);     // adds its role counters into host_out[0..15]
 
-// ldmatrix: four 8x8 b16 matrices; lane l supplies the address of row (l & 7) of matrix (l >> 3)
-__device__ __forceinline__ void ldsm_x4(uint32_t addr, uint32_t& r0, uint32_t& r1, uint32_t& r2, uint32_t& r3) {
-  asm volatile("ldmatrix.sync.aligned.m8n8.x4.shared.b16 {%0,%1,%2,%3}, [%4];" : "=r"(r0), "=r"(r1), "=r"(r2), "=r"(r3) : "r"(addr));
-}
-__device__ __forceinline__ void ldsm_x4_t(uint32_t addr, uint32_t& r0, uint32_t& r1, uint32_t& r2, uint32_t& r3) {
-  asm volatile("ldmatrix.sync.aligned.m8n8.x4.trans.shared.b16 {%0,%1,%2,%3}, [%4];" : "=r"(r0), "=r"(r1), "=r"(r2), "=r"(r3) : "r"(addr));
-}
-// D(16x8, f32) += A(16x16, f16, row) * B(16x8, f16, col)
-__device__ __forceinline__ void mma_f16_k16(float (&c)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
-  asm("mma.sync.aligned.m16n8k16.row.col.f32.f16.f16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-      : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
-      : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
 // Byte offset of (row r, 16-byte chunk q) in a tile of 64-byte rows under the TMA 64B swizzle (chunk ^= (r >> 1) & 3);
 // eight consecutive rows of one chunk column land in eight distinct 16-byte bank groups (conflict-free ldmatrix).
 __device__ __host__ __forceinline__ uint32_t sw64(int r, int q) { return (uint32_t)(r * 64 + ((q ^ ((r >> 1) & 3)) << 4)); }

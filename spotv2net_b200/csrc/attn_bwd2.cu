@@ -116,46 +116,6 @@ Bwd2Plan make_plan(const AttnParams& p) {
   return s;
 }
 
-__device__ __forceinline__ void bar_sync_compute() { asm volatile("bar.sync 1, 384;" ::: "memory"); }
-__device__ __forceinline__ void mbar_arrive2(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ float ld_tile(const unsigned char* t, int r, int c) {
-  float v;
-  const uint32_t a = smem_u32(t) + r * 128 + ((((c >> 2) ^ (r & 7)) << 4) | ((c & 3) << 2));
-  asm("ld.shared.f32 %0, [%1];" : "=f"(v) : "r"(a));
-  return v;
-}
-// 32-bit shared-window address forms of the hot-loop accesses
-__device__ __forceinline__ float lds_u32(uint32_t a) {
-  float v;
-  asm volatile("ld.shared.f32 %0, [%1];" : "=f"(v) : "r"(a));
-  return v;
-}
-__device__ __forceinline__ int lds_i32(uint32_t a) {
-  int v;
-  asm volatile("ld.shared.s32 %0, [%1];" : "=r"(v) : "r"(a));
-  return v;
-}
-__device__ __forceinline__ float4 lds128_u32(uint32_t a) {
-  float4 v;
-  asm volatile("ld.shared.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(a));
-  return v;
-}
-__device__ __forceinline__ void sts_u32(uint32_t a, float v) {
-  asm volatile("st.shared.f32 [%0], %1;" ::"r"(a), "f"(v) : "memory");
-}
-__device__ __forceinline__ float2 lds64_u32(uint32_t a) {
-  float2 v;
-  asm volatile("ld.shared.v2.f32 {%0,%1}, [%2];" : "=f"(v.x), "=f"(v.y) : "r"(a));
-  return v;
-}
-// D(16x8, f32) += A(16x16, f16, row) * B(16x8, f16, col)
-__device__ __forceinline__ void mma_f16_16x8x16(float (&c)[4], const uint32_t (&a)[4], const uint32_t (&b)[2]) {
-  asm("mma.sync.aligned.m16n8k16.row.col.f32.f16.f16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-      : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
-      : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b[0]), "r"(b[1]));
-}
 // Two fp32 values -> packed fp16 "hi" pair and "lo" pair of the scaled values (hi + lo resolves 22 bits; s is a
 // power of two that maps the tensor's largest magnitude below 2^15).  The big products of this kernel run as
 // 3 x m16n8k16 on these pairs: same accuracy as the 3xTF32 split at half the tensor-pipe time (measured:
@@ -168,57 +128,6 @@ __device__ __forceinline__ void cvt_pair(float x0, float x1, float s, uint32_t& 
   hi = *reinterpret_cast<const uint32_t*>(&h);
   lo = *reinterpret_cast<const uint32_t*>(&l);
 }
-// tf32 split for mma.sync operands: the tensor core reads only the top 19 bits of a tf32 operand register
-// (verified by the parity tests), so "hi" is the raw fp32 pattern and only lo = x - trunc(x) costs ALU work.
-__device__ __forceinline__ void split_lean(float x, uint32_t& hi, uint32_t& lo) {
-  hi = __float_as_uint(x);
-  lo = __float_as_uint(x - __uint_as_float(hi & 0xffffe000u));
-}
-
-// Edge terms of the 16 rows [m0, m0+16) of a staged chunk for the k-blocks kb0, kb0+kb_stride, ... (8 k-steps
-// each): the same branch-free 3xTF32 loop as the forward (attn_common.cuh), results added into the tile.
-template <class Sink>
-__device__ __forceinline__ void edge_logits_part(const float* Ts, const float4* vfrag, int Fe, int KS, int m0, int lane,
-                                                 int kb0, int kb_stride, Sink&& sink) {
-  constexpr int kSlots = 8;
-  const int g = lane >> 2, t = lane & 3;
-  float acc[3][4];
-#pragma unroll
-  for (int pr = 0; pr < 3; ++pr)
-#pragma unroll
-    for (int q = 0; q < 4; ++q) acc[pr][q] = 0.f;
-  const float* r0 = Ts + (size_t)(m0 + g) * Fe;
-  const float* r1 = r0 + (size_t)8 * Fe;
-  const int kmax = Fe - 1;
-  for (int ks0 = kb0 * kSlots; ks0 < KS; ks0 += kb_stride * kSlots) {
-    float a[kSlots][4];
-    float4 bf[kSlots];
-#pragma unroll
-    for (int sl = 0; sl < kSlots; ++sl) {
-      const int k0 = min((ks0 + sl) * 8 + t, kmax), k1 = min((ks0 + sl) * 8 + t + 4, kmax);
-      a[sl][0] = lds_f32(r0 + k0);
-      a[sl][1] = lds_f32(r1 + k0);
-      a[sl][2] = lds_f32(r0 + k1);
-      a[sl][3] = lds_f32(r1 + k1);
-      bf[sl] = vfrag[(ks0 + sl) * 32 + lane];
-    }
-#pragma unroll
-    for (int sl = 0; sl < kSlots; ++sl) {
-      uint32_t ah[4], al[4];
-#pragma unroll
-      for (int q = 0; q < 4; ++q) split_tf32_trunc(a[sl][q], ah[q], al[q]);
-      const uint32_t bh[2] = {__float_as_uint(bf[sl].x), __float_as_uint(bf[sl].y)};
-      const uint32_t bl[2] = {__float_as_uint(bf[sl].z), __float_as_uint(bf[sl].w)};
-      mma_tf32_16x8x8(acc[0], al, bh);
-      mma_tf32_16x8x8(acc[1], ah, bl);
-      mma_tf32_16x8x8(acc[2], ah, bh);
-    }
-  }
-  const int n = 2 * t;
-#pragma unroll
-  for (int q = 0; q < 4; ++q) sink(m0 + g + ((q & 2) ? 8 : 0), n + (q & 1), (acc[0][q] + acc[1][q]) + acc[2][q]);
-}
-
 // FIX = true: the reference's default geometry (config/GNN_param.yaml: N=30, H=6, C=500, Fe=3*42, head mean) with
 // every size a compile-time constant: index arithmetic folds, loops get fixed trip counts and the kernel stops
 // re-reading its parameter block inside the hot loops.  FIX = false: the same code with run-time sizes.
@@ -348,7 +257,7 @@ gat_attn_bwd2_kernel(const AttnBwdArgs args, const Bwd2Plan pl_, const __grid_co
     auto publish = [&](bool async_done) {          // async_done: completion comes from the copy engine's tx count
       if (!async_done) {
         __syncwarp();
-        if (lane == 0) mbar_arrive2(&full[slot]);
+        if (lane == 0) mbar_arrive(&full[slot]);
       }
       if (++slot == pl.n_slots) { slot = 0; sph ^= 1; }
     };
@@ -532,25 +441,24 @@ gat_attn_bwd2_kernel(const AttnBwdArgs args, const Bwd2Plan pl_, const __grid_co
   const uint32_t l_row0 = (uint32_t)(((l_mt * 16 + 2 * g) * Fe + t) * 4);
   const uint32_t l_hoff0 = (uint32_t)(2 * t) * head_bytes;
 
-  // slot cursor: every compute warp walks the slots in the producer's order
+  // slot cursor: every compute warp walks the slots in the producer's order; the slot wait counts its polls (it reads no
+  // clock) and traps after kSlotWaitSpins of them
+  constexpr uint32_t kSlotWaitSpins = 1u << 24;
   int slot = 0;
   uint32_t sph = 0;
   auto wait_slot = [&]() -> uint32_t {
     const uint32_t bar = a_full + (uint32_t)slot * 8u;
-    uint32_t ok = 0, spins = 0;
+    bool ok;
+    uint32_t spins = 0;
     do {
-      asm volatile(
-          "{\n\t.reg .pred p;\n\t"
-          "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-          "selp.u32 %0, 1, 0, p;\n\t}"
-          : "=r"(ok) : "r"(bar), "r"(sph) : "memory");
-      if (!ok && ++spins > (1u << 24)) __trap();                 // lost transaction: fail loudly, never hang the box
+      ok = mbar_try_wait(bar, sph);
+      if (!ok && ++spins > kSlotWaitSpins) __trap();             // lost transaction: fail loudly, never hang the box
     } while (!ok);
     return a_slots + (uint32_t)slot * pl.slot_bytes;
   };
   auto release_slot = [&]() {
     __syncwarp();
-    if (lane == 0) mbar_arrive2(&empty[slot]);
+    if (lane == 0) mbar_arrive(&empty[slot]);
     if (++slot == pl.n_slots) { slot = 0; sph ^= 1; }
   };
 
@@ -584,7 +492,7 @@ gat_attn_bwd2_kernel(const AttnBwdArgs args, const Bwd2Plan pl_, const __grid_co
         const uint32_t off = (uint32_t)pc * pl.slot_bytes;
         const int n16 = (int)(min(pl.slot_bytes, tile_bytes - off) / 16u);
         float4* dst = reinterpret_cast<float4*>(reinterpret_cast<unsigned char*>(tile) + off);
-        for (int idx = tid; idx < n16; idx += kCT) dst[idx] = lds128_u32(sa + (uint32_t)idx * 16u);
+        for (int idx = tid; idx < n16; idx += kCT) dst[idx] = lds128a(sa + (uint32_t)idx * 16u);
         release_slot();
       }
     }
@@ -607,11 +515,11 @@ gat_attn_bwd2_kernel(const AttnBwdArgs args, const Bwd2Plan pl_, const __grid_co
           float4 bf[4];
 #pragma unroll
           for (int sl = 0; sl < 4; ++sl) {
-            a[sl][0] = lds_u32(r0 + ko + sl * 32);
-            a[sl][1] = lds_u32(r1 + ko + sl * 32);
-            a[sl][2] = lds_u32(r0 + ko + sl * 32 + 16);
-            a[sl][3] = lds_u32(r1 + ko + sl * 32 + 16);
-            bf[sl] = lds128_u32(vf + sl * 512);
+            a[sl][0] = ldsa(r0 + ko + sl * 32);
+            a[sl][1] = ldsa(r1 + ko + sl * 32);
+            a[sl][2] = ldsa(r0 + ko + sl * 32 + 16);
+            a[sl][3] = ldsa(r1 + ko + sl * 32 + 16);
+            bf[sl] = lds128a(vf + sl * 512);
           }
           if ((kb + 1) * 32 > Fe) {
             // k-steps reaching past Fe: whatever lies there (stale slot bytes) must not meet the zero B
@@ -638,29 +546,29 @@ gat_attn_bwd2_kernel(const AttnBwdArgs args, const Bwd2Plan pl_, const __grid_co
         // k half 0 stores into the alpha tile, k half 1 into the (idle) dz' tile; the softmax adds them: no atomics,
         // fixed summation order
         const int rl = l_mt * 16 + 2 * g, row_base = c * pl.chunk_rows + rl;
-        const int to0 = rl < rows ? lds_i32(a_toff + (uint32_t)row_base * 4u) : -1;
-        const int to1 = rl + 1 < rows ? lds_i32(a_toff + (uint32_t)(row_base + 1) * 4u) : -1;
+        const int to0 = rl < rows ? ldsa_s32(a_toff + (uint32_t)row_base * 4u) : -1;
+        const int to1 = rl + 1 < rows ? ldsa_s32(a_toff + (uint32_t)(row_base + 1) * 4u) : -1;
         const float v0 = (acc[0][0] + acc[1][0]) + acc[2][0], v1 = (acc[0][1] + acc[1][1]) + acc[2][1];
         const float v2 = (acc[0][2] + acc[1][2]) + acc[2][2], v3 = (acc[0][3] + acc[1][3]) + acc[2][3];
         const uint32_t tb = (l_kh == 0 ? a_tile : a_D) + l_hoff0;
         if (to0 >= 0) {
-          if (2 * t < H) sts_u32(tb + (uint32_t)to0, v0);
-          if (2 * t + 1 < H) sts_u32(tb + head_bytes + (uint32_t)to0, v1);
+          if (2 * t < H) stsa(tb + (uint32_t)to0, v0);
+          if (2 * t + 1 < H) stsa(tb + head_bytes + (uint32_t)to0, v1);
         }
         if (to1 >= 0) {
-          if (2 * t < H) sts_u32(tb + (uint32_t)to1, v2);
-          if (2 * t + 1 < H) sts_u32(tb + head_bytes + (uint32_t)to1, v3);
+          if (2 * t < H) stsa(tb + (uint32_t)to1, v2);
+          if (2 * t + 1 < H) stsa(tb + head_bytes + (uint32_t)to1, v3);
         }
       }
       release_slot();
     }
-    bar_sync_compute();
+    bar_sync<1, kCT>();
     lap(0);
     // ------------------------------------------------ S: softmax ------------------------------------------------
     // (the forward's record already IS the result of this phase: signed attention coefficients)
     if (!rec) {
       softmax_phase(p, asm_, tile, sd, 1.f, nullptr, pos_mask, tid, kCT, -1, 0, (nchunks > 0 && pl.ksplit == 2 && !use_terms) ? D : nullptr);
-      bar_sync_compute();
+      bar_sync<1, kCT>();
     }
     lap(1);
     // ------------------------------------------------ A: dalpha + softmax backward ------------------------------------------------
@@ -722,7 +630,7 @@ gat_attn_bwd2_kernel(const AttnBwdArgs args, const Bwd2Plan pl_, const __grid_co
 #pragma unroll
             for (int hf = 0; hf < 2; ++hf) {
               const uint32_t ad = da ^ ((4 * ks + 2 * hf) << 4);
-              float2 x0 = lds64_u32(ad), x1 = lds64_u32(ad + 1024);
+              float2 x0 = lds64a(ad), x1 = lds64a(ad + 1024);
               if (tail) {
                 const int c = cb * 32 + 16 * ks + 8 * hf + 2 * t;
                 if (c >= C) x0.x = x1.x = 0.f;
@@ -739,7 +647,7 @@ gat_attn_bwd2_kernel(const AttnBwdArgs args, const Bwd2Plan pl_, const __grid_co
               uint32_t bh[2], bl[2];
 #pragma unroll
               for (int hf = 0; hf < 2; ++hf) {
-                float2 y = lds64_u32((pa ^ ((4 * ks + 2 * hf) << 4)) + n * 1024);
+                float2 y = lds64a((pa ^ ((4 * ks + 2 * hf) << 4)) + n * 1024);
                 if (tail) {                                // never let padding bits (possibly NaN) meet the zeros above
                   const int c = cb * 32 + 16 * ks + 8 * hf + 2 * t;
                   if (c >= C) y.x = 0.f;
@@ -747,9 +655,9 @@ gat_attn_bwd2_kernel(const AttnBwdArgs args, const Bwd2Plan pl_, const __grid_co
                 }
                 cvt_pair(y.x, y.y, s_P, bh[hf], bl[hf]);
               }
-              mma_f16_16x8x16(cacc[n], al[ks], bh);        // small terms first
-              mma_f16_16x8x16(cacc[n], ah[ks], bl);
-              mma_f16_16x8x16(cacc[n], ah[ks], bh);
+              mma_f16_k16(cacc[n], al[ks], bh[0], bh[1]);  // small terms first
+              mma_f16_k16(cacc[n], ah[ks], bl[0], bl[1]);
+              mma_f16_k16(cacc[n], ah[ks], bh[0], bh[1]);
             }
           }
           }
@@ -854,7 +762,7 @@ gat_attn_bwd2_kernel(const AttnBwdArgs args, const Bwd2Plan pl_, const __grid_co
           }
       }
     }
-    bar_sync_compute();
+    bar_sync<1, kCT>();
     lap(2);
     for (int idx = tid; idx < H * N; idx += kCT) {       // ds_j = sum over both target tiles
       const int h = idx / N, j = idx - h * N;
@@ -891,7 +799,7 @@ gat_attn_bwd2_kernel(const AttnBwdArgs args, const Bwd2Plan pl_, const __grid_co
           const int r4 = rbeg + 4 * t;
           int to[4];
 #pragma unroll
-          for (int k = 0; k < 4; ++k) to[k] = (r4 + k < rend && g < H) ? lds_i32(trow + (uint32_t)(r4 + k) * 4u) : -1;
+          for (int k = 0; k < 4; ++k) to[k] = (r4 + k < rend && g < H) ? ldsa_s32(trow + (uint32_t)(r4 + k) * 4u) : -1;
           float a[2][2][4];                                                   // [tile][k-step][fragment register]
 #pragma unroll
           for (int uu = 0; uu < 2; ++uu) {
@@ -899,15 +807,15 @@ gat_attn_bwd2_kernel(const AttnBwdArgs args, const Bwd2Plan pl_, const __grid_co
 #pragma unroll
             for (int ks = 0; ks < 2; ++ks) {
               const uint32_t ta = ta0 + (uint32_t)(2 * ks) * rowb, tb = ta + rowb;
-              a[uu][ks][0] = lds_u32(ta);
-              a[uu][ks][1] = lds_u32(ta + 32);
-              a[uu][ks][2] = lds_u32(tb);
-              a[uu][ks][3] = lds_u32(tb + 32);
+              a[uu][ks][0] = ldsa(ta);
+              a[uu][ks][1] = ldsa(ta + 32);
+              a[uu][ks][2] = ldsa(tb);
+              a[uu][ks][3] = ldsa(tb + 32);
             }
           }
           float bv[4];
 #pragma unroll
-          for (int k = 0; k < 4; ++k) bv[k] = to[k] >= 0 ? lds_u32(dgh + (uint32_t)to[k]) : 0.f;
+          for (int k = 0; k < 4; ++k) bv[k] = to[k] >= 0 ? ldsa(dgh + (uint32_t)to[k]) : 0.f;
           if (rend < rbeg + 16) {                // rows past the chunk's end hold stale slot bytes
 #pragma unroll
             for (int uu = 0; uu < 2; ++uu)
@@ -963,18 +871,18 @@ gat_attn_bwd2_kernel(const AttnBwdArgs args, const Bwd2Plan pl_, const __grid_co
 #pragma unroll
           for (int q = 0; q < 4; ++q) acc[pr][q] = 0.f;
         auto kstep = [&](int ra, int rb, uint32_t ta, uint32_t tb) {
-          const int to0 = (ra < rend && g < H) ? lds_i32(trow + (uint32_t)ra * 4u) : -1;
-          const int to1 = (rb < rend && g < H) ? lds_i32(trow + (uint32_t)rb * 4u) : -1;
-          const float b0 = to0 >= 0 ? lds_u32(dgh + (uint32_t)to0) : 0.f;
-          const float b1 = to1 >= 0 ? lds_u32(dgh + (uint32_t)to1) : 0.f;
+          const int to0 = (ra < rend && g < H) ? ldsa_s32(trow + (uint32_t)ra * 4u) : -1;
+          const int to1 = (rb < rend && g < H) ? ldsa_s32(trow + (uint32_t)rb * 4u) : -1;
+          const float b0 = to0 >= 0 ? ldsa(dgh + (uint32_t)to0) : 0.f;
+          const float b1 = to1 >= 0 ? ldsa(dgh + (uint32_t)to1) : 0.f;
           uint32_t bh[2], bl[2];
           split_lean(b0, bh[0], bl[0]);
           split_lean(b1, bh[1], bl[1]);
           float a[4];
-          a[0] = lds_u32(ta);
-          a[1] = lds_u32(ta + 32);
-          a[2] = lds_u32(tb);
-          a[3] = lds_u32(tb + 32);
+          a[0] = ldsa(ta);
+          a[1] = ldsa(ta + 32);
+          a[2] = ldsa(tb);
+          a[3] = ldsa(tb + 32);
           if (partial) {                         // rows past the chunk's end hold stale slot bytes
             if (ra >= rend) a[0] = a[1] = 0.f;
             if (rb >= rend) a[2] = a[3] = 0.f;
@@ -1003,7 +911,7 @@ gat_attn_bwd2_kernel(const AttnBwdArgs args, const Bwd2Plan pl_, const __grid_co
     }
     lap(5);
     // (the dP staging tiles reuse the dz' tile: every warp must be done reading it - phase V, or the edge_mode 1 copy-out)
-    if (P16 && pl.stage_ok) bar_sync_compute();
+    if (P16 && pl.stage_ok) bar_sync<1, kCT>();
     // ------------------------------------------------ D: dP = g alpha^T dO ------------------------------------------------
     for (int r = 0; r < pl.n_rounds; ++r) {
       const int h0 = r * pl.hpr;
@@ -1054,7 +962,7 @@ gat_attn_bwd2_kernel(const AttnBwdArgs args, const Bwd2Plan pl_, const __grid_co
             const uint32_t ta = sa + (uint32_t)k * kTile;
             float sum = 0.f;
             for (int rr = 0; rr < N; ++rr)
-              sum += lds_u32(ta + rr * 128 + ((((lane >> 2) ^ (rr & 7)) << 4) | ((lane & 3) << 2)));
+              sum += ldsa(ta + rr * 128 + ((((lane >> 2) ^ (rr & 7)) << 4) | ((lane & 3) << 2)));
             const int c = (cb0 + kc) * 32 + lane;
             if (c < C) dbias_s[(p.concat ? (h0 + khl) * C : 0) + c] += sum;       // one owner lane per column
           }
@@ -1096,15 +1004,15 @@ gat_attn_bwd2_kernel(const AttnBwdArgs args, const Bwd2Plan pl_, const __grid_co
               for (int n = 0; n < 4; ++n) {
                 // k pairs (2t, 2t+1) and (2t+8, 2t+9) of this k16 step = dO rows 16ks + ...; column 8n + g
                 const uint32_t a0 = (tb0 ^ (n << 5)) + ks * 2048, a1 = (tb1 ^ (n << 5)) + ks * 2048;
-                const float x0 = lds_u32(a0), x1 = lds_u32(a1), x2 = lds_u32(a0 + 1024), x3 = lds_u32(a1 + 1024);
+                const float x0 = ldsa(a0), x1 = ldsa(a1), x2 = ldsa(a0 + 1024), x3 = ldsa(a1 + 1024);
                 uint32_t bh[2], bl[2];
                 cvt_pair(x0, x1, s_dO, bh[0], bl[0]);
                 cvt_pair(x2, x3, s_dO, bh[1], bl[1]);
                 if (!(P16 && SINGLE)) {
-                  mma_f16_16x8x16(cacc[n], al[ks], bh);    // small terms first
-                  mma_f16_16x8x16(cacc[n], ah[ks], bl);
+                  mma_f16_k16(cacc[n], al[ks], bh[0], bh[1]);    // small terms first
+                  mma_f16_k16(cacc[n], ah[ks], bl[0], bl[1]);
                 }
-                mma_f16_16x8x16(cacc[n], ah[ks], bh);
+                mma_f16_k16(cacc[n], ah[ks], bh[0], bh[1]);
               }
             }
             if (P16 && pl.stage_ok) {
@@ -1135,7 +1043,7 @@ gat_attn_bwd2_kernel(const AttnBwdArgs args, const Bwd2Plan pl_, const __grid_co
                   cur_h[hf][n] = *reinterpret_cast<const uint32_t*>(&hh);
                   cur_l[hf][n] = *reinterpret_cast<const uint32_t*>(&ll);
                 }
-              if (lane == 0) tma_store_wait_read();                 // the previous tile's store has read the staging
+              if (lane == 0) bulk_wait_read();                      // the previous tile's store has read the staging
               __syncwarp();
 #pragma unroll
               for (int hf = 0; hf < 2; ++hf) {
@@ -1145,8 +1053,8 @@ gat_attn_bwd2_kernel(const AttnBwdArgs args, const Bwd2Plan pl_, const __grid_co
                   for (int q = 0; q < 4; ++q) {                     // staging chunk q <- tile chunk q (or q - 1, chunk 0 <- the carried one)
                     const uint32_t vh = !shift ? cur_h[hf][q] : (q == 0 ? carry_h[hf] : cur_h[hf][q - 1]);
                     const uint32_t vl = !shift ? cur_l[hf][q] : (q == 0 ? carry_l[hf] : cur_l[hf][q - 1]);
-                    asm volatile("st.shared.b32 [%0], %1;" ::"r"(stg + sw64(rr, q) + 4u * t), "r"(vh) : "memory");
-                    if (!SINGLE) asm volatile("st.shared.b32 [%0], %1;" ::"r"(stg + sw64(rows_m + rr, q) + 4u * t), "r"(vl) : "memory");
+                    stsa_b32(stg + sw64(rr, q) + 4u * t, vh);
+                    if (!SINGLE) stsa_b32(stg + sw64(rows_m + rr, q) + 4u * t, vl);
                   }
                 }
                 carry_h[hf] = cur_h[hf][3];
@@ -1157,14 +1065,14 @@ gat_attn_bwd2_kernel(const AttnBwdArgs args, const Bwd2Plan pl_, const __grid_co
               if (lane == 0) tma_store_4d(m == 0 ? &tmD0 : &tmD1, stg, cb * 32 - (shift ? 8 : 0), b * N + 16 * m, h, 0);
               if (((h * Cp) & 15) != 0 && cb == n_cb - 1 && n_cb > 1 && 32 * n_cb - 8 < Cp) {
                 // the carried last chunk still holds columns the head owns: one more box, only its first chunk inside Cp
-                if (lane == 0) tma_store_wait_read();
+                if (lane == 0) bulk_wait_read();
                 __syncwarp();
 #pragma unroll
                 for (int hf = 0; hf < 2; ++hf) {
                   const int rr = g + 8 * hf;
                   if (rr < rows_m) {
-                    asm volatile("st.shared.b32 [%0], %1;" ::"r"(stg + sw64(rr, 0) + 4u * t), "r"(carry_h[hf]) : "memory");
-                    if (!SINGLE) asm volatile("st.shared.b32 [%0], %1;" ::"r"(stg + sw64(rows_m + rr, 0) + 4u * t), "r"(carry_l[hf]) : "memory");
+                    stsa_b32(stg + sw64(rr, 0) + 4u * t, carry_h[hf]);
+                    if (!SINGLE) stsa_b32(stg + sw64(rows_m + rr, 0) + 4u * t, carry_l[hf]);
                   }
                 }
                 fence_proxy_async();
@@ -1249,15 +1157,15 @@ gat_attn_bwd2_kernel(const AttnBwdArgs args, const Bwd2Plan pl_, const __grid_co
         release_slot();
       }
     }
-    if (P16 && pl.stage_ok && lane == 0) tma_store_wait_read();   // the engine has read this warp's last dP staging tile
-    bar_sync_compute();                                   // every warp is done with alpha and with the dz' tile
+    if (P16 && pl.stage_ok && lane == 0) bulk_wait_read();        // the engine has read this warp's last dP staging tile
+    bar_sync<1, kCT>();                                   // every warp is done with alpha and with the dz' tile
     if (!use_terms) {                                     // (a kept tile is copied over the whole of it)
       for (int idx = tid; idx < tile_floats; idx += kCT) tile[idx] = 0.f;      // next graph's logits accumulate into zeros
-      bar_sync_compute();
+      bar_sync<1, kCT>();
     }
     lap(4);
   }
-  if (P16 && pl.stage_ok && lane == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");   // this lane's dP stores have landed
+  if (P16 && pl.stage_ok && lane == 0) bulk_wait();                                                // this lane's dP stores have landed
 #ifdef SPOTV2_BRINGUP
   if (tid == 0)
     for (int k = 0; k < 6; ++k) atomicAdd(&g_bwd2_counters[k], (unsigned long long)ph[k]);
@@ -1380,14 +1288,7 @@ int launch_attn_bwd2(AttnBwdArgs& a, float* dv, float* dbias, void* ws, size_t w
 }
 
 int bwd2_diag_add(unsigned long long* host_out, int reset) {
-  unsigned long long tmp[kNumCounters];
-  SPOTV2_CUDA_OK(cudaMemcpyFromSymbol(tmp, g_bwd2_counters, sizeof(tmp)));
-  for (int k = 0; k < kNumCounters; ++k) host_out[k] += tmp[k];
-  if (reset) {
-    unsigned long long zeros[kNumCounters] = {0};
-    SPOTV2_CUDA_OK(cudaMemcpyToSymbol(g_bwd2_counters, zeros, sizeof(zeros)));
-  }
-  return SPOTV2_OK;
+  return diag_add(host_out, g_bwd2_counters, reset);
 }
 
 }  // namespace spotv2

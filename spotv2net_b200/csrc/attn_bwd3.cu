@@ -112,75 +112,18 @@ Bwd3Plan make_plan3(const AttnParams& p) {
   return s;
 }
 
-// ---- small PTX helpers -----------------------------------------------------------------------------------------------
-__device__ __forceinline__ void bar_group(int id, int count) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(count) : "memory"); }
-__device__ __forceinline__ float4 lds128a(uint32_t a) {
-  float4 v;
-  asm volatile("ld.shared.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(a));
-  return v;
-}
-__device__ __forceinline__ void sts128a(uint32_t a, float4 v) {
-  asm volatile("st.shared.v4.f32 [%0], {%1,%2,%3,%4};" ::"r"(a), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w) : "memory");
-}
-__device__ __forceinline__ float2 lds64a(uint32_t a) {
-  float2 v;
-  asm volatile("ld.shared.v2.f32 {%0,%1}, [%2];" : "=f"(v.x), "=f"(v.y) : "r"(a));
-  return v;
-}
-__device__ __forceinline__ float ldsa(uint32_t a) {
-  float v;
-  asm volatile("ld.shared.f32 %0, [%1];" : "=f"(v) : "r"(a));
-  return v;
-}
-__device__ __forceinline__ void stsa(uint32_t a, float v) { asm volatile("st.shared.f32 [%0], %1;" ::"r"(a), "f"(v) : "memory"); }
 // round-to-nearest (ties away) onto the tf32 grid: what the tensor core would see of x, made explicit
 __device__ __forceinline__ float rn_tf32(float x) { return __uint_as_float((__float_as_uint(x) + 0x1000u) & 0xffffe000u); }
 // what the tensor core reads of an fp32 bit pattern handed to it as tf32: the top 19 bits
 __device__ __forceinline__ float tr_tf32(float x) { return __uint_as_float(__float_as_uint(x) & 0xffffe000u); }
-__device__ __forceinline__ void tma_load_3d_hint(uint32_t smem_dst, const CUtensorMap* tm, int c0, int c1, int c2, uint32_t bar,
-                                                 uint64_t hint) {
-  asm volatile(
-      "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1, {%3, %4, %5}], "
-      "[%2], %6;" ::"r"(smem_dst),
-      "l"(tm), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "l"(hint)
-      : "memory");
-}
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&r)[16]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]), "=r"(r[9]),
-        "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-      : "r"(taddr));
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
-// mbarrier by 32-bit shared address
+// mbarrier wait of this kernel: up to kWaitSpins polls, then the shared bounded wait with kWaitSleepNs sleeps.  The polls
+// are a loop of their own because in this form they stay a loop; inside mbar_wait_bounded the compiler unrolls all 64.
+constexpr int kWaitSpins = 64;
+constexpr unsigned kWaitSleepNs = 32;
 __device__ __forceinline__ void bar_wait(uint32_t bar, uint32_t parity) {
-  uint32_t ok = 0;
-  for (int spin = 0; spin < 64 && !ok; ++spin)
-    asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                 : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
-  if (ok) return;
-  const long long t0 = clock64();
-  while (true) {
-    asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                 : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
-    if (ok) return;
-    __nanosleep(32);
-    if (clock64() - t0 > 4000000000LL) __trap();        // a lost arrival fails loudly instead of hanging the box
-  }
-}
-__device__ __forceinline__ void bar_arrive(uint32_t bar) { asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory"); }
-__device__ __forceinline__ void bar_expect_tx(uint32_t bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void bar_commit(uint32_t bar) {      // arrives when every tcgen05.mma issued so far has retired
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void bulk_g2s_a(uint32_t smem_dst, const void* gmem_src, uint32_t bytes, uint32_t bar, uint64_t hint) {
-  asm volatile(
-      "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1], %2, [%3], %4;" ::"r"(smem_dst),
-      "l"(gmem_src), "r"(bytes), "r"(bar), "l"(hint)
-      : "memory");
+  bool ok = false;
+  for (int spin = 0; spin < kWaitSpins && !ok; ++spin) ok = mbar_try_wait(bar, parity);
+  if (!ok) mbar_wait_bounded<0, kWaitSleepNs, kWaitTrapCycles>(bar, parity);
 }
 
 // Diagnostics (spotv2_diag_counters, entries 16..31 when this kernel ran): cycles one sampling thread per role spent
@@ -191,9 +134,7 @@ __device__ __forceinline__ void bulk_g2s_a(uint32_t smem_dst, const void* gmem_s
 // 13 softmax: softmax        14 softmax: dalpha ready   15 softmax: TMEM dump + softmax backward
 __device__ unsigned long long g_bwd3_counters[kNumCounters];
 __device__ __forceinline__ void bar_wait_t(uint32_t bar, uint32_t parity, long long& acc) {
-  const long long t0 = clock64();
-  bar_wait(bar, parity);
-  acc += clock64() - t0;
+  wait_timed(acc, [&] { bar_wait(bar, parity); });
 }
 
 // a cursor over the slot ring: every role steps through the producer's slot order
@@ -278,20 +219,20 @@ gat_attn_bwd3_kernel(const AttnBwdArgs args, const Bwd3Plan pl, const __grid_con
           const uint32_t dst = acquire(), full = BAR(kBarFull + cur.slot);
           const uint32_t off = (uint32_t)pc * pl.slot_bytes;
           const uint32_t bytes = min(pl.slot_bytes, pl.tile_bytes - off);
-          bar_expect_tx(full, bytes);
-          bulk_g2s_a(dst, reinterpret_cast<const unsigned char*>(p.edge_terms + (size_t)b * tile_floats) + off, bytes, full, kEvictFirst);
+          mbar_expect_tx(full, bytes);
+          bulk_g2s_hint(dst, reinterpret_cast<const unsigned char*>(p.edge_terms + (size_t)b * tile_floats) + off, bytes, full, kEvictFirst);
           cur.advance();
         }
         for (int kb = 0; kb < pl.n_kb; ++kb) {                                   // A: P tiles of all heads + dout, 16 channels
           const uint32_t dst = acquire(), full = BAR(kBarFull + cur.slot);
-          bar_expect_tx(full, pl.a_bytes);
+          mbar_expect_tx(full, pl.a_bytes);
           for (int h = 0; h < H; ++h) tma_load_3d_hint(dst + (uint32_t)h * kPTile, &tmP, h * C + kb * kKB, 0, b, full, kEvictFirst);
           tma_load_3d_hint(dst + (uint32_t)H * kPTile, &tmG, kb * kKB, 0, b, full, kEvictNormal);
           cur.advance();
         }
         for (int cb = 0; cb < pl.n_cb; ++cb) {                                   // G: dout again, MN-major boxes (L2 hits)
           const uint32_t dst = acquire(), full = BAR(kBarFull + cur.slot);
-          bar_expect_tx(full, 4u * kGTile);
+          mbar_expect_tx(full, 4u * kGTile);
           for (int k = 0; k < 4; ++k) tma_load_3d_hint(dst + (uint32_t)k * kGTile, &tmGt, cb * kCB + k * 32, 0, b, full, kEvictFirst);
           cur.advance();
         }
@@ -300,8 +241,8 @@ gat_attn_bwd3_kernel(const AttnBwdArgs args, const Bwd3Plan pl, const __grid_con
           int rows = p.R - c * pl.chunk_rows;
           if (rows > pl.chunk_rows) rows = pl.chunk_rows;
           const uint32_t bytes = (uint32_t)rows * (uint32_t)Fe * 4u;
-          bar_expect_tx(full, bytes);
-          bulk_g2s_a(dst, p.edge_rows + ((size_t)b * p.R + (size_t)c * pl.chunk_rows) * Fe, bytes, full, kEvictFirst);
+          mbar_expect_tx(full, bytes);
+          bulk_g2s_hint(dst, p.edge_rows + ((size_t)b * p.R + (size_t)c * pl.chunk_rows) * Fe, bytes, full, kEvictFirst);
           cur.advance();
         }
       }
@@ -339,11 +280,11 @@ gat_attn_bwd3_kernel(const AttnBwdArgs args, const Bwd3Plan pl, const __grid_con
               umma_tf32(tA + (uint32_t)blk * 64u, a_lo_, b_hi, id_a32, 1u);
             }
           }
-          bar_commit(BAR(kBarEmpty + cur.slot));
-          bar_commit(BAR(kBarLoEmpty + li));
+          umma_commit(BAR(kBarEmpty + cur.slot));
+          umma_commit(BAR(kBarLoEmpty + li));
           cur.advance();
         }
-        bar_commit(BAR(kBarDAFull));
+        umma_commit(BAR(kBarDAFull));
         // ---- phase D: dP[(h,j), c] per block of 128 channels; A = alpha^T (K-major), B = dout (channel-major)
         bar_wait_t(BAR(kBarAlphaFull), gph, w_al);
         for (int cb = 0; cb < pl.n_cb; ++cb, ++lo_n, ++d_n) {
@@ -365,12 +306,12 @@ gat_attn_bwd3_kernel(const AttnBwdArgs args, const Bwd3Plan pl, const __grid_con
               umma_tf32(td, a_hi, b_hi, id_d, 1u);
             }
           }
-          bar_commit(BAR(kBarEmpty + cur.slot));
-          bar_commit(BAR(kBarLoEmpty + li));
-          bar_commit(BAR(kBarDTFull));
+          umma_commit(BAR(kBarEmpty + cur.slot));
+          umma_commit(BAR(kBarLoEmpty + li));
+          umma_commit(BAR(kBarDTFull));
           cur.advance();
         }
-        bar_commit(BAR(kBarAlphaEmpty));
+        umma_commit(BAR(kBarAlphaEmpty));
         cur.advance(pl.nchunks);
       }
       atomicAdd(&g_bwd3_counters[1], (unsigned long long)w_a);
@@ -409,7 +350,7 @@ gat_attn_bwd3_kernel(const AttnBwdArgs args, const Bwd3Plan pl, const __grid_con
       }
     };
     for (int it = 0; it < my_graphs; ++it) {
-      bar_group(3, kStT);                                                         // both warps know every fill either has seen
+      bar_sync<3, kStT>();                                                        // both warps know every fill either has seen
       if (has_v && it > 0) bar_wait_t(BAR(kBarVDone), (uint32_t)(it - 1) & 1u, w_full);
       bar_wait_t(BAR(kBarTDone), (uint32_t)it & 1u, w_full);
       cur.advance(pl.t_pieces);
@@ -423,7 +364,7 @@ gat_attn_bwd3_kernel(const AttnBwdArgs args, const Bwd3Plan pl, const __grid_con
           else lo_pass(sa, lo, 4 * kGTile / 16, 0x7fffffff);
           fence_proxy_async();
           __syncwarp();
-          if (lane == 0) bar_arrive(BAR(kBarLoFull + sw));
+          if (lane == 0) mbar_arrive(BAR(kBarLoFull + sw));
           t_lo += clock64() - t0;
         }
         cur.advance();
@@ -490,8 +431,8 @@ gat_attn_bwd3_kernel(const AttnBwdArgs args, const Bwd3Plan pl, const __grid_con
 #pragma unroll
               for (int k = 0; k < 4; ++k) {
                 const uint32_t o = (uint32_t)lane * 64u + (((uint32_t)k ^ sw_) << 4);
-                asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" ::"r"(stg + o), "r"(hi[4 * k]), "r"(hi[4 * k + 1]), "r"(hi[4 * k + 2]), "r"(hi[4 * k + 3]) : "memory");
-                asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" ::"r"(stg + 2048u + o), "r"(lo[4 * k]), "r"(lo[4 * k + 1]), "r"(lo[4 * k + 2]), "r"(lo[4 * k + 3]) : "memory");
+                sts128a_b32(stg + o, hi[4 * k], hi[4 * k + 1], hi[4 * k + 2], hi[4 * k + 3]);
+                sts128a_b32(stg + 2048u + o, lo[4 * k], lo[4 * k + 1], lo[4 * k + 2], lo[4 * k + 3]);
               }
               __syncwarp();
               const int pc = (lane & 7) * 4;                                        // first of this lane's 4 channels in the piece
@@ -501,8 +442,8 @@ gat_attn_bwd3_kernel(const AttnBwdArgs args, const Bwd3Plan pl, const __grid_con
                 for (int it8 = 0; it8 < 8; ++it8) {
                   const int j = 4 * it8 + (lane >> 3);
                   const uint32_t o = (uint32_t)j * 64u + ((((uint32_t)(lane & 7) >> 1) ^ (uint32_t)((j >> 1) & 3)) << 4) + (uint32_t)(lane & 1) * 8u;
-                  asm volatile("ld.shared.v2.b32 {%0,%1}, [%2];" : "=r"(vh[it8].x), "=r"(vh[it8].y) : "r"(stg + o));
-                  asm volatile("ld.shared.v2.b32 {%0,%1}, [%2];" : "=r"(vl[it8].x), "=r"(vl[it8].y) : "r"(stg + 2048u + o));
+                  vh[it8] = lds64a_b32(stg + o);
+                  vl[it8] = lds64a_b32(stg + 2048u + o);
                 }
 #pragma unroll
                 for (int it8 = 0; it8 < 8; ++it8) {
@@ -526,12 +467,12 @@ gat_attn_bwd3_kernel(const AttnBwdArgs args, const Bwd3Plan pl, const __grid_con
           }
         }
         tc_fence_before();
-        bar_group(2, kDeT);
-        if (de == 0) bar_arrive(BAR(kBarDTEmpty));
+        bar_sync<2, kDeT>();
+        if (de == 0) mbar_arrive(BAR(kBarDTEmpty));
         t_de += clock64() - t0;
       }
     }
-    bar_group(2, kDeT);
+    bar_sync<2, kDeT>();
     for (int c = de; c < C; c += kDeT) args.dbias_part[(size_t)blockIdx.x * p.ldo + c] = ldsa(a_dbias + (uint32_t)c * 4u);
     if (de == 0) {
       atomicAdd(&g_bwd3_counters[2], (unsigned long long)w_dt);
@@ -575,17 +516,17 @@ gat_attn_bwd3_kernel(const AttnBwdArgs args, const Bwd3Plan pl, const __grid_con
         const uint32_t sa = a_slots + (uint32_t)cur.slot * pl.slot_bytes, off = (uint32_t)pc * pl.slot_bytes;
         const int n16 = (int)(min(pl.slot_bytes, pl.tile_bytes - off) / 16u);
         for (int idx = tid; idx < n16; idx += kSmT) sts128a(a_work + off + (uint32_t)idx * 16u, lds128a(sa + (uint32_t)idx * 16u));
-        bar_group(1, kSmT);
-        if (tid == 0) bar_arrive(BAR(kBarEmpty + cur.slot));
+        bar_sync<1, kSmT>();
+        if (tid == 0) mbar_arrive(BAR(kBarEmpty + cur.slot));
         cur.advance();
       }
-      if (tid == 0) bar_arrive(BAR(kBarTDone));
+      if (tid == 0) mbar_arrive(BAR(kBarTDone));
       cur.advance(pl.n_kb + pl.n_cb);                                            // on to this graph's V slots
       for (int k = 0; k < 2; ++k) {
         const int idx = tid + k * kSmT;
         if (idx < N * 2 * H) stsa(a_sd + (uint32_t)idx * 4u, sd_reg[k]);
       }
-      bar_group(1, kSmT);
+      bar_sync<1, kSmT>();
       // ------------------------------------------------ softmax (thread = head h, target i) ------------------------------------------------
       const long long t_s0 = clock64();
       uint32_t mask = 0u, keep = 0xffffffffu;
@@ -621,8 +562,8 @@ gat_attn_bwd3_kernel(const AttnBwdArgs args, const Bwd3Plan pl, const __grid_con
         }
       }
       fence_proxy_async();
-      bar_group(1, kSmT);
-      if (tid == 0) bar_arrive(BAR(kBarAlphaFull));
+      bar_sync<1, kSmT>();
+      if (tid == 0) mbar_arrive(BAR(kBarAlphaFull));
       // alpha column of this thread: kept in registers across the TMEM dump (which overwrites the work tile)
       float al[32];
 #pragma unroll
@@ -632,7 +573,7 @@ gat_attn_bwd3_kernel(const AttnBwdArgs args, const Bwd3Plan pl, const __grid_con
       bar_wait_t(BAR(kBarDAFull), gph, w_da);
       const long long t_b0 = clock64();
       tc_fence_after();
-      bar_group(1, kSmT);                                                        // every alpha column is in registers
+      bar_sync<1, kSmT>();                                                       // every alpha column is in registers
       if (h < H) {
         const uint32_t taddr = tA + (uint32_t)(h >> 2) * 64u + ((uint32_t)((h & 3) * 32) << 16);
         const uint32_t row = a_work + (uint32_t)((h * N + lane) * kNS3) * 4u;    // lane = source j
@@ -653,8 +594,8 @@ gat_attn_bwd3_kernel(const AttnBwdArgs args, const Bwd3Plan pl, const __grid_con
         }
       }
       tc_fence_before();
-      bar_group(1, kSmT);
-      if (tid == 0) bar_arrive(BAR(kBarDAEmpty));
+      bar_sync<1, kSmT>();
+      if (tid == 0) mbar_arrive(BAR(kBarDAEmpty));
       // ------------------------------------------------ softmax / LeakyReLU backward (thread = head h, target i) ------------------------------------------------
       float share = 0.f;
       if (on) {
@@ -683,7 +624,7 @@ gat_attn_bwd3_kernel(const AttnBwdArgs args, const Bwd3Plan pl, const __grid_con
         if (args.dsd) args.dsd[((size_t)b * N + i) * 2 * H + H + h] = dd;
         else args.dP_aug[((size_t)b * N + i) * p.ldp + HC + H + h] = dd;
       }
-      bar_group(1, kSmT);
+      bar_sync<1, kSmT>();
       if (on) {                                                                  // ds_j = row sum of dz (thread = head h, source j = lane)
         const uint32_t row = a_work + (uint32_t)((h * N + lane) * kNS3) * 4u;
         float ds = 0.f;
@@ -692,18 +633,18 @@ gat_attn_bwd3_kernel(const AttnBwdArgs args, const Bwd3Plan pl, const __grid_con
         if (args.dsd) args.dsd[((size_t)b * N + lane) * 2 * H + h] = ds;
         else args.dP_aug[((size_t)b * N + lane) * p.ldp + HC + h] = ds;
       }
-      bar_group(1, kSmT);
+      bar_sync<1, kSmT>();
       if (on) {                                                                  // dz' = dz + dz_ii / (N - 1) off the diagonal, 0 on it
         for (int j = 0; j < N; ++j) {
           const uint32_t a = col + (uint32_t)j * (kNS3 * 4);
           stsa(a, j == i ? 0.f : ldsa(a) + share);
         }
       }
-      bar_group(1, kSmT);
+      bar_sync<1, kSmT>();
       if (p.dterms_out) {                                                        // edge_mode 1: d(edge terms) leaves in the tile layout
         float4* dst = reinterpret_cast<float4*>(p.dterms_out + (size_t)b * tile_floats);
         for (int idx = tid; idx < tile_floats / 4; idx += kSmT) dst[idx] = lds128a(a_work + (uint32_t)idx * 16u);
-        bar_group(1, kSmT);
+        bar_sync<1, kSmT>();
       }
       t_sb += clock64() - t_b0;
       // ------------------------------------------------ V: dv += dz'^T . edge rows (exact fp32 on the CUDA cores) ------------------------------------------------
@@ -731,7 +672,7 @@ gat_attn_bwd3_kernel(const AttnBwdArgs args, const Bwd3Plan pl, const __grid_con
 #pragma unroll
             for (int u = 0; u < 2; ++u) {
               const int r = min(rb + u * kSmWarps, rows - 1);
-              asm volatile("ld.shared.s32 %0, [%1];" : "=r"(off[u]) : "r"(a_table + (uint32_t)(c * pl.chunk_rows + r) * 4u));
+              off[u] = ldsa_s32(a_table + (uint32_t)(c * pl.chunk_rows + r) * 4u);
               e0[u] = f0_on ? lds64a(sa + (uint32_t)(r * Fe + f0) * 4u) : make_float2(0.f, 0.f);
               e1[u] = f1_on ? lds64a(sa + (uint32_t)(r * Fe + f1) * 4u) : make_float2(0.f, 0.f);
             }
@@ -756,12 +697,12 @@ gat_attn_bwd3_kernel(const AttnBwdArgs args, const Bwd3Plan pl, const __grid_con
               }
             }
           }
-          bar_group(1, kSmT);
-          if (tid == 0) bar_arrive(BAR(kBarEmpty + cur.slot));
+          bar_sync<1, kSmT>();
+          if (tid == 0) mbar_arrive(BAR(kBarEmpty + cur.slot));
           cur.advance();
           t_v += clock64() - t0;
         }
-        if (tid == 0) bar_arrive(BAR(kBarVDone));
+        if (tid == 0) mbar_arrive(BAR(kBarVDone));
 #pragma unroll
         for (int f = 0; f < 4; ++f)
 #pragma unroll
@@ -800,20 +741,6 @@ gat_attn_bwd3_kernel(const AttnBwdArgs args, const Bwd3Plan pl, const __grid_con
   tc_fence_before();
   __syncthreads();
   if (warp == kWarpMma) tmem_dealloc(tmem_base, 512);
-}
-
-int make_tmap3_f32(CUtensorMap* tm, const float* base, uint64_t d0, uint64_t d1, uint64_t d2, uint64_t stride1_elems,
-                   uint64_t stride2_elems, uint32_t b0, uint32_t b1, CUtensorMapSwizzle swz) {
-  EncodeTiledFn fn = encode_fn();
-  if (!fn) return fail(SPOTV2_ERR_NO_DEVICE, "cuTensorMapEncodeTiled is not available from the driver");
-  cuuint64_t dims[3] = {d0, d1, d2};
-  cuuint64_t strides[2] = {stride1_elems * sizeof(float), stride2_elems * sizeof(float)};
-  cuuint32_t box[3] = {b0, b1, 1};
-  cuuint32_t estr[3] = {1, 1, 1};
-  CUresult r = fn(tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<float*>(base), dims, strides, box, estr,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, swz, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) return fail(SPOTV2_ERR_CUDA, "cuTensorMapEncodeTiled (attention backward, 3-D) failed with CUresult %d", (int)r);
-  return SPOTV2_OK;
 }
 
 }  // namespace
@@ -867,14 +794,7 @@ int launch_attn_bwd3(AttnBwdArgs& a, float* dv, float* dbias, void* ws, size_t w
 }
 
 int bwd3_diag_add(unsigned long long* host_out, int reset) {
-  unsigned long long tmp[kNumCounters];
-  SPOTV2_CUDA_OK(cudaMemcpyFromSymbol(tmp, g_bwd3_counters, sizeof(tmp)));
-  for (int k = 0; k < kNumCounters; ++k) host_out[k] += tmp[k];
-  if (reset) {
-    unsigned long long zeros[kNumCounters] = {0};
-    SPOTV2_CUDA_OK(cudaMemcpyToSymbol(g_bwd3_counters, zeros, sizeof(zeros)));
-  }
-  return SPOTV2_OK;
+  return diag_add(host_out, g_bwd3_counters, reset);
 }
 
 }  // namespace spotv2

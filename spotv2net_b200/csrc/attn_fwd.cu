@@ -37,38 +37,6 @@ constexpr int kCbPerPass = 8;         // channel blocks per pass: one per MMA wa
 // wait-cycle diagnostics of this kernel (see spotv2_diag_counters)
 __device__ unsigned long long g_diag_counters[kNumCounters];
 
-__device__ __forceinline__ void bar_sync_group_a() { asm volatile("bar.sync 1, 96;" ::: "memory"); }
-__device__ __forceinline__ void bar_sync_group_b() { asm volatile("bar.sync 2, 256;" ::: "memory"); }
-__device__ __forceinline__ void mbar_arrive_cta(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-
-// 32-bit shared-window address forms of the hot-loop accesses (generic pointers make the compiler re-derive the
-// window base before every access) and the 2-op tf32 split: the tensor core reads only the top 19 bits of a
-// tf32 operand register, so "hi" is the raw fp32 pattern and only lo = x - trunc(x) costs ALU work.
-__device__ __forceinline__ float f_lds(uint32_t a) {
-  float v;
-  asm volatile("ld.shared.f32 %0, [%1];" : "=f"(v) : "r"(a));
-  return v;
-}
-__device__ __forceinline__ float4 f_lds128(uint32_t a) {
-  float4 v;
-  asm volatile("ld.shared.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(a));
-  return v;
-}
-__device__ __forceinline__ int f_ldsi(uint32_t a) {
-  int v;
-  asm volatile("ld.shared.s32 %0, [%1];" : "=r"(v) : "r"(a));
-  return v;
-}
-__device__ __forceinline__ void f_sts(uint32_t a, float v) {
-  asm volatile("st.shared.f32 [%0], %1;" ::"r"(a), "f"(v) : "memory");
-}
-__device__ __forceinline__ void split_lean(float x, uint32_t& hi, uint32_t& lo) {
-  hi = __float_as_uint(x);
-  lo = __float_as_uint(x - __uint_as_float(hi & 0xffffe000u));
-}
-
 // FIX: the reference's default geometry (N=30, H=6, C=500, Fe=126, head mean, PyG edge order) as compile-time
 // constants, so index arithmetic folds and the parameter block is not re-read inside the hot loops.
 template <int NPAIRS, bool VEC2, bool FIX>
@@ -171,7 +139,7 @@ gat_attn_fwd_kernel(const AttnFwdArgs args, const AttnSmem sm_, const uint32_t o
           mbar_expect_tx(&tile_full[buf], bytes);
           bulk_g2s(tile, p.edge_terms + (size_t)b * tile_floats, bytes, &tile_full[buf]);
         } else {
-          mbar_arrive_cta(&tile_full[buf]);
+          mbar_arrive(&tile_full[buf]);
         }
         continue;
       }
@@ -186,7 +154,7 @@ gat_attn_fwd_kernel(const AttnFwdArgs args, const AttnSmem sm_, const uint32_t o
         } else {
           const float* src = p.edge_rows + ((size_t)b * p.R + (size_t)c * sm.chunk_rows) * p.Fe;
           for (int idx = tid; idx < rows * p.Fe; idx += kGroupA) stage[s][idx] = src[idx];
-          bar_sync_group_a();
+          bar_sync<1, kGroupA>();
         }
         const long long tc0 = clock64();
         if (warp * 16 < rows) {
@@ -204,11 +172,11 @@ gat_attn_fwd_kernel(const AttnFwdArgs args, const AttnSmem sm_, const uint32_t o
             float4 bf[8];
 #pragma unroll
             for (int sl = 0; sl < 8; ++sl) {
-              a[sl][0] = f_lds(r0 + ko + sl * 32);
-              a[sl][1] = f_lds(r1 + ko + sl * 32);
-              a[sl][2] = f_lds(r0 + ko + sl * 32 + 16);
-              a[sl][3] = f_lds(r1 + ko + sl * 32 + 16);
-              bf[sl] = f_lds128(vf + sl * 512);
+              a[sl][0] = ldsa(r0 + ko + sl * 32);
+              a[sl][1] = ldsa(r1 + ko + sl * 32);
+              a[sl][2] = ldsa(r0 + ko + sl * 32 + 16);
+              a[sl][3] = ldsa(r1 + ko + sl * 32 + 16);
+              bf[sl] = lds128a(vf + sl * 512);
             }
 #pragma unroll
             for (int sl = 0; sl < 8; ++sl) {
@@ -223,20 +191,20 @@ gat_attn_fwd_kernel(const AttnFwdArgs args, const AttnSmem sm_, const uint32_t o
             }
           }
           const int rl = warp * 16 + 2 * g, row_base = c * sm.chunk_rows + rl;
-          const int to0 = rl < rows ? f_ldsi(a_table + (uint32_t)row_base * 4u) : -1;
-          const int to1 = rl + 1 < rows ? f_ldsi(a_table + (uint32_t)(row_base + 1) * 4u) : -1;
+          const int to0 = rl < rows ? ldsa_s32(a_table + (uint32_t)row_base * 4u) : -1;
+          const int to1 = rl + 1 < rows ? ldsa_s32(a_table + (uint32_t)(row_base + 1) * 4u) : -1;
           const uint32_t tb = a_tile0 + (uint32_t)(buf * tile_floats * 4) + (uint32_t)(2 * t) * head_bytes;
           if (to0 >= 0) {
-            if (2 * t < H) f_sts(tb + (uint32_t)to0, (acc[0][0] + acc[1][0]) + acc[2][0]);
-            if (2 * t + 1 < H) f_sts(tb + head_bytes + (uint32_t)to0, (acc[0][1] + acc[1][1]) + acc[2][1]);
+            if (2 * t < H) stsa(tb + (uint32_t)to0, (acc[0][0] + acc[1][0]) + acc[2][0]);
+            if (2 * t + 1 < H) stsa(tb + head_bytes + (uint32_t)to0, (acc[0][1] + acc[1][1]) + acc[2][1]);
           }
           if (to1 >= 0) {
-            if (2 * t < H) f_sts(tb + (uint32_t)to1, (acc[0][2] + acc[1][2]) + acc[2][2]);
-            if (2 * t + 1 < H) f_sts(tb + head_bytes + (uint32_t)to1, (acc[0][3] + acc[1][3]) + acc[2][3]);
+            if (2 * t < H) stsa(tb + (uint32_t)to1, (acc[0][2] + acc[1][2]) + acc[2][2]);
+            if (2 * t + 1 < H) stsa(tb + head_bytes + (uint32_t)to1, (acc[0][3] + acc[1][3]) + acc[2][3]);
           }
         }
         const long long tc1 = clock64();
-        bar_sync_group_a();                              // stage s consumed by all three warps
+        bar_sync<1, kGroupA>();                          // stage s consumed by all three warps
         t_call += tc1 - tc0;
         (void)t_mma;
         t_bar += clock64() - tc1;
@@ -246,12 +214,12 @@ gat_attn_fwd_kernel(const AttnFwdArgs args, const AttnSmem sm_, const uint32_t o
         // keep the edge terms for the backward (it then reads 6 floats per edge instead of the Fe-wide rows).  All of
         // group A's scatters are behind the chunk loop's last bar.sync; diagonal entries hold stale finite values
         // that no consumer reads.
-        if (nchunks == 0) bar_sync_group_a();
+        if (nchunks == 0) bar_sync<1, kGroupA>();
         float4* dst = reinterpret_cast<float4*>(p.edge_terms + (size_t)b * tile_floats);
         const float4* src = reinterpret_cast<const float4*>(tile);
         for (int idx = tid; idx < tile_floats / 4; idx += kGroupA) dst[idx] = src[idx];
       }
-      mbar_arrive_cta(&tile_full[buf]);                  // release: edge terms of this graph visible to group B
+      mbar_arrive(&tile_full[buf]);                      // release: edge terms of this graph visible to group B
     }
     if (tid == 0) {
       atomicAdd(&g_diag_counters[kCntRingFull], (unsigned long long)w_ring);
@@ -283,8 +251,8 @@ gat_attn_fwd_kernel(const AttnFwdArgs args, const AttnSmem sm_, const uint32_t o
       softmax_phase(p, sm, tile, reinterpret_cast<const float*>(smem_raw + off_sdtile + buf * kPTileBytes), out_scale,
                     args.alpha_out ? args.alpha_out + (size_t)b * H * N * N : nullptr, nullptr, tid - kGroupA, kGroupB,
                     -1, /*sd_swizzled=*/1, nullptr, b);
-      bar_sync_group_b();                                // alpha tile complete
-      if (tid == kGroupA) mbar_arrive_cta(&sd_empty[buf]);
+      bar_sync<2, kGroupB>();                            // alpha tile complete
+      if (tid == kGroupA) mbar_arrive(&sd_empty[buf]);
       for (int pass = 0; pass < n_pass; ++pass) {
         const int G = min(kCbPerPass, n_cb - pass * kCbPerPass);     // valid channel blocks in this pass
         const bool mine = wb < G;                          // this warp's channel block: pass * 8 + wb
@@ -356,7 +324,7 @@ gat_attn_fwd_kernel(const AttnFwdArgs args, const AttnSmem sm_, const uint32_t o
           for (int ks = 0; ks < 4; ++ks) {
 #pragma unroll
             for (int n = 0; n < 4; ++n) {
-              const float b0 = f_lds((pt0 ^ (n << 5)) + ks * 1024), b1 = f_lds((pt1 ^ (n << 5)) + ks * 1024);
+              const float b0 = ldsa((pt0 ^ (n << 5)) + ks * 1024), b1 = ldsa((pt1 ^ (n << 5)) + ks * 1024);
               uint32_t bh[2], bl[2];
               split_lean(b0, bh[0], bl[0]);
               split_lean(b1, bh[1], bl[1]);
@@ -369,7 +337,7 @@ gat_attn_fwd_kernel(const AttnFwdArgs args, const AttnSmem sm_, const uint32_t o
             }
           }
           __syncwarp();
-          if (lane == 0) mbar_arrive_cta(&ptile_empty[slot]);        // tile consumed
+          if (lane == 0) mbar_arrive(&ptile_empty[slot]);            // tile consumed
           if (p.concat) {                                  // every head is its own output block
             store(h * C);
             clear();
@@ -378,7 +346,7 @@ gat_attn_fwd_kernel(const AttnFwdArgs args, const AttnSmem sm_, const uint32_t o
         if (!p.concat && mine) store(0);                   // head mean (alpha pre-scaled by 1/H) + bias
       }
       if (p.terms_in) fence_proxy_async();               // our generic-proxy writes to the tile precede the next bulk copy into it
-      mbar_arrive_cta(&tile_empty[buf]);                 // this thread is done reading the alpha tile
+      mbar_arrive(&tile_empty[buf]);                     // this thread is done reading the alpha tile
     }
     if (tid == kGroupA) {
       atomicAdd(&g_diag_counters[kCntTileFull], (unsigned long long)w_tf);
@@ -410,7 +378,7 @@ gat_attn_fwd_kernel(const AttnFwdArgs args, const AttnSmem sm_, const uint32_t o
           *reinterpret_cast<float*>(dst + r * 128 + ((((c >> 2) ^ (r & 7)) << 4) | ((c & 3) << 2))) = v;
         }
         __syncwarp();
-        if (lane == 0) mbar_arrive_cta(full_bar);          // release: the tile is visible to the consumers
+        if (lane == 0) mbar_arrive(full_bar);              // release: the tile is visible to the consumers
       }
     };
     uint32_t q = 0;
@@ -495,19 +463,16 @@ int attn_fwd_dispatch(const AttnFwdArgs& a, cudaStream_t st) {
 
 }  // namespace spotv2
 
-namespace spotv2 { int bwd_diag_read(unsigned long long* host_out, int reset); }
+namespace spotv2 { int bwd_diag_add(unsigned long long* host_out, int reset); }
 using namespace spotv2;
 
 extern "C" int spotv2_diag_counters(unsigned long long* host_out, int reset) {
   SPOTV2_REQUIRE(host_out, "diag_counters: null pointer");
   SPOTV2_CUDA_OK(cudaDeviceSynchronize());
-  SPOTV2_CUDA_OK(cudaMemcpyFromSymbol(host_out, g_diag_counters, sizeof(unsigned long long) * kNumCounters));
-  if (reset) {
-    unsigned long long zeros[kNumCounters] = {0};
-    SPOTV2_CUDA_OK(cudaMemcpyToSymbol(g_diag_counters, zeros, sizeof(zeros)));
-  }
+  for (int k = 0; k < 2 * kNumCounters; ++k) host_out[k] = 0;
+  if (int rc = diag_add(host_out, g_diag_counters, reset)) return rc;
   if (int rc = fwd16_diag_add(host_out, reset)) return rc;      // whichever forward ran contributes; the other adds zeros
-  return bwd_diag_read(host_out + kNumCounters, reset);      // entries 16..31: backward phase times
+  return bwd_diag_add(host_out + kNumCounters, reset);       // entries 16..31: backward phase times
 }
 
 extern "C" int spotv2_gat_attn_fwd(const spotv2_gat_desc* d, const float* P_aug,

@@ -35,27 +35,6 @@ struct Fwd16Plan {
   uint32_t off_bar, off_table, off_vfrag, off_sd, off_tile, off_ahi, off_alo, off_ring, ring_stage, off_sdslot, off_slots, total;
 };
 
-__device__ __forceinline__ void bar_a() { asm volatile("bar.sync 1, 96;" ::: "memory"); }
-__device__ __forceinline__ void bar_b() { asm volatile("bar.sync 2, 256;" ::: "memory"); }
-__device__ __forceinline__ void arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ float q_lds(uint32_t a) {
-  float v;
-  asm volatile("ld.shared.f32 %0, [%1];" : "=f"(v) : "r"(a));
-  return v;
-}
-__device__ __forceinline__ float4 q_lds128(uint32_t a) {
-  float4 v;
-  asm volatile("ld.shared.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(a));
-  return v;
-}
-__device__ __forceinline__ int q_ldsi(uint32_t a) {
-  int v;
-  asm volatile("ld.shared.s32 %0, [%1];" : "=r"(v) : "r"(a));
-  return v;
-}
-__device__ __forceinline__ void q_sts(uint32_t a, float v) { asm volatile("st.shared.f32 [%0], %1;" ::"r"(a), "f"(v) : "memory"); }
 // cycle accounting per role (one sampling thread each; read through spotv2_diag_counters, entries [0, 16)):
 // 0 A: edge ring wait, 1 A: tile buffer free, 2 B: edge terms ready, 3 B: P tiles, 4 P: slot free, 5/6/7 role totals,
 // 8 A: logits arithmetic, 9 B: softmax, 10 B: conversions, 11 B: s|d tile, 12 A: chunk barriers, 13 A: edge-term copy-out
@@ -65,30 +44,22 @@ __device__ unsigned long long g_fwd16_counters[kNumCounters];
 __device__ __noinline__ void wait_report(int id, int it, uint32_t parity) {
   printf("attn_fwd16: wait %d timed out (block %d thread %d graph-iteration %d parity %u)\n", id, (int)blockIdx.x, (int)threadIdx.x, it, parity);
 }
+constexpr int kWaitSpins = 16;
+constexpr unsigned kWaitSleepNs = 64;
+constexpr long long kWaitLimit = 400000000LL;         // ~0.2 s: a tenth of the ~2 s the other kernels allow
 __device__ __forceinline__ void wait_id(uint64_t* bar, uint32_t parity, int id, int it) {
-  for (int spin = 0; spin < 16; ++spin)
-    if (mbar_try_wait(bar, parity)) return;
-  const long long t0 = clock64();
-  while (!mbar_try_wait(bar, parity)) {
-    __nanosleep(64);
-    if (clock64() - t0 > 400000000LL) { wait_report(id, it, parity); __trap(); }
-  }
+  mbar_wait_bounded<kWaitSpins, kWaitSleepNs, kWaitLimit>(smem_u32(bar), parity, [=] { wait_report(id, it, parity); });
 }
 // role counters cost ~4 K cycles per graph on the logit warps' critical path: compiled in with -DSPOTV2_BRINGUP only
 // (tools/fwd16_waits.py reads them); the product build measures nothing
 #ifdef SPOTV2_BRINGUP
-__device__ __forceinline__ long long tick() { return clock64(); }
+constexpr bool kRoleCounters = true;
 #else
-__device__ __forceinline__ long long tick() { return 0; }
+constexpr bool kRoleCounters = false;
 #endif
+__device__ __forceinline__ long long tick() { return kRoleCounters ? clock64() : 0; }
 __device__ __forceinline__ void wait_id_t(uint64_t* bar, uint32_t parity, int id, int it, long long& acc) {
-  const long long t0 = tick();
-  wait_id(bar, parity, id, it);
-  acc += tick() - t0;
-}
-__device__ __forceinline__ void split_raw(float x, uint32_t& hi, uint32_t& lo) {    // tf32: hi = raw fp32 (top 19 bits are read)
-  hi = __float_as_uint(x);
-  lo = __float_as_uint(x - __uint_as_float(hi & 0xffffe000u));
+  wait_timed<kRoleCounters>(acc, [&] { wait_id(bar, parity, id, it); });
 }
 
 template <bool FIX, bool SINGLE>
@@ -183,7 +154,7 @@ gat_attn_fwd16_kernel(const AttnFwdArgs args, const Fwd16Plan pl_, const __grid_
           mbar_expect_tx(&tile_full[buf], bytes);
           bulk_g2s(tile, p.edge_terms + (size_t)b * tile_floats, bytes, &tile_full[buf]);
         } else {
-          arrive(&tile_full[buf]);
+          mbar_arrive(&tile_full[buf]);
         }
         continue;
       }
@@ -197,7 +168,7 @@ gat_attn_fwd16_kernel(const AttnFwdArgs args, const Fwd16Plan pl_, const __grid_
         } else {
           const float* src = p.edge_rows + ((size_t)b * p.R + (size_t)c * pl.chunk_rows) * p.Fe;
           for (int idx = tid; idx < rows * p.Fe; idx += kGA) stage(s)[idx] = src[idx];
-          bar_a();
+          bar_sync<1, kGA>();
         }
         const long long tl0 = tick();
         if (warp * 16 < rows) {
@@ -218,11 +189,11 @@ gat_attn_fwd16_kernel(const AttnFwdArgs args, const Fwd16Plan pl_, const __grid_
             const uint32_t ko = (uint32_t)ks * 32u, vf = a_vfrag + ((uint32_t)ks * 32u + (uint32_t)lane) * 16u;
 #pragma unroll
             for (int sl = 0; sl < 4; ++sl) {
-              a[sl][0] = q_lds(r0 + ko + sl * 32);
-              a[sl][1] = q_lds(r1 + ko + sl * 32);
-              a[sl][2] = q_lds(r0 + ko + sl * 32 + 16);
-              a[sl][3] = q_lds(r1 + ko + sl * 32 + 16);
-              bf[sl] = q_lds128(vf + sl * 512);
+              a[sl][0] = ldsa(r0 + ko + sl * 32);
+              a[sl][1] = ldsa(r1 + ko + sl * 32);
+              a[sl][2] = ldsa(r0 + ko + sl * 32 + 16);
+              a[sl][3] = ldsa(r1 + ko + sl * 32 + 16);
+              bf[sl] = lds128a(vf + sl * 512);
             }
           };
           auto mma4 = [&](const float (&a)[4][4], const float4 (&bf)[4]) {
@@ -230,7 +201,7 @@ gat_attn_fwd16_kernel(const AttnFwdArgs args, const Fwd16Plan pl_, const __grid_
             for (int sl = 0; sl < 4; ++sl) {
               uint32_t ah[4], al[4];
 #pragma unroll
-              for (int q = 0; q < 4; ++q) split_raw(a[sl][q], ah[q], al[q]);
+              for (int q = 0; q < 4; ++q) split_lean(a[sl][q], ah[q], al[q]);
               const uint32_t bh[2] = {__float_as_uint(bf[sl].x), __float_as_uint(bf[sl].y)};
               const uint32_t bl[2] = {__float_as_uint(bf[sl].z), __float_as_uint(bf[sl].w)};
               mma_tf32_16x8x8(acc[0], al, bh);
@@ -249,20 +220,20 @@ gat_attn_fwd16_kernel(const AttnFwdArgs args, const Fwd16Plan pl_, const __grid_
 #pragma unroll
           for (int q = 0; q < 4; ++q) res[q] = (acc[0][q] + acc[1][q]) + acc[2][q];
           const int rl = warp * 16 + 2 * g, row_base = c * pl.chunk_rows + rl;
-          const int to0 = rl < rows ? q_ldsi(a_table + (uint32_t)row_base * 4u) : -1;
-          const int to1 = rl + 1 < rows ? q_ldsi(a_table + (uint32_t)(row_base + 1) * 4u) : -1;
+          const int to0 = rl < rows ? ldsa_s32(a_table + (uint32_t)row_base * 4u) : -1;
+          const int to1 = rl + 1 < rows ? ldsa_s32(a_table + (uint32_t)(row_base + 1) * 4u) : -1;
           const uint32_t tb = a_tile0 + (uint32_t)(buf * tile_floats * 4) + (uint32_t)(2 * t) * head_bytes;
           if (to0 >= 0) {
-            if (2 * t < H) q_sts(tb + (uint32_t)to0, res[0]);
-            if (2 * t + 1 < H) q_sts(tb + head_bytes + (uint32_t)to0, res[1]);
+            if (2 * t < H) stsa(tb + (uint32_t)to0, res[0]);
+            if (2 * t + 1 < H) stsa(tb + head_bytes + (uint32_t)to0, res[1]);
           }
           if (to1 >= 0) {
-            if (2 * t < H) q_sts(tb + (uint32_t)to1, res[2]);
-            if (2 * t + 1 < H) q_sts(tb + head_bytes + (uint32_t)to1, res[3]);
+            if (2 * t < H) stsa(tb + (uint32_t)to1, res[2]);
+            if (2 * t + 1 < H) stsa(tb + head_bytes + (uint32_t)to1, res[3]);
           }
         }
         const long long tl1 = tick();
-        bar_a();
+        bar_sync<1, kGA>();
         t_log += tl1 - tl0;
         t_bar += tick() - tl1;
         if (p.bulk_ok && tid == 0 && k + kEdgeStages < total_chunks) issue(k + kEdgeStages);
@@ -274,17 +245,14 @@ gat_attn_fwd16_kernel(const AttnFwdArgs args, const Fwd16Plan pl_, const __grid_
         // the tile, because the softmax group rewrites it in place.
         const long long to0 = tick();
         fence_proxy_async();
-        bar_a();
+        bar_sync<1, kGA>();
         if (tid == 0) {
-          asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(p.edge_terms + (size_t)b * tile_floats),
-                       "r"(smem_u32(tile)), "r"((uint32_t)tile_floats * 4u)
-                       : "memory");
-          asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-          asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
+          bulk_s2g_commit(p.edge_terms + (size_t)b * tile_floats, smem_u32(tile), (uint32_t)tile_floats * 4u);
+          bulk_wait_read();
         }
         t_out += tick() - to0;
       }
-      arrive(&tile_full[buf]);
+      mbar_arrive(&tile_full[buf]);
     }
     if (tid == 0) {
       atomicAdd(&g_fwd16_counters[0], (unsigned long long)w_ring);
@@ -349,17 +317,14 @@ gat_attn_fwd16_kernel(const AttnFwdArgs args, const Fwd16Plan pl_, const __grid_
       const long long tc1 = tick();
       wait_id_t(&tile_full[buf], (it >> 1) & 1, 4, it, w_tf);
       const long long ts0 = tick();
-      bar_b();                                           // sd complete (and everyone is past the previous graph's MMAs)
+      bar_sync<2, kGB>();                                // sd complete (and everyone is past the previous graph's MMAs)
       softmax_phase_regs(p, NS, tile, sd, out_scale, args.alpha_out ? args.alpha_out + (size_t)b * H * N * N : nullptr, nullptr, tb_,
                          kGB, nullptr, b, rec);
       if (rec) fence_proxy_async();                      // the copy engine reads what this thread wrote
-      bar_b();                                           // alpha tile complete
+      bar_sync<2, kGB>();                                // alpha tile complete
       if (rec && tb_ == 0) {
         // the backward's record: ONE bulk store of the finished tile (edge_mode 1: over the edge terms this graph came from)
-        asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(p.edge_terms + (size_t)b * tile_floats),
-                     "r"(smem_u32(tile)), "r"((uint32_t)tile_floats * 4u)
-                     : "memory");
-        asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+        bulk_s2g_commit(p.edge_terms + (size_t)b * tile_floats, smem_u32(tile), (uint32_t)tile_floats * 4u);
       }
       const long long tc2 = tick();
       t_smx += tc2 - ts0;
@@ -381,9 +346,9 @@ gat_attn_fwd16_kernel(const AttnFwdArgs args, const Fwd16Plan pl_, const __grid_
         }
       }
       if (p.terms_in) fence_proxy_async();               // generic-proxy writes to the tile precede the next bulk copy into it
-      if (rec && tb_ == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");   // the engine has read the record
-      arrive(&tile_empty[buf]);                          // the fp32 tile is free for the logit group
-      bar_b();                                           // alpha pair tiles complete
+      if (rec && tb_ == 0) bulk_wait_read();                                                // the engine has read the record
+      mbar_arrive(&tile_empty[buf]);                     // the fp32 tile is free for the logit group
+      bar_sync<2, kGB>();                                // alpha pair tiles complete
       t_cnv += (tc1 - tc0) + (tick() - tc2);
       for (int pass = 0; pass < n_pass; ++pass) {
         const int G = min(kCbPass, n_cb - pass * kCbPass);
@@ -485,7 +450,7 @@ gat_attn_fwd16_kernel(const AttnFwdArgs args, const Fwd16Plan pl_, const __grid_
             }
           }
           __syncwarp();
-          if (lane == 0) arrive(&p_empty[slot]);
+          if (lane == 0) mbar_arrive(&p_empty[slot]);
           if (!mine) continue;
           if (p.concat) {
             store(h * C);
@@ -538,14 +503,7 @@ gat_attn_fwd16_kernel(const AttnFwdArgs args, const Fwd16Plan pl_, const __grid_
 }  // namespace
 
 int fwd16_diag_add(unsigned long long* host_out, int reset) {
-  unsigned long long tmp[kNumCounters];
-  SPOTV2_CUDA_OK(cudaMemcpyFromSymbol(tmp, g_fwd16_counters, sizeof(tmp)));
-  for (int k = 0; k < kNumCounters; ++k) host_out[k] += tmp[k];
-  if (reset) {
-    unsigned long long zeros[kNumCounters] = {0};
-    SPOTV2_CUDA_OK(cudaMemcpyToSymbol(g_fwd16_counters, zeros, sizeof(zeros)));
-  }
-  return SPOTV2_OK;
+  return diag_add(host_out, g_fwd16_counters, reset);
 }
 
 // Shared-memory carve-up of the p_format 1 forward for a problem; n_slots * grp < 4 means it does not fit.

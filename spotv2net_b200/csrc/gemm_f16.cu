@@ -107,14 +107,10 @@ __device__ __noinline__ void gemm_wait_report(int id, uint32_t parity) {
   printf("gemm3x_f16: wait on %s timed out (block %d rank %u thread %d parity %u)\n", names[id], (int)blockIdx.x,
          cluster_ctarank(), (int)threadIdx.x, parity);
 }
+constexpr int kWaitSpins = 16;
+constexpr unsigned kWaitSleepNs = 64;
 __device__ __forceinline__ void hwait(uint64_t* bar, uint32_t parity, int id) {
-  for (int spin = 0; spin < 16; ++spin)
-    if (mbar_try_wait(bar, parity)) return;
-  const long long t0 = clock64();
-  while (!mbar_try_wait(bar, parity)) {
-    __nanosleep(64);
-    if (clock64() - t0 > 4000000000LL) { gemm_wait_report(id, parity); __trap(); }
-  }
+  mbar_wait_bounded<kWaitSpins, kWaitSleepNs, kWaitTrapCycles>(smem_u32(bar), parity, [=] { gemm_wait_report(id, parity); });
 }
 
 // CTAS = 2: pair tiles on a cluster of two CTAs (launched with cluster dimension 2); CTAS = 1: every CTA computes a
@@ -372,7 +368,7 @@ gemm3x_f16_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constan
           for (int pln = 0; pln < 2; ++pln) {
             if (pln == 1 && p.pair_out != 1) break;
             unsigned char* hb = box + ((p.pair_out == 1 ? 2 * cc + pln : cc) & (S::kPairBoxes - 1)) * 2048;
-            if (lane == 0) asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(S::kPairBoxes - 1) : "memory");
+            if (lane == 0) bulk_wait_read<S::kPairBoxes - 1>();
             __syncwarp();
 #pragma unroll
             for (int c = 0; c < 4; ++c)
@@ -383,10 +379,8 @@ gemm3x_f16_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constan
             __syncwarp();
             if (lane == 0) {
               if (col0 + cc * 32 < p.N && row_base < p.M && !(SPOTV2_DBG(p) & 1))
-                asm volatile("cp.async.bulk.tensor.3d.global.shared::cta.bulk_group [%0, {%2, %3, %4}], [%1];" ::"l"(&tmC),
-                             "r"(smem_u32(hb)), "r"(col0 + cc * 32), "r"(row_base), "r"(pln)
-                             : "memory");
-              asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+                tma_store_3d(&tmC, smem_u32(hb), col0 + cc * 32, row_base, pln);
+              bulk_commit();
             }
           }
         }
@@ -400,7 +394,7 @@ gemm3x_f16_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constan
 #pragma unroll
         for (int cc = 0; cc < HALF / 16; ++cc) {
           unsigned char* hb = box + (cc & 1) * 2048;
-          if (lane == 0) asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory");   // the store before last has been read
+          if (lane == 0) bulk_wait_read<1>();                                             // the store before last has been read
           __syncwarp();
 #pragma unroll
           for (int c = 0; c < 4; ++c)
@@ -410,10 +404,8 @@ gemm3x_f16_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constan
           __syncwarp();
           if (lane == 0) {
             if (col0 + cc * 16 < p.N && row_base < p.M)
-              asm volatile("cp.async.bulk.tensor.3d.global.shared::cta.bulk_group [%0, {%2, %3, %4}], [%1];" ::"l"(&tmC),
-                           "r"(smem_u32(hb)), "r"(col0 + cc * 16), "r"(row_base), "r"(sp)
-                           : "memory");
-            asm volatile("cp.async.bulk.commit_group;" ::: "memory");       // always commit: keeps the group count in step with cc
+              tma_store_3d(&tmC, smem_u32(hb), col0 + cc * 16, row_base, sp);
+            bulk_commit();                                                  // always commit: keeps the group count in step with cc
           }
         }
       } else if (!(SPOTV2_DBG(p) & 1)) {
@@ -444,7 +436,7 @@ gemm3x_f16_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constan
     }
   }
 
-  if (warp >= 4 && lane == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");   // this lane's bulk stores have landed
+  if (warp >= 4 && lane == 0) bulk_wait();                                                // this lane's bulk stores have landed
   tc_fence_before();
   if constexpr (CTAS == 2) {
     cluster_sync();           // both CTAs have drained their TMEM and sent their last arrivals to the leader

@@ -5,9 +5,6 @@
 namespace spotv2 {
 
 // ---- PTX wrappers -----------------------------------------------------------------------------
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tmem_alloc(uint32_t* smem_dst, uint32_t ncols) {
@@ -32,9 +29,11 @@ __device__ __forceinline__ void umma_f16(uint32_t tmem_d, uint64_t adesc, uint64
       "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accum)
       : "memory");
 }
-__device__ __forceinline__ void umma_commit(uint64_t* bar) {   // implies tcgen05.fence::before_thread_sync
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
+// arrives on the barrier when every tcgen05.mma issued so far has retired; implies tcgen05.fence::before_thread_sync
+__device__ __forceinline__ void umma_commit(uint32_t bar) {
+  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
 }
+__device__ __forceinline__ void umma_commit(uint64_t* bar) { umma_commit(smem_u32(bar)); }
 
 // ---- CTA pairs (cluster of 2, cta_group::2): one MMA of M = 256 spans both CTAs' shared memory and TMEM -------------
 __device__ __forceinline__ uint32_t cluster_ctarank() {
@@ -81,6 +80,15 @@ __device__ __forceinline__ void umma_commit_pair(uint64_t* bar, uint16_t cta_mas
                : "memory");
 }
 
+__device__ __forceinline__ void tmem_wait_ld() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
+__device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&r)[16]) {
+  asm volatile(
+      "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
+      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]), "=r"(r[9]),
+        "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
+      : "r"(taddr));
+  tmem_wait_ld();
+}
 __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&r)[32]) {
   asm volatile(
       "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,%21,"
@@ -90,7 +98,7 @@ __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&r)[32]) {
         "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]),
         "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
       : "r"(taddr));
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+  tmem_wait_ld();
 }
 __device__ __forceinline__ bool elect_one() {
   uint32_t pred;
