@@ -1126,7 +1126,8 @@ def test_full_batch_gradients_match_chunked_oracle(cuda_lib):
     cannot hold 4096 graphs (2 x 44 GB of PyG intermediates), but its parameter gradients are sums over graphs, so it
     runs in 64 chunks of 64 graphs and autograd accumulates them in fp64.  Covers what the small cases cannot: the
     per-CTA partial reductions of dv / dbias / ds|dd over 4096 graphs on 148 CTAs and the 16-way split-K of the
-    weight-gradient GEMM (what the reference does in one pass: 5_train_SpotV2Net.py:150-159)."""
+    weight-gradient GEMM (what the reference does in one pass: 5_train_SpotV2Net.py:150-159), and the input gradient
+    (proj_bwd_input on the padded dP pair over 960 row tiles), chunk by chunk."""
     import copy
     B, N, L, H, C_ = 4096, 30, 42, 6, 500
     Fin, Fe, chunk = N * L, 3 * L, 64
@@ -1138,7 +1139,7 @@ def test_full_batch_gradients_match_chunked_oracle(cuda_lib):
     ours.load_state_dict(ref.state_dict())
     ours.to(DEV)
     g = torch.Generator(device=DEV).manual_seed(3)
-    x = torch.randn(B * N, Fin, device=DEV, generator=g)
+    x = torch.randn(B * N, Fin, device=DEV, generator=g).requires_grad_()
     ea = torch.randn(B * N * (N - 1), Fe, device=DEV, generator=g)
     dout = torch.randn(B * N, C_, device=DEV, generator=g)
     ei, _ = sv.batched_topology(B, N, DEV)
@@ -1150,16 +1151,20 @@ def test_full_batch_gradients_match_chunked_oracle(cuda_lib):
 
     def oracle_grads(dtype):
         m = copy.deepcopy(ref).to(dtype)
-        worst = 0.0
+        worst, worst_dx = 0.0, 0.0
         for c0 in range(0, B, chunk):
             rows, erows = slice(c0 * N, (c0 + chunk) * N), slice(c0 * N * (N - 1), (c0 + chunk) * N * (N - 1))
-            o = m(x[rows].cpu().to(dtype), ei_c, ea[erows].cpu().to(dtype))
+            xc = x[rows].detach().cpu().to(dtype).requires_grad_()
+            o = m(xc, ei_c, ea[erows].cpu().to(dtype))
             o.backward(dout[rows].cpu().to(dtype))            # .grad accumulates over the chunks
             worst = max(worst, relerr(out[rows], o.detach()))
-        return {"g_" + k: p.grad for k, p in m.named_parameters()}, worst
+            worst_dx = max(worst_dx, relerr(x.grad[rows], xc.grad))
+        return {"g_" + k: p.grad for k, p in m.named_parameters()}, worst, worst_dx
 
-    g64, worst_out = oracle_grads(torch.float64)
+    g64, worst_out, worst_dx = oracle_grads(torch.float64)
+    print(f"B=4096 chunked fp64 oracle: worst out error {worst_out:.2e}, worst x.grad error {worst_dx:.2e}")
     assert worst_out < TOL, worst_out
+    assert worst_dx < TOL, worst_dx
     mine = {"g_" + k: p.grad for k, p in ours.named_parameters()}
     errs = {k: relerr(mine[k], g64[k]) for k in g64}
     print("B=4096 gradient errors vs the chunked fp64 oracle:", {k: f"{v:.2e}" for k, v in errs.items()})

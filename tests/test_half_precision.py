@@ -282,7 +282,7 @@ def dense_attention(P, s, d_, T, v, bias, dout, H, concat, slope, mask=None, kee
     dal = dad if mask is None else dad * mask * keep_scale
     dl = alpha * (dal - (alpha * dal).sum(2, keepdim=True))
     dz = dl * torch.where(z > 0, torch.ones_like(z), torch.full_like(z, slope))
-    res = dict(alpha=ad, out=out, dP=torch.einsum("bijh,bihc->bjhc", ad, dO), ds=dz.sum(1), dd=dz.sum(2), dbias=dout.sum(0),
+    res = dict(alpha=ad, out=out, dP=torch.einsum("bijh,bihc->bjhc", ad, dO), dz=dz, ds=dz.sum(1), dd=dz.sum(2), dbias=dout.sum(0),
                dO=dO, aP=torch.einsum("bijh,bjhc->bihc", ad, P.abs()), adO=torch.einsum("bijh,bihc->bjhc", ad, dO.abs()))
     if T is not None:
         diag = torch.diagonal(dz, dim1=1, dim2=2).permute(0, 2, 1)
