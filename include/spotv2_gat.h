@@ -209,6 +209,19 @@ int spotv2_gat_attn_bwd(const spotv2_gat_desc* d, const float* P_aug, const floa
                         float* dv_or_null, float* d_edge_terms_or_null, float* dbias_or_null, void* ws, size_t ws_bytes,
                         void* stream);
 
+/* spotv2_gat_attn_bwd with the gradient through the attention coefficients the forward returned: d_alpha [B, H, N(source j),
+ * N(target i)] fp32 (the layout of alpha_or_null; spotv2_alpha_to_pyg_grad makes it from a PyG-order gradient) is dL/d(alpha m/(1-p)),
+ * the coefficients after attention dropout (m = keep mask; m = 1 without dropout).  It joins dalpha = g dO P^T (g = 1/H for the
+ * head mean, 1 for concat) before the dropout factor: dalpha_ij = m_ij/(1-p) (<g dO_i, P_j> + d_alpha_ij); everything after
+ * that (softmax, LeakyReLU, ds | dd, dz', dv, d_edge_terms) follows unchanged.  d_alpha is required; the preconditions and the
+ * other arguments are those of spotv2_gat_attn_bwd. */
+int spotv2_gat_attn_bwd_dalpha(const spotv2_gat_desc* d, const float* P_aug, const float* p_amax_or_null,
+                               const float* edge_rows, const float* edge_terms_or_null,
+                               const int32_t* table, const float* v, const float* dout, float* dP_aug_or_null,
+                               void* dP_hi_or_null, void* dP_lo_or_null, float* dp_scale_or_null,
+                               float* dv_or_null, float* d_edge_terms_or_null, float* dbias_or_null, void* ws, size_t ws_bytes,
+                               void* stream, const float* d_alpha);
+
 /* Gradient w.r.t. the edge rows (edge_mode 0): d_edge_rows [B, R, Fe] in PyG row order,
  *   d_edge_rows[b*R + r, :] = sum_h d_edge_terms[b][h][j][i] * v[h, :]   for table[r] = (i << 16) | j,
  *   d_edge_rows[b*R + r, :] = 0                                           for SPOTV2_ROW_SKIP rows,
@@ -246,6 +259,12 @@ int spotv2_gat_attn_bwd_pair(const spotv2_gat_desc* d, const void* P_hi, const v
                              const float* v, const float* dout, void* dP_hi, void* dP_lo_or_null, float* dp_scale,
                              float* dv_or_null, float* d_edge_terms_or_null, float* dbias_or_null, void* ws,
                              size_t ws_bytes, void* stream);
+/* spotv2_gat_attn_bwd_pair with the gradient through the returned coefficients, as spotv2_gat_attn_bwd_dalpha. */
+int spotv2_gat_attn_bwd_pair_dalpha(const spotv2_gat_desc* d, const void* P_hi, const void* P_lo_or_null, const float* p_scale,
+                                    const float* sd, const float* edge_rows, const float* edge_terms_or_null, const int32_t* table,
+                                    const float* v, const float* dout, void* dP_hi, void* dP_lo_or_null, float* dp_scale,
+                                    float* dv_or_null, float* d_edge_terms_or_null, float* dbias_or_null, void* ws,
+                                    size_t ws_bytes, void* stream, const float* d_alpha);
 
 /* ---- structured edge source (SURVEY.md 8f-2; csrc/windows.cu) ---------------------------------------------------
  * In the reference's dataset (utils/dataset.py:228-242) edge_attr is a pure function of the window of co-volatility
@@ -284,6 +303,12 @@ int spotv2_gat_unfold(const spotv2_gat_desc* d, const float* W, const float* a_s
  * order, then the B*N self loops: alpha_pyg [B*R_real + B*N, H]. */
 int spotv2_alpha_to_pyg(const spotv2_gat_desc* d, const float* alpha_tile, const int32_t* table,
                         float* alpha_pyg, void* stream);
+/* Its inverse for gradients: d_alpha_pyg [B*R + B*N, H] (same order) -> d_alpha_tile [B, H, N(j), N(i)], the d_alpha input of
+ * the _dalpha backward entry points.  Real-edge rows go through the table, loop rows give the diagonal, SPOTV2_ROW_SKIP rows
+ * (input self loops, absent from what PyG returns) are ignored.  With the table of a complete graph every tile entry is
+ * written exactly once: the output needs no clearing. */
+int spotv2_alpha_to_pyg_grad(const spotv2_gat_desc* d, const float* d_alpha_pyg, const int32_t* table,
+                             float* d_alpha_tile, void* stream);
 
 /* Graph-batch collation on the device (replaces PyG DataLoader/Batch.from_data_list
  * over CovarianceLaggedDataset, /root/reference/utils/dataset.py:182-289 and

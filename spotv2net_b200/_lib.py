@@ -42,6 +42,7 @@ SIGNATURES = {
     "spotv2_proj_fwd_pair": (C.c_int, [_DP] + [_vp] * 9 + [_sz, _vp]),
     "spotv2_gat_attn_fwd_pair": (C.c_int, [_DP] + [_vp] * 12),
     "spotv2_gat_attn_bwd_pair": (C.c_int, [_DP] + [_vp] * 16 + [_sz, _vp]),
+    "spotv2_gat_attn_bwd_pair_dalpha": (C.c_int, [_DP] + [_vp] * 16 + [_sz, _vp, _vp]),
     "spotv2_edge_table_build": (C.c_int, [_vp, _i64, _i32, _i32, _i32, _vp, _vp, _vp]),
     "spotv2_edge_table_dense": (C.c_int, [_i32, _vp, _vp]),
     "spotv2_gat_fold": (C.c_int, [_DP] + [_vp] * 8),
@@ -53,6 +54,7 @@ SIGNATURES = {
     "spotv2_gat_edge_terms_bytes": (C.c_int, [_DP, C.POINTER(_sz)]),
     "spotv2_gat_attn_fwd": (C.c_int, [_DP] + [_vp] * 9 + [_sz, _vp]),
     "spotv2_gat_attn_bwd": (C.c_int, [_DP] + [_vp] * 15 + [_sz, _vp]),
+    "spotv2_gat_attn_bwd_dalpha": (C.c_int, [_DP] + [_vp] * 15 + [_sz, _vp, _vp]),
     "spotv2_gat_edge_rows_grad": (C.c_int, [_DP] + [_vp] * 5),
     "spotv2_edge_terms_from_windows_workspace_bytes": (C.c_int, [_DP, C.POINTER(_sz)]),
     "spotv2_edge_terms_from_windows": (C.c_int, [_DP, _vp, _i32, _i32, _vp, _vp, _vp, _vp, _sz, _vp]),
@@ -62,6 +64,7 @@ SIGNATURES = {
     "spotv2_proj_bwd_input": (C.c_int, [_DP] + [_vp] * 7 + [_sz, _vp]),
     "spotv2_gat_unfold": (C.c_int, [_DP] + [_vp] * 13),
     "spotv2_alpha_to_pyg": (C.c_int, [_DP, _vp, _vp, _vp, _vp]),
+    "spotv2_alpha_to_pyg_grad": (C.c_int, [_DP, _vp, _vp, _vp, _vp]),
     "spotv2_collate_windows": (C.c_int, [_vp, _vp, _i32, _i32, _i32, _vp, _i32, _vp, _vp, _vp, _vp]),
     "spotv2_stack_scale": (C.c_int, [_vp, _i64, _vp, _vp]),
     "spotv2_collate_windows_pair": (C.c_int, [_vp, _vp, _i32, _i32, _i32, _vp, _i32, _vp, _vp, _vp, _i32, _vp, _vp, _vp, _vp]),

@@ -84,13 +84,17 @@ int reduce_partials2(const float* part_a, int nparts_a, int len_a, float* out_a,
 
 // Pipelined kernel.  Returns SPOTV2_ERR_UNSUPPORTED (without setting an error) when the plan does not fit.
 bool attn_bwd2_fits(const AttnParams& p);
-int launch_attn_bwd2(AttnBwdArgs& a, float* dv, float* dbias, void* ws, size_t ws_bytes, cudaStream_t st);
+// d_alpha (null = none): [B, H, N, N] gradient w.r.t. the coefficients the forward returned (spotv2_gat_attn_bwd_dalpha);
+// the launchers below take it the same way
+int launch_attn_bwd2(AttnBwdArgs& a, float* dv, float* dbias, void* ws, size_t ws_bytes, cudaStream_t st,
+                     const float* d_alpha = nullptr);
 size_t attn_bwd2_partials_bytes(const spotv2_gat_desc* d);
 int bwd2_diag_add(unsigned long long* host_out, int reset);      // adds its phase counters into host_out[0..5]
 
 // tcgen05 kernel (attn_bwd3.cu): head-mean layers, N <= 31, edge terms kept by the forward.
 bool attn_bwd3_applies(const AttnParams& p);
-int launch_attn_bwd3(AttnBwdArgs& a, float* dv, float* dbias, void* ws, size_t ws_bytes, cudaStream_t st);
+int launch_attn_bwd3(AttnBwdArgs& a, float* dv, float* dbias, void* ws, size_t ws_bytes, cudaStream_t st,
+                     const float* d_alpha = nullptr);
 size_t attn_bwd3_partials_bytes(const spotv2_gat_desc* d);
 int bwd3_diag_add(unsigned long long* host_out, int reset);     // adds its 16 wait / work counters into host_out[0..15]
 
@@ -101,6 +105,6 @@ size_t attn_large_bwd_ws_bytes(const spotv2_gat_desc* d);
 int attn_large_fwd(const AttnParams& p, const float* bias, float* out, float* alpha_out, void* ws, size_t ws_bytes,
                    cudaStream_t st);
 int attn_large_bwd(const spotv2_gat_desc* d, AttnBwdArgs& a, float* dv, float* dbias, void* ws, size_t ws_bytes,
-                   cudaStream_t st);
+                   cudaStream_t st, const float* d_alpha = nullptr);
 
 }  // namespace spotv2

@@ -190,64 +190,17 @@ lg_softmax_kernel(const float* __restrict__ P_aug, const float* Zraw, float* A, 
 // Softmax + LeakyReLU backward, same thread layout.  dA holds dalpha on entry and dz on exit (diagonal included:
 // it is the self loop's dz); fill[b,h,i] = dz_ii / (N - 1), the gradient every incoming edge term of i receives
 // through the mean fill; dd_i goes to column HC + H + h of dP_aug.
-__global__ void __launch_bounds__(kSmX * kSmY)
-lg_softmax_bwd_kernel(const float* __restrict__ P_aug, const float* __restrict__ Zraw, float* A,
-                      float* dA, const float* __restrict__ gii, float* __restrict__ fill, float* dP_aug, int N,
-                      int H, int HC, int ldp, float slope, const DropoutParams drop) {
-  extern __shared__ float s_src[];
-  __shared__ float red[kSmY][kSmX];
-  __shared__ float s_dzii[kSmX];
-  const int b = blockIdx.z, h = blockIdx.y, tx = threadIdx.x, ty = threadIdx.y;
-  const float* Pb = P_aug + (size_t)b * N * ldp;
-  for (int j = ty * kSmX + tx; j < N; j += kSmX * kSmY) s_src[j] = Pb[(size_t)j * ldp + HC + h];
-  __syncthreads();
-  const int i = blockIdx.x * kSmX + tx;
-  const bool live = i < N;
-  const int ic = live ? i : N - 1;
-  const size_t base = ((size_t)b * H + h) * N * N + ic;
-  const float* zc = Zraw ? Zraw + base : nullptr;
-  float* ac = A + base;
-  float* dc = dA + base;
-  const float di = Pb[(size_t)ic * ldp + HC + H + h];
-  const float g_ii = gii[((size_t)b * H + h) * N + ic];
-  // attention dropout: the forward used alpha * m (m = keep / (1 - p)), so dalpha = m * d(alpha m); A leaves this
-  // kernel as alpha * m for the dP product
-  const unsigned long long ebase = (((unsigned long long)b * H + h) * N + ic) * N;
-  auto mfac = [&](int j) { return drop.p > 0.f ? (dropout_keep(drop, ebase + j) ? drop.scale : 0.f) : 1.f; };
-  float dot = 0.f;
-#pragma unroll 8
-  for (int j = ty; j < N; j += kSmY) dot = fmaf(ac[(size_t)j * N], dc[(size_t)j * N] * mfac(j), dot);
-  red[ty][tx] = dot;
-  __syncthreads();
-  dot = 0.f;
-#pragma unroll
-  for (int k = 0; k < kSmY; ++k) dot += red[k][tx];
-  __syncthreads();
-  float dd = 0.f;
-#pragma unroll 8
-  for (int j = ty; j < N; j += kSmY) {
-    const float g = (j == ic) ? g_ii : (zc ? zc[(size_t)j * N] : 0.f);
-    const float z = g + s_src[j] + di;
-    const float m = mfac(j), al = ac[(size_t)j * N];
-    const float dl = al * (dc[(size_t)j * N] * m - dot);
-    const float dz = z > 0.f ? dl : dl * slope;
-    dd += dz;
-    if (j == ic) s_dzii[tx] = dz;
-    if (live) {
-      dc[(size_t)j * N] = dz;
-      if (drop.p > 0.f) ac[(size_t)j * N] = al * m;
-    }
-  }
-  red[ty][tx] = dd;
-  __syncthreads();
-  if (ty == 0 && live) {
-    dd = 0.f;
-#pragma unroll
-    for (int k = 0; k < kSmY; ++k) dd += red[k][tx];
-    fill[((size_t)b * H + h) * N + i] = s_dzii[tx] / (float)(N > 1 ? N - 1 : 1);
-    dP_aug[((size_t)b * N + i) * ldp + HC + H + h] = dd;
-  }
-}
+// The kernel without and with the gradient through the returned coefficients (spotv2_gat_attn_bwd_dalpha)
+#define SPOTV2_KERNEL_NAME lg_softmax_bwd_kernel
+#define SPOTV2_GA 0
+#include "attn_large_softmax_bwd.cuh"
+#undef SPOTV2_KERNEL_NAME
+#undef SPOTV2_GA
+#define SPOTV2_KERNEL_NAME lg_softmax_bwd_dalpha_kernel
+#define SPOTV2_GA 1
+#include "attn_large_softmax_bwd.cuh"
+#undef SPOTV2_KERNEL_NAME
+#undef SPOTV2_GA
 
 // ds_j = sum_i dz[j][i] -> column HC + h of dP_aug.  One warp per (b, h, j) row, fixed lane-strided order.
 __global__ void __launch_bounds__(256)
@@ -544,7 +497,7 @@ int attn_large_fwd(const AttnParams& p, const float* bias, float* out, float* al
 }
 
 int attn_large_bwd(const spotv2_gat_desc* d, AttnBwdArgs& a, float* dv, float* dbias, void* ws, size_t ws_bytes,
-                   cudaStream_t st) {
+                   cudaStream_t st, const float* d_alpha) {
   const AttnParams& p = a.p;
   if (!ws || ws_bytes < attn_large_bwd_ws_bytes(d))
     return fail(SPOTV2_ERR_WORKSPACE, "attn_bwd (N=%d > 32) needs %zu B of workspace, got %zu", p.N,
@@ -588,8 +541,12 @@ int attn_large_bwd(const spotv2_gat_desc* d, AttnBwdArgs& a, float* dv, float* d
   }
   {
     dim3 grid((p.N + kSmX - 1) / kSmX, p.H, p.B);
-    lg_softmax_bwd_kernel<<<grid, dim3(kSmX, kSmY), (size_t)p.N * sizeof(float), st>>>(p.P_aug, Zr, A, dA, gii, fill, dP, p.N, p.H, HC,
-                                                                          p.ldp, p.slope, p.drop);
+    if (d_alpha)
+      lg_softmax_bwd_dalpha_kernel<<<grid, dim3(kSmX, kSmY), (size_t)p.N * sizeof(float), st>>>(p.P_aug, Zr, A, dA, gii, fill, dP, p.N,
+                                                                                   p.H, HC, p.ldp, p.slope, p.drop, d_alpha);
+    else
+      lg_softmax_bwd_kernel<<<grid, dim3(kSmX, kSmY), (size_t)p.N * sizeof(float), st>>>(p.P_aug, Zr, A, dA, gii, fill, dP, p.N, p.H, HC,
+                                                                            p.ldp, p.slope, p.drop);
     SPOTV2_CUDA_OK(cudaGetLastError());
     const long long warps = (long long)p.B * p.H * p.N;
     lg_rowsum_kernel<<<(unsigned)((warps * 32 + 255) / 256), 256, 0, st>>>(dA, dP, p.B, p.N, p.H, HC, p.ldp);

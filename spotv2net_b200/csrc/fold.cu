@@ -198,6 +198,57 @@ __global__ void alpha_to_pyg_kernel(const float* __restrict__ tile, const int32_
   }
 }
 
+// Inverse of alpha_to_pyg_kernel for gradients: [B*R rows | B*N loops] x H -> tile [B, H, N(j), N(i)].  The table of a
+// complete graph names every ordered pair i != j exactly once and the loop rows give the diagonal, so every tile entry is
+// written exactly once (no atomics, no clearing pass); SPOTV2_ROW_SKIP rows (input self loops) are not read.  Threads run
+// over (graph, head, row) with the row fastest: a warp's stores follow the table (source-major in PyG's order, so mostly
+// consecutive), its loads are H floats apart inside the graph's block of rows, which the other heads' warps read as well.
+__global__ void alpha_to_pyg_grad_kernel(const float* __restrict__ d_pyg, const int32_t* __restrict__ table,
+                                         float* __restrict__ d_tile, int B, int N, int H, int R) {
+  const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  const int64_t n_real = (int64_t)B * R * H, n_all = n_real + (int64_t)B * N * H;
+  if (idx >= n_all) return;
+  if (idx < n_real) {
+    const int64_t bh = idx / R;
+    const int r = (int)(idx - bh * R);
+    const int64_t b = bh / H;
+    const int h = (int)(bh - b * H);
+    const int code = table[r];
+    if (code >= 0) d_tile[((size_t)bh * N + (code & 0xffff)) * N + (code >> 16)] = d_pyg[((size_t)b * R + r) * H + h];
+  } else {
+    const int64_t k = idx - n_real;
+    const int64_t bh = k / N;
+    const int i = (int)(k - bh * N);
+    const int64_t b = bh / H;
+    const int h = (int)(bh - b * H);
+    d_tile[((size_t)bh * N + i) * N + i] = d_pyg[(size_t)B * R * H + ((size_t)b * N + i) * H + h];
+  }
+}
+
+// The same for graphs whose tile fits in shared memory (H*N*N floats <= 48 KB; every N <= 32 with H <= 8): one block per graph
+// reads its rows coalesced, scatters them into the tile in shared memory and writes the tile out in order, so that neither
+// the loads nor the stores of a warp are strided.  Every entry is written by the scatter (complete table), none is cleared.
+__global__ void __launch_bounds__(256)
+alpha_to_pyg_grad_graph_kernel(const float* __restrict__ d_pyg, const int32_t* __restrict__ table, float* __restrict__ d_tile,
+                               int B, int N, int H, int R) {
+  extern __shared__ float t_s[];                 // [H][N(j)][N(i)]
+  const int b = blockIdx.x, NN = N * N;
+  const float* rows = d_pyg + (size_t)b * R * H;
+  for (int idx = threadIdx.x; idx < R * H; idx += blockDim.x) {
+    const int r = idx / H, h = idx - r * H;
+    const int code = table[r];
+    if (code >= 0) t_s[h * NN + (code & 0xffff) * N + (code >> 16)] = rows[idx];
+  }
+  const float* loops = d_pyg + (size_t)B * R * H + (size_t)b * N * H;
+  for (int idx = threadIdx.x; idx < N * H; idx += blockDim.x) {
+    const int i = idx / H, h = idx - i * H;
+    t_s[h * NN + i * N + i] = loops[idx];
+  }
+  __syncthreads();
+  float* dst = d_tile + (size_t)b * H * NN;
+  for (int idx = threadIdx.x; idx < H * NN; idx += blockDim.x) dst[idx] = t_s[idx];
+}
+
 // ---- window collation (utils/dataset.py:182-289 layouts, SURVEY.md Appendix B) -------------
 __global__ void collate_x_kernel(const float* __restrict__ M_vol, const int32_t* __restrict__ t0,
                                  int N, int L, float* __restrict__ x, float* __restrict__ y) {
@@ -358,6 +409,23 @@ extern "C" int spotv2_alpha_to_pyg(const spotv2_gat_desc* d, const float* alpha_
   const int64_t total = ((int64_t)d->B * d->R + (int64_t)d->B * d->N) * d->H;
   alpha_to_pyg_kernel<<<(unsigned)((total + 255) / 256), 256, 0, as_stream(stream)>>>(
       alpha_tile, table, alpha_pyg, d->B, d->N, d->H, d->R);
+  SPOTV2_CUDA_OK(cudaGetLastError());
+  return SPOTV2_OK;
+}
+
+extern "C" int spotv2_alpha_to_pyg_grad(const spotv2_gat_desc* d, const float* d_alpha_pyg, const int32_t* table,
+                                        float* d_alpha_tile, void* stream) {
+  if (int rc = check_desc(d)) return rc;
+  SPOTV2_REQUIRE(d_alpha_pyg && table && d_alpha_tile, "alpha_to_pyg_grad: d_alpha_pyg, table and d_alpha_tile must be non-null");
+  const size_t tile_bytes = (size_t)d->H * d->N * d->N * sizeof(float);
+  if (tile_bytes <= 48 * 1024) {
+    alpha_to_pyg_grad_graph_kernel<<<(unsigned)d->B, 256, tile_bytes, as_stream(stream)>>>(
+        d_alpha_pyg, table, d_alpha_tile, d->B, d->N, d->H, d->R);
+  } else {
+    const int64_t total = ((int64_t)d->B * d->R + (int64_t)d->B * d->N) * d->H;
+    alpha_to_pyg_grad_kernel<<<(unsigned)((total + 255) / 256), 256, 0, as_stream(stream)>>>(
+        d_alpha_pyg, table, d_alpha_tile, d->B, d->N, d->H, d->R);
+  }
   SPOTV2_CUDA_OK(cudaGetLastError());
   return SPOTV2_OK;
 }

@@ -289,18 +289,21 @@ class _GatLayerFn(torch.autograd.Function):
         ctx.edge_scale = edge_scale if Fe else None
         ctx.edge_mean = edge_mean if (Fe and edge_scale is not None) else None
         ctx.save_for_backward(x, ea, W, a_src, a_dst, W_e, a_edge, W_aug, v, P_aug, x16, x_blk, p_amax, et, sd32)
+        ctx.out_shape, ctx.device = out.shape, dev
         if want_alpha:
-            ctx.mark_non_differentiable(alpha)
+            # alpha (after attention dropout) is differentiable, as in PyG: a loss on it reaches every input through the
+            # attention backward's d_alpha term.  Unused outputs arrive as None in the backward, not as zeros.
+            ctx.set_materialize_grads(False)
             return out, alpha
         return out, None
 
     @staticmethod
-    def backward(ctx, dout, _dalpha=None):
-        with torch.cuda.device(dout.device):
-            return _GatLayerFn._backward(ctx, dout)
+    def backward(ctx, dout, dalpha=None):
+        with torch.cuda.device(ctx.device):
+            return _GatLayerFn._backward(ctx, dout, dalpha)
 
     @staticmethod
-    def _backward(ctx, dout):
+    def _backward(ctx, dout, dalpha=None):
         lib = _lib.load()
         x, ea, W, a_src, a_dst, W_e, a_edge, W_aug, v, P_aug, x16, x_blk, p_amax, et, sd32 = ctx.saved_tensors
         desc, topo, Fe = ctx.desc, ctx.topo, ctx.Fe
@@ -310,7 +313,11 @@ class _GatLayerFn(torch.autograd.Function):
         st = stream_ptr(dev)
         H, Cc = desc.H, desc.C
         HC = H * Cc
-        dout = dout.contiguous()
+        # a loss on alpha alone: out received no gradient
+        dout = torch.zeros(ctx.out_shape, device=dev, dtype=torch.float32) if dout is None else dout.contiguous()
+        # dalpha: [B, H, N, N] gradient w.r.t. the returned coefficients, the _dalpha entry points' extra input
+        if dalpha is not None:
+            dalpha = dalpha.to(torch.float32).contiguous()
         _, ws_a, ws_p = _workspace(desc)
         ws = torch.empty(max(ws_a, ws_p), device=dev, dtype=torch.uint8)
         # on the tensor-core path the attention backward emits dP directly as the GEMMs' fp16 operand pair
@@ -332,15 +339,23 @@ class _GatLayerFn(torch.autograd.Function):
         # d(edge terms) out: structured source (dv from the windows), or edge_attr.grad wanted (dv as usual)
         d_et = torch.empty_like(et) if (win is not None or want_dea) else None
         if pair:
-            check(lib.spotv2_gat_attn_bwd_pair(C.byref(desc), ptr(P_aug[0]), ptr(P_aug[1]) if P_aug.shape[0] > 1 else None, ptr(p_amax),
-                                               ptr(sd32), ptr(ea), ptr(et), ptr(topo.table) if (Fe and win is None) else None, ptr(v),
-                                               ptr(dout), ptr(ph), ptr(pl), ptr(dp_blk), ptr(dv) if win is None else None,
-                                               ptr(d_et), ptr(dbias), ptr(ws), ws.numel(), st), "spotv2_gat_attn_bwd_pair")
+            args = (C.byref(desc), ptr(P_aug[0]), ptr(P_aug[1]) if P_aug.shape[0] > 1 else None, ptr(p_amax),
+                    ptr(sd32), ptr(ea), ptr(et), ptr(topo.table) if (Fe and win is None) else None, ptr(v),
+                    ptr(dout), ptr(ph), ptr(pl), ptr(dp_blk), ptr(dv) if win is None else None,
+                    ptr(d_et), ptr(dbias), ptr(ws), ws.numel(), st)
+            if dalpha is None:
+                check(lib.spotv2_gat_attn_bwd_pair(*args), "spotv2_gat_attn_bwd_pair")
+            else:
+                check(lib.spotv2_gat_attn_bwd_pair_dalpha(*args, ptr(dalpha)), "spotv2_gat_attn_bwd_pair_dalpha")
         else:
-            check(lib.spotv2_gat_attn_bwd(C.byref(desc), ptr(P_aug), ptr(p_amax), ptr(ea), ptr(et),
-                                          ptr(topo.table) if (Fe and win is None) else None, ptr(v),
-                                          ptr(dout), ptr(dP_aug), ptr(ph), ptr(pl), ptr(dp_blk), ptr(dv) if win is None else None,
-                                          ptr(d_et), ptr(dbias), ptr(ws), ws.numel(), st), "spotv2_gat_attn_bwd")
+            args = (C.byref(desc), ptr(P_aug), ptr(p_amax), ptr(ea), ptr(et),
+                    ptr(topo.table) if (Fe and win is None) else None, ptr(v),
+                    ptr(dout), ptr(dP_aug), ptr(ph), ptr(pl), ptr(dp_blk), ptr(dv) if win is None else None,
+                    ptr(d_et), ptr(dbias), ptr(ws), ws.numel(), st)
+            if dalpha is None:
+                check(lib.spotv2_gat_attn_bwd(*args), "spotv2_gat_attn_bwd")
+            else:
+                check(lib.spotv2_gat_attn_bwd_dalpha(*args, ptr(dalpha)), "spotv2_gat_attn_bwd_dalpha")
         if win is not None:
             wsz = C.c_size_t()
             check(lib.spotv2_windows_dv_workspace_bytes(C.byref(desc), C.byref(wsz)), "windows_dv_workspace_bytes")
@@ -398,6 +413,34 @@ class _GatLayerFn(torch.autograd.Function):
         if not Fe and W_e is not None:          # layer has lin_edge but was called with edge_attr=None
             dW_e, da_edge = torch.zeros_like(W_e), torch.zeros_like(a_edge)
         return (dx, d_ea, dW, da_src, da_dst, dW_e, da_edge, dbias) + (None,) * 11 + (d_scale, d_mean)
+
+
+class _AlphaToPyg(torch.autograd.Function):
+    """Attention tile [B, H, N, N] -> PyG order [B*R + B*N, H] (input self-loop rows zero), and back for the gradient."""
+
+    @staticmethod
+    def forward(ctx, alpha_tile, topo, desc):
+        lib = _lib.load()
+        dev = alpha_tile.device
+        ctx.topo, ctx.desc = topo, desc
+        alpha = torch.empty(topo.B * topo.R + topo.B * topo.N, desc.H, device=dev, dtype=torch.float32)
+        with torch.cuda.device(dev):
+            check(lib.spotv2_alpha_to_pyg(C.byref(desc), ptr(alpha_tile), ptr(topo.table), ptr(alpha), stream_ptr(dev)),
+                  "spotv2_alpha_to_pyg")
+        return alpha
+
+    @staticmethod
+    def backward(ctx, g):
+        lib = _lib.load()
+        topo, desc = ctx.topo, ctx.desc
+        g = g.to(torch.float32).contiguous()
+        dev = g.device
+        # every tile entry is written once (the table of a complete graph): no zero fill
+        d_tile = torch.empty(topo.B, desc.H, topo.N, topo.N, device=dev, dtype=torch.float32)
+        with torch.cuda.device(dev):
+            check(lib.spotv2_alpha_to_pyg_grad(C.byref(desc), ptr(g), ptr(topo.table), ptr(d_tile), stream_ptr(dev)),
+                  "spotv2_alpha_to_pyg_grad")
+        return d_tile, None, None
 
 
 # --------------------------------------------------------------------------- module
@@ -556,17 +599,14 @@ class GATConv(nn.Module):
         return out, self._attention_weights(alpha_tile, topo, edge_index)
 
     def _attention_weights(self, alpha_tile: Tensor, topo: Topology, edge_index: Tensor):
-        """(edge_index with self loops appended, alpha [E', H]) in PyG order (App. A.4)."""
+        """(edge_index with self loops appended, alpha [E', H]) in PyG order (App. A.4); alpha carries gradient."""
         lib = _lib.load()
         dev = alpha_tile.device
         H = self.heads
         desc = GatDesc(topo.B, topo.N, self.in_channels, 0, H, self.out_channels, topo.R, int(self.concat),
                        float(self.negative_slope), lib.spotv2_gat_ldp(H, self.out_channels), 0, 0, 0.0, 0, 0, 0)
         n = topo.B * topo.N
-        alpha = torch.empty(topo.B * topo.R + n, H, device=dev, dtype=torch.float32)
-        with torch.cuda.device(dev):
-            check(lib.spotv2_alpha_to_pyg(C.byref(desc), ptr(alpha_tile), ptr(topo.table), ptr(alpha), stream_ptr(dev)),
-                  "spotv2_alpha_to_pyg")
+        alpha = _AlphaToPyg.apply(alpha_tile, topo, desc)
         loops = torch.arange(n, device=dev, dtype=edge_index.dtype)
         if topo.has_skips:                               # PyG drops input self loops before appending its own
             keep = edge_index[0] != edge_index[1]

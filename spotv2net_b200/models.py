@@ -42,7 +42,10 @@ class GATModel(nn.Module):
         self.dropout = dropout
         self.activation = activation
         # 6_results.ipynb's analysis variant of this class calls every layer with return_attention_weights=True and keeps
-        # the result in self.attention_weights; set collect_attention = True for the same behaviour
+        # the result in self.attention_weights; set collect_attention = True for the same behaviour.  Under autograd (training,
+        # no torch.no_grad) each alpha is differentiable, so a loss may penalise or supervise the coefficients; each layer's
+        # [B, H, N, N] attention tile (88 MB at the default geometry with B = 4096) then stays alive as long as the graph
+        # holds that alpha.  spotv2net_b200.attention_weights runs under no_grad and keeps nothing.
         self.collect_attention = False
         self.attention_weights = []
         self.standardize = standardize

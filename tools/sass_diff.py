@@ -76,7 +76,7 @@ def sass_by_function(binaries: list[Path]) -> dict[str, list[str]]:
                 insn = " ".join(m.group(1).split())
                 body.append(REL_TARGET.sub(r"\1<target>\2", insn))
             elif line.strip() and not line.strip().startswith(("code for", ".target", "Fatbin", "===", "arch =", "code version",
-                                                                "host =", "compile_size", "identifier")):
+                                                                "host =", "compile_size", "identifier", "compressed")):
                 body.append(" ".join(line.split()))
         if name is not None and name != "<end>":
             out[name] = body
