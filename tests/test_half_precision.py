@@ -266,9 +266,11 @@ def dense_logits(s, d_, T, v):
     return s.unsqueeze(1) + d_.unsqueeze(2) + gt
 
 
-def dense_attention(P, s, d_, T, v, bias, dout, H, concat, slope, mask=None, keep_scale=1.0):
+def dense_attention(P, s, d_, T, v, bias, dout, H, concat, slope, mask=None, keep_scale=1.0, d_alpha=None):
     """fp64 forward and backward of the attention stage from a GIVEN projection: P [B, N, H, C], s / d [B, N, H], T the
-    target-major edge tile [B, N, N, Fe] or None, v [H, Fe]; mask [B, i, j, H] (True = kept) replays attention dropout."""
+    target-major edge tile [B, N, N, Fe] or None, v [H, Fe]; mask [B, i, j, H] (True = kept) replays attention dropout;
+    d_alpha [B, i, j, H]: the gradient through the returned (post-dropout) coefficients, which joins dalpha before the
+    dropout factor."""
     B, N, _, C_ = P.shape
     z = dense_logits(s, d_, T, v)
     alpha = torch.softmax(torch.where(z > 0, z, z * slope), dim=2)                  # [b, i, j, h]
@@ -279,6 +281,8 @@ def dense_attention(P, s, d_, T, v, bias, dout, H, concat, slope, mask=None, kee
         out = out + bias
     dO = dout.view(B, N, H, C_) if concat else (dout.view(B, N, 1, C_) / H).expand(B, N, H, C_)
     dad = torch.einsum("bihc,bjhc->bijh", dO, P)
+    if d_alpha is not None:
+        dad = dad + d_alpha
     dal = dad if mask is None else dad * mask * keep_scale
     dl = alpha * (dal - (alpha * dal).sum(2, keepdim=True))
     dz = dl * torch.where(z > 0, torch.ones_like(z), torch.full_like(z, slope))
